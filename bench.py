@@ -2,6 +2,10 @@
 """bench.py — the hot path of BASELINE.json's north_star.
 
     python bench.py --gpus N --steps K --warmup W [--config 2|3|4|5]      (our arm)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR      (config 2, plus the last step's outputs)
+
+--dump-outputs exists for config 2 of our arm only: configs 1, 3, 4, 5 and --impl reference refuse it, so
+their outputs cannot be compared between builds this way.
     python bench.py --impl reference --gpus N --steps K ... [--config C]   (CPU port of the reference)
 
 Default (--config 2, the configuration BASELINE.json's metric is quoted on; BASELINE.json
@@ -196,7 +200,7 @@ def run_reference(args):
     sample = f"the full [256,64,56,56] per-GPU tensor per step, {steps} steps, {threads} host threads (batch-sliced)"
     line = {
         "impl": "reference", "metric": METRIC, "value": round(gbs, 3), "unit": "GB/s", "n_gpus": args.gpus,
-        "steps": args.steps, "warmup": args.warmup, "ms_per_step": round(dt * 1e3, 3), "higher_is_better": True,
+        "steps": steps, "warmup": args.warmup, "ms_per_step": round(dt * 1e3, 3), "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config_dict(args.sparsity),
         "elems_per_s": round(eps, 1),
         "cpu_baseline": {"value": round(gbs, 3), "unit": "GB/s", "cores": threads, "kind": "port", "sample": sample},
@@ -384,6 +388,9 @@ def run_ours(args):
     barrier()
     t_wall = time.perf_counter() - t_wall
     ms = start.elapsed_time(end)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, y=y, gx=gx, magnitude=st["mag"], mask=st["mask"], scale=st["scale"],
+                     decimal=st["dec"])
     if t_wall < 0.5:
         # the timed region is shorter than a few nvidia-smi samples: keep the identical
         # load running (untimed) so the sampler sees the clocks this workload runs at
@@ -688,9 +695,29 @@ def run_ours(args):
         sys.exit(3)
 
 
+DUMP_SAMPLE = 1 << 22        # draws per large output: ~4.0 M distinct elements, 16 MB of float32 each
+
+
+def dump_outputs(torch, out_dir, **arrays):
+    """Writes `out_dir/<name>.npy` as float32.  Outputs of more than DUMP_SAMPLE elements are reduced to the
+    same seeded, sorted sample of flat indices in every run, so two builds can be compared element for element."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    samples = {}
+    for name, a in arrays.items():
+        flat = a.detach().reshape(-1).float()
+        n = flat.numel()
+        if n > DUMP_SAMPLE:
+            if n not in samples:
+                samples[n] = torch.from_numpy(np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLE)))
+            flat = flat[samples[n].to(flat.device)]
+        np.save(out / f"{name}.npy", flat.cpu().numpy())
+
+
 def time_gpu_eager(torch, x, g, C, sparsity, n, our_ms):
-    """The reference's own eager ATen op sequence (oracle/torch_eager.py, checked against the imported
-    reference in tests/test_torch_eager_vs_reference.py) on the same CUDA tensors: what stock qsparse
+    """The reference's own eager ATen op sequence (oracle/torch_eager.py, checked against the reference's
+    recorded outputs in tests/test_torch_eager_vs_reference.py) on the same CUDA tensors: what stock qsparse
     costs on this B200."""
     from oracle.torch_eager import PruneQuantizeEager
     eager = PruneQuantizeEager(C, x.device, sparsity=sparsity, bits=BITS)
@@ -810,7 +837,9 @@ def multi_gpu_parity(torch, dist, ops, x, LAYOUT, C, k, BITS, world, rank, dev, 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000,
+                    help="timed steps of the config-2 GPU run; configs 1, 3-5 and --impl reference cap it to bound "
+                         "their run time, and every JSON line reports the count that was timed")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=[1, 2, 3, 4, 5],
@@ -833,7 +862,15 @@ def main():
     ap.add_argument("--l2-persist-mb", type=int, default=None, help="development: tuning key 21 (L2 set-aside, MB)")
     ap.add_argument("--c1-decimal", action="store_true", help="config 1: DecimalQuantizer instead of the default ScalerQuantizer")
     ap.add_argument("--strong", action="store_true", help="config 5: strong scaling (total size fixed as N grows)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="config 2 of our arm only (configs 1, 3-5 and --impl reference refuse it): write what the last "
+                         "timed step computed on rank 0 as DIR/<name>.npy (float32): y and gx (a fixed seeded "
+                         "sample of 4 M elements each), magnitude, mask, scale, decimal")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 2 or args.impl != "ours"):
+        ap.error("--dump-outputs is implemented for --config 2 --impl ours")
     if args.config == 2 and args.sparsity is None:
         args.sparsity = 0.75
     if args.impl == "reference":

@@ -265,7 +265,7 @@ def cpu_c3(threads, steps):
         step()
     dt = (time.perf_counter() - t0) / steps
     n = w.size
-    return {"value": round(8 * n / dt / 1e9, 3), "unit": "GB/s", "cores": threads, "kind": "port",
+    return {"value": round(8 * n / dt / 1e9, 3), "unit": "GB/s", "cores": threads, "kind": "port", "steps": steps,
             "sample": f"{steps} accesses of the full [4096,4096] weight, row-sliced over the threads, {dt*1e3:.1f} ms/step",
             "elems_per_s": round(n / dt, 1), "ms_per_step": round(dt * 1e3, 3)}
 
@@ -534,7 +534,7 @@ def cpu_c4(threads, sparsity):
     list(pool.map(one, range(layers)))
     dt = time.perf_counter() - t0
     n = sum(w.size for w in ws)
-    return {"value": round(29 * n / dt / 1e9, 3), "unit": "GB/s", "cores": layers, "kind": "port",
+    return {"value": round(29 * n / dt / 1e9, 3), "unit": "GB/s", "cores": layers, "kind": "port", "steps": 1,
             "sample": f"one step over {layers} of the 29 layers ([512,512,3,3] each, one per thread; qsort-based threshold), "
                       f"{dt:.1f} s", "elems_per_s": round(n / dt, 1)}
 
@@ -709,7 +709,7 @@ def cpu_c5(threads):
     for _ in range(steps):
         list(pool.map(part, sl))
     dt = (time.perf_counter() - t0) / steps
-    return {"value": round(18 * n / dt / 1e9, 3), "unit": "GB/s", "cores": threads, "kind": "port",
+    return {"value": round(18 * n / dt / 1e9, 3), "unit": "GB/s", "cores": threads, "kind": "port", "steps": steps,
             "sample": f"{steps} forward+backward passes over 2^26 elements, sliced over the threads, {dt*1e3:.0f} ms/step",
             "elems_per_s": round(n / dt, 1)}
 
@@ -968,7 +968,8 @@ def run_reference(args):
         for _ in range(n):
             cstep()
         dt = (time.perf_counter() - t0) / n
-        cpu = {"value": round(1 / dt, 2), "unit": "steps/s", "cores": threads, "kind": "port", "ms_per_step": round(dt * 1e3, 3),
+        cpu = {"value": round(1 / dt, 2), "unit": "steps/s", "cores": threads, "kind": "port", "steps": n,
+               "ms_per_step": round(dt * 1e3, 3),
                "sample": f"{n} steady-state training steps of the eager restatement of the reference's layers on CPU tensors"}
         metric, cfg = C1_METRIC, c1_config("ScalerQuantizer")
     elif args.config == 3:
@@ -982,7 +983,7 @@ def run_reference(args):
         cpu = cpu_c5(threads)
         metric, cfg = C5_METRIC, c5_config(args.strong, [20, 22, 24, 26, 28, 30, 32])
     v = cpu["value"]
-    return {"impl": "reference", "metric": metric, "value": v, "unit": cpu["unit"], "n_gpus": args.gpus, "steps": args.steps,
+    return {"impl": "reference", "metric": metric, "value": v, "unit": cpu["unit"], "n_gpus": args.gpus, "steps": cpu["steps"],
             "warmup": args.warmup, "ms_per_step": cpu.get("ms_per_step"), "higher_is_better": True,
             "scaling": "strong" if (args.config == 5 and args.strong) else "weak", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "config": cfg, "cpu_baseline": cpu,

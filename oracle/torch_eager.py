@@ -159,7 +159,7 @@ def masked_pow2_fwd_bwd(x, g, mask, decimal, bits=8):
 # config 1: the reference's LAYERS as eager nn.Modules (control flow of qsparse/quantize.py:473-518 and
 # qsparse/sparse.py:99-122,215-273 incl. their `.item()` host syncs), so that the converted MNIST net of
 # examples/mnist.py can be timed on the GPU box without the reference tree.  Checked step for step against the
-# imported reference in tests/test_torch_eager_vs_reference.py.
+# reference's recorded run in tests/test_torch_eager_vs_reference.py.
 # ---------------------------------------------------------------------------------------------------------
 import torch.nn as nn
 import torch.nn.functional as F
