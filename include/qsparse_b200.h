@@ -36,6 +36,15 @@ extern "C" {
 #define QSB_E_ALIGN (-3)      /* pointer not 4-byte aligned                     */
 #define QSB_E_UNSUPPORTED (-4)
 
+/* element type of a tensor argument of the *_dt entry points.  16-bit inputs are
+ * upcast on load (exact) and computed in fp32, so a bf16 / fp16 x gives bit for
+ * bit what the fp32 entry point gives on x converted to fp32; 16-bit outputs are
+ * rounded to nearest even (what a cast of the fp32 result rounds to).  16-bit
+ * pointers need only 2-byte alignment.  Any other code is QSB_E_BADARG. */
+#define QSB_DTYPE_F32 0
+#define QSB_DTYPE_BF16 1
+#define QSB_DTYPE_F16 2
+
 /* mask_kind */
 #define QSB_MASK_NONE 0
 #define QSB_MASK_CHANNEL 1 /* uint8 mask[channels]  (structured prune)          */
@@ -137,6 +146,22 @@ int qsb_fq_line_fwd(const float *x, float *y, const float *lines_dev,
                     int mask_kind, int64_t outer, int64_t channels,
                     int64_t inner, void *stream);
 
+/* The three forwards on an x of element type x_dtype (QSB_DTYPE_*); y stays fp32.
+ * The fp32 entry points above are the QSB_DTYPE_F32 case. */
+int qsb_fq_pow2_fwd_dt(const void *x, int x_dtype, float *y, const float *decimal_dev,
+                       int64_t n_decimal, double decimal_host,
+                       const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                       int64_t channels, int64_t inner, void *stream);
+int qsb_fq_scaler_fwd_dt(const void *x, int x_dtype, float *y, const float *scaler_dev,
+                         int64_t n_scaler, float scaler_host,
+                         const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                         int64_t channels, int64_t inner, void *stream);
+int qsb_fq_line_fwd_dt(const void *x, int x_dtype, float *y, const float *lines_dev,
+                       int64_t n_lines, float lo_host, float hi_host, int bits,
+                       int float_zero_point, const uint8_t *mask_dev,
+                       int mask_kind, int64_t outer, int64_t channels,
+                       int64_t inner, void *stream);
+
 /* Integer export (SURVEY 8f-3): the integer CODE of a fake-quantizer, one byte per
  * element (5 B/elem instead of 8), for deployment after quantization-aware training.
  *   kind 0 (decimal): q = clamp(int32_rz(x * 2^d), -2^(b-1), 2^(b-1)-1)   as int8
@@ -175,13 +200,21 @@ int qsb_quant_export_int4(const float *x, uint8_t *q_out, int kind,
  * g_clamped_out: where v is written; pass g itself for the reference's in-place
  *   side effect (quantize.py:72), or NULL to skip it.
  * gx_out: where v * mask is written (the autograd of `x * mask`,
- *   sparse.py:66,116); NULL when mask_kind == QSB_MASK_NONE.
+ *   sparse.py:66,116), or v itself when mask_kind == QSB_MASK_NONE; may be NULL.
  * ---------------------------------------------------------------------- */
 int qsb_ste_bwd(const float *g, float *g_clamped_out, float *gx_out,
                 const float *scale_dev, int64_t n_scale, double scale_host,
                 int scale_is_decimal, int bits, int notch,
                 const uint8_t *mask_dev, int mask_kind, int64_t outer,
                 int64_t channels, int64_t inner, void *stream);
+/* The same with gx_out of element type gx_dtype (QSB_DTYPE_*): the input gradient
+ * of a 16-bit x written in x's dtype in the same pass that clamps g in place
+ * (g and g_clamped_out stay fp32). */
+int qsb_ste_bwd_dt(const float *g, float *g_clamped_out, void *gx_out, int gx_dtype,
+                   const float *scale_dev, int64_t n_scale, double scale_host,
+                   int scale_is_decimal, int bits, int notch,
+                   const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                   int64_t channels, int64_t inner, void *stream);
 
 /* ------------------------------------------------------------------------
  * K6  prune mask apply, forward and backward (same arithmetic).
@@ -191,6 +224,12 @@ int qsb_ste_bwd(const float *g, float *g_clamped_out, float *gx_out,
 int qsb_mask_apply(const float *x, float *y, const uint8_t *mask_dev,
                    int mask_kind, int64_t outer, int64_t channels,
                    int64_t inner, void *stream);
+/* x of element type x_dtype, y of element type y_dtype (QSB_DTYPE_*): a 16-bit
+ * activation masked into an fp32 y (forward), an fp32 gradient masked into a
+ * 16-bit gx (backward).  y may alias x only when the dtypes are equal. */
+int qsb_mask_apply_dt(const void *x, int x_dtype, void *y, int y_dtype,
+                      const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                      int64_t channels, int64_t inner, void *stream);
 
 /* ------------------------------------------------------------------------
  * K3  statistic reductions, one read of x for any combination of `what`.
@@ -223,6 +262,16 @@ int qsb_reduce_stats_fused(const float *x, int what, int64_t outer, int64_t chan
                            double *abssum, double *nnz, float *tensor_min,
                            void *workspace, int64_t workspace_bytes,
                            unsigned int *arrival_counter_dev, void *stream);
+/* qsb_reduce_stats on an x of element type x_dtype (QSB_DTYPE_*).  The reduction plan —
+ * segments, row bands, vectors of 8, fp32 pre-sums and with them the summation order — is
+ * the same function of the shape for every dtype (vectors are counted from x[0], i.e. as
+ * for an fp32 x that starts on a 32-byte boundary), so a 16-bit x gives the statistics of
+ * its fp32 copy bit for bit.  The tile kernel that tuning key 20 can select for short rows
+ * is fp32 only: with it a 16-bit x returns QSB_E_UNSUPPORTED. */
+int qsb_reduce_stats_dt(const void *x, int x_dtype, int what, int64_t outer, int64_t channels,
+                        int64_t inner, float *absmax, float *mn, float *mx,
+                        double *abssum, double *nnz, float *tensor_min,
+                        void *workspace, int64_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------
  * K4  tiny on-device parameter updates (no host sync).
@@ -489,6 +538,10 @@ int qsb_prune_quant_params(float *magnitude, uint8_t *mask, float *scale,
 int qsb_reduce_partials(const float *x, int64_t outer, int64_t channels,
                         int64_t inner, void *workspace, int64_t workspace_bytes,
                         void *stream);
+/* x of element type x_dtype (QSB_DTYPE_*); plan and summation order as qsb_reduce_stats_dt. */
+int qsb_reduce_partials_dt(const void *x, int x_dtype, int64_t outer, int64_t channels,
+                           int64_t inner, void *workspace, int64_t workspace_bytes,
+                           void *stream);
 
 typedef struct qsb_p2p_group qsb_p2p_group;
 /* exchange-buffer size for `world` ranks (<= 16) and `channels` channels */
@@ -568,6 +621,19 @@ int qsb_reduce_prune_quant_step(const float *x, int64_t outer, int64_t channels,
                                 double *abssum_out, float *absmax_out,
                                 int stats_local, int64_t *step_counter_dev,
                                 uint64_t *timing_out_dev, void *stream);
+/* x of element type x_dtype (QSB_DTYPE_*); plan and summation order as qsb_reduce_stats_dt. */
+int qsb_reduce_prune_quant_step_dt(const void *x, int x_dtype, int64_t outer, int64_t channels,
+                                   int64_t inner, void *workspace,
+                                   int64_t workspace_bytes,
+                                   unsigned int *arrival_counter_dev,
+                                   float *magnitude, uint8_t *mask, float *scale,
+                                   float *decimal_out, qsb_p2p_group *group,
+                                   int64_t step_stamp, double count, int64_t t_prune,
+                                   int update_magnitude, int refresh_mask, int64_t k,
+                                   int bits, int64_t t_quant, int update_scale,
+                                   double *abssum_out, float *absmax_out,
+                                   int stats_local, int64_t *step_counter_dev,
+                                   uint64_t *timing_out_dev, void *stream);
 
 /* ------------------------------------------------------------------------
  * Host-buffer entry points (what a host-side caller that keeps its tensors in

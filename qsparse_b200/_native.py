@@ -18,6 +18,9 @@ _PKG = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ.get("QSPARSE_B200_LIB", _PKG / "lib" / "libqsparse_b200.so"))
 
 MASK_NONE, MASK_CHANNEL, MASK_ELEMENT = 0, 1, 2
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2
+# element types the activation kernels read and write natively (QSB_DTYPE_*)
+NATIVE_DTYPES = {torch.float32: DTYPE_F32, torch.bfloat16: DTYPE_BF16, torch.float16: DTYPE_F16}
 STAT_ABSMAX, STAT_MINMAX, STAT_ABSSUM, STAT_NNZ = 1, 2, 4, 8
 
 # name -> (restype, argtypes); mirrors include/qsparse_b200.h one to one
@@ -38,6 +41,19 @@ _SIGNATURES = {
     "qsb_ste_bwd": (c_int, [_P, _P, _P, _P, c_int64, c_double, c_int, c_int, c_int, _P, c_int,
                             c_int64, c_int64, c_int64, _P]),
     "qsb_mask_apply": (c_int, [_P, _P, _P, c_int, c_int64, c_int64, c_int64, _P]),
+    "qsb_fq_pow2_fwd_dt": (c_int, [_P, c_int, _P, _P, c_int64, c_double, _P, c_int, c_int64, c_int64, c_int64, _P]),
+    "qsb_fq_scaler_fwd_dt": (c_int, [_P, c_int, _P, _P, c_int64, c_float, _P, c_int, c_int64, c_int64, c_int64, _P]),
+    "qsb_fq_line_fwd_dt": (c_int, [_P, c_int, _P, _P, c_int64, c_float, c_float, c_int, c_int, _P, c_int,
+                                   c_int64, c_int64, c_int64, _P]),
+    "qsb_ste_bwd_dt": (c_int, [_P, _P, _P, c_int, _P, c_int64, c_double, c_int, c_int, c_int, _P, c_int,
+                               c_int64, c_int64, c_int64, _P]),
+    "qsb_mask_apply_dt": (c_int, [_P, c_int, _P, c_int, _P, c_int, c_int64, c_int64, c_int64, _P]),
+    "qsb_reduce_stats_dt": (c_int, [_P, c_int, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64,
+                                    _P]),
+    "qsb_reduce_partials_dt": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, c_int64, _P]),
+    "qsb_reduce_prune_quant_step_dt": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, c_int64, _P, _P, _P, _P, _P,
+                                               _P, c_int64, c_double, c_int64, c_int, c_int, c_int64, c_int, c_int64,
+                                               c_int, _P, _P, c_int, _P, _P, _P]),
     "qsb_reduce_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64]),
     "qsb_reduce_stats": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P]),
     "qsb_reduce_stats_fused": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P,
@@ -214,6 +230,21 @@ def as_f32_contiguous(t: torch.Tensor) -> torch.Tensor:
     if not t.is_contiguous():
         t = t.contiguous()
     return t
+
+
+def dtype_code(t: torch.Tensor) -> int:
+    return NATIVE_DTYPES[t.dtype]
+
+
+def as_native(t: torch.Tensor) -> torch.Tensor:
+    """fp32, bf16 and fp16 tensors as they are (the activation kernels read 16-bit values natively and
+    compute in fp32, so the results equal those of ``t.float()`` bit for bit); any other dtype as fp32."""
+    return t if t.dtype in NATIVE_DTYPES else t.float()
+
+
+def as_native_contiguous(t: torch.Tensor) -> torch.Tensor:
+    t = as_native(t)
+    return t if t.is_contiguous() else t.contiguous()
 
 
 def channel_layout(shape, channel_index: int) -> Tuple[int, int, int]:

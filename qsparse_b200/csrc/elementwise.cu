@@ -30,8 +30,8 @@ namespace qsb {
 // library builds on one box: 142.0 -> 140.1 us (forward alone 140.8, backward alone 142.9), dense line 165.1 -> 164.0
 // (profiles/r02_store_hint_ab.json).  Smaller outputs keep the default policy: a consumer may find them in L2.
 constexpr int64_t kStreamStoreBytes = 96ll << 20;
-template <class Op>
-int launch_map_big_out(const Op &op, const MapIO &io, const Layout &L, cudaStream_t stream) {
+template <class Op, class IO>
+int launch_map_big_out(const Op &op, const IO &io, const Layout &L, cudaStream_t stream) {
   if (L.numel() * 4 >= kStreamStoreBytes) return launch_map<Op, Hint::STREAM, Hint::STREAM>(op, io, L, stream);
   return launch_map<Op, Hint::STREAM, Hint::KEEP>(op, io, L, stream);
 }
@@ -360,15 +360,16 @@ Layout effective_layout(int64_t outer, int64_t channels, int64_t inner,
 
 }  // namespace
 
-extern "C" int qsb_fq_pow2_fwd(const float *x, float *y,
-                               const float *decimal_dev, int64_t n_decimal,
-                               double decimal_host, const uint8_t *mask_dev,
-                               int mask_kind, int64_t outer, int64_t channels,
-                               int64_t inner, void *stream) {
+extern "C" int qsb_fq_pow2_fwd_dt(const void *x_, int x_dtype, float *y,
+                                  const float *decimal_dev, int64_t n_decimal,
+                                  double decimal_host, const uint8_t *mask_dev,
+                                  int mask_kind, int64_t outer, int64_t channels,
+                                  int64_t inner, void *stream) {
+  if (!dtype_ok(x_dtype)) return QSB_E_BADARG;
   if (int e = check_layout(outer, channels, inner)) return e;
   if (int e = check_mask(mask_dev, mask_kind, outer * channels * inner)) return e;
   if (outer * channels * inner == 0) return 0;
-  if (!x || !y) return QSB_E_BADARG;
+  if (!x_ || !y) return QSB_E_BADARG;
   int stride = 0;
   if (decimal_dev) {
     stride = param_stride(n_decimal, channels);
@@ -376,26 +377,37 @@ extern "C" int qsb_fq_pow2_fwd(const float *x, float *y,
   }
   const bool per_channel = stride == 1 || mask_kind == QSB_MASK_CHANNEL;
   const Layout L = effective_layout(outer, channels, inner, per_channel);
-  MapIO io{x, nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
-           y, nullptr, nullptr};
   // Python: toi = 2.0**decimal (double) then cast to the tensor dtype.
   const float toi = (float)pow(2.0, decimal_host);
   const float tof = (float)pow(2.0, -decimal_host);
-  return dispatch_mask(mask_kind, [&](auto mk) {
-    Pow2Op<decltype(mk)::value> op{decimal_dev, stride, toi, tof, mask_dev};
-    return launch_map_big_out(op, io, L, (cudaStream_t)stream);
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    MapIOT<T> io{static_cast<const T *>(x_), nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
+                 y, nullptr, nullptr};
+    return dispatch_mask(mask_kind, [&](auto mk) {
+      Pow2Op<decltype(mk)::value> op{decimal_dev, stride, toi, tof, mask_dev};
+      return launch_map_big_out(op, io, L, (cudaStream_t)stream);
+    });
   });
 }
 
-extern "C" int qsb_fq_scaler_fwd(const float *x, float *y,
-                                 const float *scaler_dev, int64_t n_scaler,
-                                 float scaler_host, const uint8_t *mask_dev,
-                                 int mask_kind, int64_t outer, int64_t channels,
-                                 int64_t inner, void *stream) {
+extern "C" int qsb_fq_pow2_fwd(const float *x, float *y, const float *decimal_dev, int64_t n_decimal,
+                               double decimal_host, const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                               int64_t channels, int64_t inner, void *stream) {
+  return qsb_fq_pow2_fwd_dt(x, QSB_DTYPE_F32, y, decimal_dev, n_decimal, decimal_host, mask_dev, mask_kind, outer,
+                            channels, inner, stream);
+}
+
+extern "C" int qsb_fq_scaler_fwd_dt(const void *x_, int x_dtype, float *y,
+                                    const float *scaler_dev, int64_t n_scaler,
+                                    float scaler_host, const uint8_t *mask_dev,
+                                    int mask_kind, int64_t outer, int64_t channels,
+                                    int64_t inner, void *stream) {
+  if (!dtype_ok(x_dtype)) return QSB_E_BADARG;
   if (int e = check_layout(outer, channels, inner)) return e;
   if (int e = check_mask(mask_dev, mask_kind, outer * channels * inner)) return e;
   if (outer * channels * inner == 0) return 0;
-  if (!x || !y) return QSB_E_BADARG;
+  if (!x_ || !y) return QSB_E_BADARG;
   int stride = 0;
   if (scaler_dev) {
     stride = param_stride(n_scaler, channels);
@@ -403,25 +415,36 @@ extern "C" int qsb_fq_scaler_fwd(const float *x, float *y,
   }
   const bool per_channel = stride == 1 || mask_kind == QSB_MASK_CHANNEL;
   const Layout L = effective_layout(outer, channels, inner, per_channel);
-  MapIO io{x, nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
-           y, nullptr, nullptr};
-  return dispatch_mask(mask_kind, [&](auto mk) {
-    ScalerOp<decltype(mk)::value> op{scaler_dev, stride, scaler_host, mask_dev};
-    return launch_map_big_out(op, io, L, (cudaStream_t)stream);
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    MapIOT<T> io{static_cast<const T *>(x_), nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
+                 y, nullptr, nullptr};
+    return dispatch_mask(mask_kind, [&](auto mk) {
+      ScalerOp<decltype(mk)::value> op{scaler_dev, stride, scaler_host, mask_dev};
+      return launch_map_big_out(op, io, L, (cudaStream_t)stream);
+    });
   });
 }
 
-extern "C" int qsb_fq_line_fwd(const float *x, float *y, const float *lines_dev,
-                               int64_t n_lines, float lo_host, float hi_host,
-                               int bits, int float_zero_point,
-                               const uint8_t *mask_dev, int mask_kind,
-                               int64_t outer, int64_t channels, int64_t inner,
-                               void *stream) {
+extern "C" int qsb_fq_scaler_fwd(const float *x, float *y, const float *scaler_dev, int64_t n_scaler,
+                                 float scaler_host, const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                                 int64_t channels, int64_t inner, void *stream) {
+  return qsb_fq_scaler_fwd_dt(x, QSB_DTYPE_F32, y, scaler_dev, n_scaler, scaler_host, mask_dev, mask_kind, outer,
+                              channels, inner, stream);
+}
+
+extern "C" int qsb_fq_line_fwd_dt(const void *x_, int x_dtype, float *y, const float *lines_dev,
+                                  int64_t n_lines, float lo_host, float hi_host,
+                                  int bits, int float_zero_point,
+                                  const uint8_t *mask_dev, int mask_kind,
+                                  int64_t outer, int64_t channels, int64_t inner,
+                                  void *stream) {
+  if (!dtype_ok(x_dtype)) return QSB_E_BADARG;
   if (int e = check_layout(outer, channels, inner)) return e;
   if (int e = check_mask(mask_dev, mask_kind, outer * channels * inner)) return e;
   if (bits < 0 || bits > 62) return QSB_E_BADARG;
   if (outer * channels * inner == 0) return 0;
-  if (!x || !y) return QSB_E_BADARG;
+  if (!x_ || !y) return QSB_E_BADARG;
   int stride = 0;
   if (lines_dev) {
     stride = param_stride(n_lines, channels);
@@ -430,25 +453,35 @@ extern "C" int qsb_fq_line_fwd(const float *x, float *y, const float *lines_dev,
   }
   const bool per_channel = stride == 1 || mask_kind == QSB_MASK_CHANNEL;
   const Layout L = effective_layout(outer, channels, inner, per_channel);
-  MapIO io{x, nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
-           y, nullptr, nullptr};
   const double N = ldexp(1.0, bits);
   const float n_levels = (float)N;
   const float q_max = (float)(N - 1.0);
-  return dispatch_mask(mask_kind, [&](auto mk) {
-    constexpr int MK = decltype(mk)::value;
-    if (float_zero_point) {
-      LineOp<MK, true> op{lines_dev, stride, lo_host, hi_host,
-                          n_levels,  q_max,  mask_dev};
-      return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(
-          op, io, L, (cudaStream_t)stream);
-    } else {
-      LineOp<MK, false> op{lines_dev, stride, lo_host, hi_host,
-                           n_levels,  q_max,  mask_dev};
-      return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(
-          op, io, L, (cudaStream_t)stream);
-    }
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    MapIOT<T> io{static_cast<const T *>(x_), nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
+                 y, nullptr, nullptr};
+    return dispatch_mask(mask_kind, [&](auto mk) {
+      constexpr int MK = decltype(mk)::value;
+      if (float_zero_point) {
+        LineOp<MK, true> op{lines_dev, stride, lo_host, hi_host,
+                            n_levels,  q_max,  mask_dev};
+        return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(
+            op, io, L, (cudaStream_t)stream);
+      } else {
+        LineOp<MK, false> op{lines_dev, stride, lo_host, hi_host,
+                             n_levels,  q_max,  mask_dev};
+        return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(
+            op, io, L, (cudaStream_t)stream);
+      }
+    });
   });
+}
+
+extern "C" int qsb_fq_line_fwd(const float *x, float *y, const float *lines_dev, int64_t n_lines, float lo_host,
+                               float hi_host, int bits, int float_zero_point, const uint8_t *mask_dev,
+                               int mask_kind, int64_t outer, int64_t channels, int64_t inner, void *stream) {
+  return qsb_fq_line_fwd_dt(x, QSB_DTYPE_F32, y, lines_dev, n_lines, lo_host, hi_host, bits, float_zero_point,
+                            mask_dev, mask_kind, outer, channels, inner, stream);
 }
 
 /* integer codes of the three fake-quantizers */
@@ -566,12 +599,13 @@ extern "C" int qsb_quant_export_int4(const float *x, uint8_t *q_out, int kind,
   return 0;
 }
 
-extern "C" int qsb_ste_bwd(const float *g, float *g_clamped_out, float *gx_out,
-                           const float *scale_dev, int64_t n_scale,
-                           double scale_host, int scale_is_decimal, int bits,
-                           int notch, const uint8_t *mask_dev, int mask_kind,
-                           int64_t outer, int64_t channels, int64_t inner,
-                           void *stream) {
+extern "C" int qsb_ste_bwd_dt(const float *g, float *g_clamped_out, void *gx_out, int gx_dtype,
+                              const float *scale_dev, int64_t n_scale,
+                              double scale_host, int scale_is_decimal, int bits,
+                              int notch, const uint8_t *mask_dev, int mask_kind,
+                              int64_t outer, int64_t channels, int64_t inner,
+                              void *stream) {
+  if (!dtype_ok(gx_dtype)) return QSB_E_BADARG;
   if (int e = check_layout(outer, channels, inner)) return e;
   if (int e = check_mask(mask_dev, mask_kind, outer * channels * inner)) return e;
   if (outer * channels * inner == 0) return 0;
@@ -591,31 +625,46 @@ extern "C" int qsb_ste_bwd(const float *g, float *g_clamped_out, float *gx_out,
   const float n_hi = lm1 + (float)notch;
   float s_host = (float)scale_host;
   if (scale_is_decimal) s_host = (float)pow(2.0, -scale_host);
-  MapIO io{g, nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
-           g_clamped_out, gx_out, nullptr};
   const bool gc = g_clamped_out != nullptr, gx = gx_out != nullptr;
-  return dispatch_mask(mask_kind, [&](auto mk) {
-    constexpr int MK = decltype(mk)::value;
-    auto run = [&](auto op) {
-      return launch_map_big_out(op, io, L, (cudaStream_t)stream);
-    };
-    if (gc && gx)
-      return run(SteOp<MK, true, true>{scale_dev, stride, s_host,
-                                       scale_is_decimal != 0, n_lo, n_hi,
-                                       mask_dev});
-    if (gc)
-      return run(SteOp<MK, true, false>{scale_dev, stride, s_host,
+  // without gx the output type does not matter: one instantiation
+  return dispatch_dtype(gx ? gx_dtype : QSB_DTYPE_F32, [&](auto *tg) {
+    using TG = std::remove_pointer_t<decltype(tg)>;
+    MapIOT<float, float, TG> io{g, nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
+                                g_clamped_out, static_cast<TG *>(gx_out), nullptr};
+    return dispatch_mask(mask_kind, [&](auto mk) {
+      constexpr int MK = decltype(mk)::value;
+      auto run = [&](auto op) {
+        return launch_map_big_out(op, io, L, (cudaStream_t)stream);
+      };
+      if (gc && gx)
+        return run(SteOp<MK, true, true>{scale_dev, stride, s_host,
+                                         scale_is_decimal != 0, n_lo, n_hi,
+                                         mask_dev});
+      if constexpr (std::is_same<TG, float>::value) {
+        if (gc)
+          return run(SteOp<MK, true, false>{scale_dev, stride, s_host,
+                                            scale_is_decimal != 0, n_lo, n_hi,
+                                            mask_dev});
+      }
+      return run(SteOp<MK, false, true>{scale_dev, stride, s_host,
                                         scale_is_decimal != 0, n_lo, n_hi,
                                         mask_dev});
-    return run(SteOp<MK, false, true>{scale_dev, stride, s_host,
-                                      scale_is_decimal != 0, n_lo, n_hi,
-                                      mask_dev});
+    });
   });
 }
 
-extern "C" int qsb_mask_apply(const float *x, float *y, const uint8_t *mask_dev,
-                              int mask_kind, int64_t outer, int64_t channels,
-                              int64_t inner, void *stream) {
+extern "C" int qsb_ste_bwd(const float *g, float *g_clamped_out, float *gx_out, const float *scale_dev,
+                           int64_t n_scale, double scale_host, int scale_is_decimal, int bits, int notch,
+                           const uint8_t *mask_dev, int mask_kind, int64_t outer, int64_t channels,
+                           int64_t inner, void *stream) {
+  return qsb_ste_bwd_dt(g, g_clamped_out, gx_out, QSB_DTYPE_F32, scale_dev, n_scale, scale_host, scale_is_decimal,
+                        bits, notch, mask_dev, mask_kind, outer, channels, inner, stream);
+}
+
+extern "C" int qsb_mask_apply_dt(const void *x, int x_dtype, void *y, int y_dtype, const uint8_t *mask_dev,
+                                 int mask_kind, int64_t outer, int64_t channels,
+                                 int64_t inner, void *stream) {
+  if (!dtype_ok(x_dtype) || !dtype_ok(y_dtype)) return QSB_E_BADARG;
   if (int e = check_layout(outer, channels, inner)) return e;
   if (int e = check_mask(mask_dev, mask_kind, outer * channels * inner)) return e;
   if (mask_kind == QSB_MASK_NONE) return QSB_E_BADARG;
@@ -623,16 +672,37 @@ extern "C" int qsb_mask_apply(const float *x, float *y, const uint8_t *mask_dev,
   if (!x || !y) return QSB_E_BADARG;
   const Layout L = effective_layout(outer, channels, inner,
                                     mask_kind == QSB_MASK_CHANNEL);
-  MapIO io{x, nullptr, mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr,
-           y, nullptr, nullptr};
-  if (mask_kind == QSB_MASK_CHANNEL) {
-    MaskApplyOp<QSB_MASK_CHANNEL> op{mask_dev};
-    return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(
-        op, io, L, (cudaStream_t)stream);
-  }
-  MaskApplyOp<QSB_MASK_ELEMENT> op{mask_dev};
-  return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(
-      op, io, L, (cudaStream_t)stream);
+  // (16-bit in, fp32 out): the forward of `x * mask`; (fp32 in, 16-bit out): its backward; (T, T): plain
+  if (x_dtype != QSB_DTYPE_F32 && y_dtype != QSB_DTYPE_F32 && x_dtype != y_dtype) return QSB_E_UNSUPPORTED;
+  const int dt16 = x_dtype != QSB_DTYPE_F32 ? x_dtype : y_dtype;
+  return dispatch_dtype(dt16, [&](auto *t16) {
+    using T = std::remove_pointer_t<decltype(t16)>;
+    auto run = [&](auto io) {
+      if (mask_kind == QSB_MASK_CHANNEL) {
+        MaskApplyOp<QSB_MASK_CHANNEL> op{mask_dev};
+        return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(op, io, L, (cudaStream_t)stream);
+      }
+      MaskApplyOp<QSB_MASK_ELEMENT> op{mask_dev};
+      return launch_map<decltype(op), Hint::STREAM, Hint::KEEP>(op, io, L, (cudaStream_t)stream);
+    };
+    const uint8_t *inb = mask_kind == QSB_MASK_ELEMENT ? mask_dev : nullptr;
+    if constexpr (std::is_same<T, float>::value) {
+      return run(MapIO{static_cast<const float *>(x), nullptr, inb, static_cast<float *>(y), nullptr, nullptr});
+    } else {
+      if (x_dtype == y_dtype)
+        return run(MapIOT<T, T>{static_cast<const T *>(x), nullptr, inb, static_cast<T *>(y), nullptr, nullptr});
+      if (y_dtype == QSB_DTYPE_F32)
+        return run(MapIOT<T, float>{static_cast<const T *>(x), nullptr, inb, static_cast<float *>(y), nullptr,
+                                    nullptr});
+      return run(MapIOT<float, T>{static_cast<const float *>(x), nullptr, inb, static_cast<T *>(y), nullptr,
+                                  nullptr});
+    }
+  });
+}
+
+extern "C" int qsb_mask_apply(const float *x, float *y, const uint8_t *mask_dev, int mask_kind, int64_t outer,
+                              int64_t channels, int64_t inner, void *stream) {
+  return qsb_mask_apply_dt(x, QSB_DTYPE_F32, y, QSB_DTYPE_F32, mask_dev, mask_kind, outer, channels, inner, stream);
 }
 
 #ifdef QSB_KERNEL_TIMING

@@ -29,14 +29,18 @@
 
 namespace qsb {
 
-struct MapIO {
-  const float *in0;
+// TI: element type of in0, TO0 / TO1: of out0 / out1 (float, or __nv_bfloat16 / __half for 16-bit
+// activations and their gradients); the ops always compute in fp32.
+template <class TI = float, class TO0 = float, class TO1 = float>
+struct MapIOT {
+  const TI *in0;
   const float *in1;
   const uint8_t *inb;
-  float *out0;
-  float *out1;
+  TO0 *out0;
+  TO1 *out1;
   uint8_t *outb;
 };
+using MapIO = MapIOT<>;
 
 // Op requirements:
 //   struct P;                                  per-channel derived constants
@@ -124,9 +128,9 @@ inline int reverse_for() {
 // ---------------------------------------------------------------------------
 // per-tensor
 // ---------------------------------------------------------------------------
-template <class Op, int V, int U, Hint LH, Hint SH>
+template <class Op, int V, int U, Hint LH, Hint SH, class IO>
 __global__ void __launch_bounds__(QSB_THREADS)
-    map_kernel(Op op, MapIO io, int64_t n, int reverse) {
+    map_kernel(Op op, IO io, int64_t n, int reverse) {
   pdl_wait();
   pdl_trigger();
   using P = typename Op::P;
@@ -169,19 +173,19 @@ __global__ void __launch_bounds__(QSB_THREADS)
     if (e < n) {
       float o0, o1;
       uint8_t ob;
-      op.apply(io.in0[e], Op::kIn1 ? io.in1[e] : 0.f,
+      op.apply(to_f(io.in0[e]), Op::kIn1 ? io.in1[e] : 0.f,
                Op::kInB ? io.inb[e] : (uint8_t)1, p, o0, o1, ob);
-      if constexpr (Op::kOut0) io.out0[e] = o0;
-      if constexpr (Op::kOut1) io.out1[e] = o1;
+      if constexpr (Op::kOut0) st1(io.out0 + e, o0);
+      if constexpr (Op::kOut1) st1(io.out1 + e, o1);
       if constexpr (Op::kOutB) io.outb[e] = ob;
     }
   }
 }
 
-template <class Op, int V, int U, Hint LH, Hint SH>
-int launch_map_tensor(const Op &op, const MapIO &io, int64_t n,
+template <class Op, int V, int U, Hint LH, Hint SH, class IO>
+int launch_map_tensor(const Op &op, const IO &io, int64_t n,
                       cudaStream_t stream) {
-  auto kern = map_kernel<Op, V, U, LH, SH>;
+  auto kern = map_kernel<Op, V, U, LH, SH, IO>;
   constexpr int64_t kTile = (int64_t)QSB_THREADS * V * U;
   const int64_t tiles = (n + kTile - 1) / kTile;
   int64_t grid = tiles;
@@ -317,9 +321,9 @@ __device__ __forceinline__ void advance32(uint32_t &col, uint32_t &c,
   if (c >= G.channels) c -= G.channels;
 }
 
-template <class Op, int V, int U, int MODE, Hint LH, Hint SH>
+template <class Op, int V, int U, int MODE, Hint LH, Hint SH, class IO>
 __global__ void __launch_bounds__(QSB_THREADS)
-    map_chan_kernel(Op op, MapIO io, int64_t n, ChanGeom G) {
+    map_chan_kernel(Op op, IO io, int64_t n, ChanGeom G) {
   pdl_wait();
   pdl_trigger();
   using P = typename Op::P;
@@ -442,10 +446,10 @@ __global__ void __launch_bounds__(QSB_THREADS)
       const P pj = param_of((uint32_t)(row % G.channels));
       float o0, o1;
       uint8_t ob;
-      op.apply(io.in0[e], Op::kIn1 ? io.in1[e] : 0.f,
+      op.apply(to_f(io.in0[e]), Op::kIn1 ? io.in1[e] : 0.f,
                Op::kInB ? io.inb[e] : (uint8_t)1, pj, o0, o1, ob);
-      if constexpr (Op::kOut0) io.out0[e] = o0;
-      if constexpr (Op::kOut1) io.out1[e] = o1;
+      if constexpr (Op::kOut0) st1(io.out0 + e, o0);
+      if constexpr (Op::kOut1) st1(io.out1 + e, o1);
       if constexpr (Op::kOutB) io.outb[e] = ob;
     }
   }
@@ -455,9 +459,9 @@ __global__ void __launch_bounds__(QSB_THREADS)
 // per-channel, one CTA per tile, window table (inner >= V)
 // ---------------------------------------------------------------------------
 constexpr uint32_t kUnifyInner = 512;  // P(a warp holds a straddling vector) > ~0.35 below this row length
-template <class Op, int V, int U, int MODE, Hint LH, Hint SH>
+template <class Op, int V, int U, int MODE, Hint LH, Hint SH, class IO>
 __global__ void __launch_bounds__(QSB_THREADS)
-    map_chan_win_kernel(Op op, MapIO io, int64_t n, uint32_t inner,
+    map_chan_win_kernel(Op op, IO io, int64_t n, uint32_t inner,
                         uint32_t channels, int reverse) {
   pdl_wait();
   pdl_trigger();
@@ -574,10 +578,10 @@ __global__ void __launch_bounds__(QSB_THREADS)
       const P pj = tab[(uint32_t)((col0 + (uint32_t)(e - t0)) / inner)];
       float o0, o1;
       uint8_t ob;
-      op.apply(io.in0[e], Op::kIn1 ? io.in1[e] : 0.f,
+      op.apply(to_f(io.in0[e]), Op::kIn1 ? io.in1[e] : 0.f,
                Op::kInB ? io.inb[e] : (uint8_t)1, pj, o0, o1, ob);
-      if constexpr (Op::kOut0) io.out0[e] = o0;
-      if constexpr (Op::kOut1) io.out1[e] = o1;
+      if constexpr (Op::kOut0) st1(io.out0 + e, o0);
+      if constexpr (Op::kOut1) st1(io.out1 + e, o1);
       if constexpr (Op::kOutB) io.outb[e] = ob;
     }
   }
@@ -586,11 +590,11 @@ __global__ void __launch_bounds__(QSB_THREADS)
 #endif
 }
 
-template <class Op, int V, int U, int MODE, Hint LH, Hint SH>
-int launch_map_chan_win(const Op &op, const MapIO &io, int64_t n,
+template <class Op, int V, int U, int MODE, Hint LH, Hint SH, class IO>
+int launch_map_chan_win(const Op &op, const IO &io, int64_t n,
                         const Layout &L, cudaStream_t stream) {
   using P = typename Op::P;
-  auto kern = map_chan_win_kernel<Op, V, U, MODE, LH, SH>;
+  auto kern = map_chan_win_kernel<Op, V, U, MODE, LH, SH, IO>;
   constexpr int64_t kTile = (int64_t)QSB_THREADS * V * U;
   const int64_t tiles = (n + kTile - 1) / kTile;
   const size_t rows_max = (size_t)((L.inner - 1 + kTile - 1) / L.inner + 2);
@@ -601,11 +605,11 @@ int launch_map_chan_win(const Op &op, const MapIO &io, int64_t n,
   return 0;
 }
 
-template <class Op, int V, int U, int MODE, Hint LH, Hint SH>
-int launch_map_chan_variant(const Op &op, const MapIO &io, int64_t n,
+template <class Op, int V, int U, int MODE, Hint LH, Hint SH, class IO>
+int launch_map_chan_variant(const Op &op, const IO &io, int64_t n,
                             const Layout &L, cudaStream_t stream) {
   using P = typename Op::P;
-  auto kern = map_chan_kernel<Op, V, U, MODE, LH, SH>;
+  auto kern = map_chan_kernel<Op, V, U, MODE, LH, SH, IO>;
   constexpr int64_t kTile = (int64_t)QSB_THREADS * V * U;
   ChanGeom G;
   G.inner = (uint32_t)L.inner;
@@ -644,9 +648,9 @@ int launch_map_chan_variant(const Op &op, const MapIO &io, int64_t n,
 // memory.  Measured on [32768, 4096]: pow2 290 -> see profiles (was 0.57 of the copy peak),
 // line 486 us (0.34).
 // ---------------------------------------------------------------------------
-template <class Op, int U, Hint LH, Hint SH>
+template <class Op, int U, Hint LH, Hint SH, class IO>
 __global__ void __launch_bounds__(QSB_THREADS)
-    map_lastdim_kernel(Op op, MapIO io, int64_t n_vec, uint32_t groups, int64_t span) {
+    map_lastdim_kernel(Op op, IO io, int64_t n_vec, uint32_t groups, int64_t span) {
   pdl_wait();
   pdl_trigger();
   using P = typename Op::P;
@@ -705,10 +709,10 @@ __global__ void __launch_bounds__(QSB_THREADS)
   }
 }
 
-template <class Op, Hint LH, Hint SH>
-int launch_map_lastdim(const Op &op, const MapIO &io, int64_t n, const Layout &L, cudaStream_t stream) {
+template <class Op, Hint LH, Hint SH, class IO>
+int launch_map_lastdim(const Op &op, const IO &io, int64_t n, const Layout &L, cudaStream_t stream) {
   constexpr int U = 2;
-  auto kern = map_lastdim_kernel<Op, U, LH, SH>;
+  auto kern = map_lastdim_kernel<Op, U, LH, SH, IO>;
   static int occ = 0;
   if (occ == 0) {
     int o = 0;
@@ -730,8 +734,8 @@ int launch_map_lastdim(const Op &op, const MapIO &io, int64_t n, const Layout &L
 // Picks per-tensor vs per-channel addressing and the widest vector the pointers
 // allow (32 B -> V = 8; otherwise scalar for the channel kernel, 16 B -> V = 4
 // for the per-tensor kernel).
-template <class Op, Hint LH = Hint::STREAM, Hint SH = Hint::KEEP>
-int launch_map(const Op &op, const MapIO &io, const Layout &L,
+template <class Op, Hint LH = Hint::STREAM, Hint SH = Hint::KEEP, class IO = MapIO>
+int launch_map(const Op &op, const IO &io, const Layout &L,
                cudaStream_t stream) {
   const int64_t n = L.numel();
   if (n <= 0) return 0;
@@ -741,32 +745,33 @@ int launch_map(const Op &op, const MapIO &io, const Layout &L,
     // alignment, i.e. the same element alignment as 4V bytes of floats.
     if (p) bits |= reinterpret_cast<uintptr_t>(p) * scale;
   };
-  acc(io.in0, 1);
+  // 16-bit streams: a V-element vector needs 2V-byte alignment, i.e. the same as 4V bytes of floats
+  acc(io.in0, 4 / (int)sizeof(*io.in0));
   if (Op::kIn1) acc(io.in1, 1);
-  if (Op::kOut0) acc(io.out0, 1);
-  if (Op::kOut1) acc(io.out1, 1);
+  if (Op::kOut0) acc(io.out0, 4 / (int)sizeof(*io.out0));
+  if (Op::kOut1) acc(io.out1, 4 / (int)sizeof(*io.out1));
   if (Op::kInB) acc(io.inb, 4);
   if (Op::kOutB) acc(io.outb, is_pack4<Op>::value ? 8 : 4);  // packed nibbles: V / 2 bytes per vector
   if (bits & 3) return QSB_E_ALIGN;
   if (L.channels <= 1) {
-    if ((bits & 31) == 0) return launch_map_tensor<Op, 8, 2, LH, SH>(op, io, n, stream);
-    if ((bits & 15) == 0) return launch_map_tensor<Op, 4, 4, LH, SH>(op, io, n, stream);
-    return launch_map_tensor<Op, 1, 4, LH, SH>(op, io, n, stream);
+    if ((bits & 31) == 0) return launch_map_tensor<Op, 8, 2, LH, SH, IO>(op, io, n, stream);
+    if ((bits & 15) == 0) return launch_map_tensor<Op, 4, 4, LH, SH, IO>(op, io, n, stream);
+    return launch_map_tensor<Op, 1, 4, LH, SH, IO>(op, io, n, stream);
   }
   if (L.inner >= (1LL << 31) || L.channels >= (1LL << 31)) return QSB_E_UNSUPPORTED;
   if ((bits & 31) == 0) {
     if (map_tuning().chan_ctas_per_sm == 0) {
-      if (L.inner % 8 == 0) return launch_map_chan_win<Op, 8, 2, 0, LH, SH>(op, io, n, L, stream);
-      if (L.inner >= 8) return launch_map_chan_win<Op, 8, 2, 1, LH, SH>(op, io, n, L, stream);
+      if (L.inner % 8 == 0) return launch_map_chan_win<Op, 8, 2, 0, LH, SH, IO>(op, io, n, L, stream);
+      if (L.inner >= 8) return launch_map_chan_win<Op, 8, 2, 1, LH, SH, IO>(op, io, n, L, stream);
     } else {  // benchmark knob: the persistent full-table kernel for every shape
-      if (L.inner % 8 == 0) return launch_map_chan_variant<Op, 8, 2, 0, LH, SH>(op, io, n, L, stream);
-      if (L.inner >= 8) return launch_map_chan_variant<Op, 8, 2, 1, LH, SH>(op, io, n, L, stream);
+      if (L.inner % 8 == 0) return launch_map_chan_variant<Op, 8, 2, 0, LH, SH, IO>(op, io, n, L, stream);
+      if (L.inner >= 8) return launch_map_chan_variant<Op, 8, 2, 1, LH, SH, IO>(op, io, n, L, stream);
     }
     if (L.inner == 1 && L.channels % 8 == 0 && map_tuning().lastdim)
-      return launch_map_lastdim<Op, LH, SH>(op, io, n, L, stream);
-    return launch_map_chan_variant<Op, 8, 2, 2, LH, SH>(op, io, n, L, stream);
+      return launch_map_lastdim<Op, LH, SH, IO>(op, io, n, L, stream);
+    return launch_map_chan_variant<Op, 8, 2, 2, LH, SH, IO>(op, io, n, L, stream);
   }
-  return launch_map_chan_variant<Op, 1, 4, 0, LH, SH>(op, io, n, L, stream);
+  return launch_map_chan_variant<Op, 1, 4, 0, LH, SH, IO>(op, io, n, L, stream);
 }
 
 }  // namespace qsb

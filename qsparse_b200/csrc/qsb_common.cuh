@@ -1,7 +1,11 @@
 // Shared device/host helpers for the qsparse_b200 kernels (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 #include "../../include/qsparse_b200.h"
 
@@ -33,7 +37,7 @@ struct DeviceProps {
 // Cached per device (queried once; never synchronises).
 const DeviceProps &device_props();
 
-inline bool aligned_to(const void *p, uintptr_t a) {
+__host__ __device__ inline bool aligned_to(const void *p, uintptr_t a) {
   return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0;
 }
 
@@ -217,6 +221,120 @@ __device__ __forceinline__ void st_vec(float *p, const VecF<V> &r) {
     }
   } else {
     p[0] = r.v[0];
+  }
+}
+
+// ---------------------------------------------------------------------------
+// 16-bit activations (bf16 / fp16): V elements per access — 8 -> one 128-bit
+// access — upcast into the same VecF<V>, so every op computes in fp32 exactly as
+// on an fp32 input (bf16 -> fp32 and fp16 -> fp32 are exact).  Stores round
+// to nearest even like torch's CUDA cast (__float2bfloat16_rn / __float2half_rn).
+// The L2 level qualifier is only legal on 256-bit accesses: STREAM loads and
+// stores of 16-bit data use the default L2 policy, like the 128-bit fp32 forms.
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ float to_f(float v) { return v; }
+__device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float to_f(__half v) { return __half2float(v); }
+__device__ __forceinline__ void st1(float *p, float v) { *p = v; }
+__device__ __forceinline__ void st1(__nv_bfloat16 *p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void st1(__half *p, float v) { *p = __float2half_rn(v); }
+
+// two packed 16-bit values (element 0 in the low half) -> two floats
+__device__ __forceinline__ void unpack2(uint32_t w, const __nv_bfloat16 *, float &a, float &b) {
+  a = __uint_as_float(w << 16);
+  b = __uint_as_float(w & 0xffff0000u);
+}
+__device__ __forceinline__ void unpack2(uint32_t w, const __half *, float &a, float &b) {
+  a = __half2float(__ushort_as_half((unsigned short)(w & 0xffffu)));
+  b = __half2float(__ushort_as_half((unsigned short)(w >> 16)));
+}
+__device__ __forceinline__ uint32_t pack2(float a, float b, const __nv_bfloat16 *) {
+  return (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(a)) |
+         ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(b)) << 16);
+}
+__device__ __forceinline__ uint32_t pack2(float a, float b, const __half *) {
+  return (uint32_t)__half_as_ushort(__float2half_rn(a)) | ((uint32_t)__half_as_ushort(__float2half_rn(b)) << 16);
+}
+
+template <class T>
+inline constexpr bool is_half16 = std::is_same<T, __nv_bfloat16>::value || std::is_same<T, __half>::value;
+
+// 8 packed 16-bit values as one 128-bit load; kept packed (4 registers instead of 8) until unpack8()
+__device__ __forceinline__ uint4 ld_raw16(const void *p) {
+  uint4 w;
+  asm volatile("ld.global.L1::no_allocate.v4.b32 {%0,%1,%2,%3}, [%4];"
+               : "=r"(w.x), "=r"(w.y), "=r"(w.z), "=r"(w.w)
+               : "l"(p));
+  return w;
+}
+template <class T>
+__device__ __forceinline__ VecF<8> unpack8(const uint4 &w) {
+  VecF<8> r;
+  unpack2(w.x, (const T *)nullptr, r.v[0], r.v[1]);
+  unpack2(w.y, (const T *)nullptr, r.v[2], r.v[3]);
+  unpack2(w.z, (const T *)nullptr, r.v[4], r.v[5]);
+  unpack2(w.w, (const T *)nullptr, r.v[6], r.v[7]);
+  return r;
+}
+
+template <int V, Hint H, class T, std::enable_if_t<is_half16<T>, int> = 0>
+__device__ __forceinline__ VecF<V> ld_vec(const T *p) {
+  VecF<V> r;
+  if constexpr (V == 8) {
+    r = unpack8<T>(ld_raw16(p));
+  } else if constexpr (V == 4) {
+    uint32_t w[2];
+    asm volatile("ld.global.L1::no_allocate.v2.b32 {%0,%1}, [%2];" : "=r"(w[0]), "=r"(w[1]) : "l"(p));
+    unpack2(w[0], p, r.v[0], r.v[1]);
+    unpack2(w[1], p, r.v[2], r.v[3]);
+  } else {
+    static_assert(V == 1, "V must be 1, 4 or 8");
+    r.v[0] = to_f(p[0]);
+  }
+  return r;
+}
+
+template <int V, Hint H, class T, std::enable_if_t<is_half16<T>, int> = 0>
+__device__ __forceinline__ void st_vec(T *p, const VecF<V> &r) {
+  if constexpr (V == 8) {
+    uint32_t w[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) w[k] = pack2(r.v[2 * k], r.v[2 * k + 1], (const T *)nullptr);
+    asm volatile("st.global.L1::no_allocate.v4.b32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(w[0]), "r"(w[1]),
+                 "r"(w[2]), "r"(w[3])
+                 : "memory");
+  } else if constexpr (V == 4) {
+    const uint32_t w0 = pack2(r.v[0], r.v[1], (const T *)nullptr), w1 = pack2(r.v[2], r.v[3], (const T *)nullptr);
+    asm volatile("st.global.L1::no_allocate.v2.b32 [%0], {%1,%2};" ::"l"(p), "r"(w0), "r"(w1) : "memory");
+  } else {
+    st1(p, r.v[0]);
+  }
+}
+
+// 8 elements of a vector whose 16-byte alignment is only known at run time (a 16-bit view may start at
+// any even byte address): one 128-bit load when it is aligned, else element by element.
+template <Hint H, class T>
+__device__ __forceinline__ VecF<8> ld_vec8_any(const T *p, bool vec_ok) {
+  if constexpr (!is_half16<T>) {
+    return ld_vec<8, H>(p);
+  } else {
+    if (vec_ok) return ld_vec<8, H>(p);
+    VecF<8> r;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) r.v[j] = to_f(p[j]);
+    return r;
+  }
+}
+
+// dtype codes of the C-ABI (QSB_DTYPE_*) -> element type; any other code is QSB_E_BADARG
+inline bool dtype_ok(int dt) { return dt == QSB_DTYPE_F32 || dt == QSB_DTYPE_BF16 || dt == QSB_DTYPE_F16; }
+template <class F>
+inline int dispatch_dtype(int dt, F &&f) {
+  switch (dt) {
+    case QSB_DTYPE_F32: return f((float *)nullptr);
+    case QSB_DTYPE_BF16: return f((__nv_bfloat16 *)nullptr);
+    case QSB_DTYPE_F16: return f((__half *)nullptr);
+    default: return QSB_E_BADARG;
   }
 }
 

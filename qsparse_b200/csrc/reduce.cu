@@ -454,14 +454,24 @@ __device__ __forceinline__ VecF<8> ld_vec8_policy(const float *p, uint64_t pol) 
       : "l"(p), "l"(pol));
   return r;
 }
+// 8 16-bit values, 16-byte aligned: one 128-bit load with the policy, still packed
+__device__ __forceinline__ uint4 ld_raw16_policy(const void *p, uint64_t pol) {
+  uint4 w;
+  asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.b32 {%0,%1,%2,%3}, [%4], %5;"
+               : "=r"(w.x), "=r"(w.y), "=r"(w.z), "=r"(w.w)
+               : "l"(p), "l"(pol));
+  return w;
+}
 
 // ---------------------------------------------------------------------------
 // stage 1, row mode.  U = 256-bit loads in flight per lane and round, MINB = resident CTAs
 // per SM the register budget is set for (the plan's warp count follows, row_ctas_per_sm()).
 // ---------------------------------------------------------------------------
-template <int WHAT, int U, int MINB, class Tail>
+// T: element type of x; VEC (16-bit x only): x is 16-byte aligned, so every vector is one 128-bit load —
+// false for a view that starts at any other even address (element loads, same vectors, same order)
+template <int WHAT, int U, int MINB, class Tail, class T, bool VEC = true>
 __global__ void __launch_bounds__(QSB_THREADS, MINB)
-    reduce_rows_kernel(const float *__restrict__ x, int64_t rows, int64_t inner,
+    reduce_rows_kernel(const T *__restrict__ x, int64_t rows, int64_t inner,
                        int64_t seg, int64_t segs_per_row, int64_t vwarps,
                        Partials P, int cta_combine, int channels, const __grid_constant__ Tail tail) {
   pdl_wait();
@@ -472,6 +482,9 @@ __global__ void __launch_bounds__(QSB_THREADS, MINB)
   const int lane = threadIdx.x & 31;
   const int64_t warps_phys = (int64_t)gridDim.x * (QSB_THREADS / 32);
   const int64_t items = rows * segs_per_row;
+  // 16-bit x: vectors start at multiples of 8 elements from x[0] (what an fp32 copy of x starting on a 32-byte
+  // boundary gets)
+  static_assert(VEC || is_half16<T>, "an fp32 x is always read with 256-bit loads");
   auto run_vw = [&](Acc<WHAT> &acc, int64_t vw) {
     // every item of a virtual warp belongs to ONE channel
     uint64_t pol = 0;
@@ -487,31 +500,58 @@ __global__ void __launch_bounds__(QSB_THREADS, MINB)
       const int64_t s = item - row * segs_per_row;
       const int64_t c0 = s * seg;
       const int64_t c1 = (c0 + seg < inner) ? c0 + seg : inner;
-      const float *p = x + row * inner + c0;
+      const T *p = x + row * inner + c0;
       const int64_t len = c1 - c0;
-      // head: scalars up to the first 32-byte boundary
-      int64_t head = ((32 - (reinterpret_cast<uintptr_t>(p) & 31)) & 31) >> 2;
+      // head: scalars up to the first 32-byte boundary (16-bit x: up to the next multiple of 8 elements)
+      int64_t head;
+      if constexpr (is_half16<T>) head = (8 - ((row * inner + c0) & 7)) & 7;
+      else head = ((32 - (reinterpret_cast<uintptr_t>(p) & 31)) & 31) >> 2;
       if (head > len) head = len;
-      if (lane < head) acc.add(p[lane]);
-      const float *pv = p + head;
+      if (lane < head) acc.add(to_f(p[lane]));
+      const T *pv = p + head;
       const int64_t nv = (len - head) >> 3;
       // body: 256-bit loads, up to U in flight per lane (predicated, so short pieces do not
       // fall back to one load per round trip); vector order per lane is the same for every U
       for (int64_t j = lane; j < nv; j += 32 * U) {
-        VecF<8> v[U];
+        if constexpr (!VEC) {  // element loads, one vector at a time
 #pragma unroll
-        for (int u = 0; u < U; ++u)
-          if (j + 32 * u < nv) {
-            if (std::is_same<Tail, StepTail>::value && use_pol) v[u] = ld_vec8_policy(pv + ((j + 32 * u) << 3), pol);
-            else v[u] = ld_vec<8, Hint::KEEP>(pv + ((j + 32 * u) << 3));
-          }
+          for (int u = 0; u < U; ++u)
+            if (j + 32 * u < nv) {
+              const VecF<8> w = ld_vec8_any<Hint::KEEP>(pv + ((j + 32 * u) << 3), false);
+              acc.template add_n<8>(w.v);
+            }
+        } else if constexpr (is_half16<T>) {
+          // the U loads in flight stay packed (4 registers each, half of fp32's) until they are accumulated:
+          // unpacked up front, the 4-load variant at 64 registers spilled
+          uint4 w[U];
 #pragma unroll
-        for (int u = 0; u < U; ++u)
-          if (j + 32 * u < nv) acc.template add_n<8>(v[u].v);
+          for (int u = 0; u < U; ++u)
+            if (j + 32 * u < nv) {
+              if (std::is_same<Tail, StepTail>::value && use_pol) w[u] = ld_raw16_policy(pv + ((j + 32 * u) << 3), pol);
+              else w[u] = ld_raw16(pv + ((j + 32 * u) << 3));
+            }
+#pragma unroll
+          for (int u = 0; u < U; ++u)
+            if (j + 32 * u < nv) {
+              const VecF<8> v = unpack8<T>(w[u]);
+              acc.template add_n<8>(v.v);
+            }
+        } else {
+          VecF<8> v[U];
+#pragma unroll
+          for (int u = 0; u < U; ++u)
+            if (j + 32 * u < nv) {
+              if (std::is_same<Tail, StepTail>::value && use_pol) v[u] = ld_vec8_policy(pv + ((j + 32 * u) << 3), pol);
+              else v[u] = ld_vec<8, Hint::KEEP>(pv + ((j + 32 * u) << 3));
+            }
+#pragma unroll
+          for (int u = 0; u < U; ++u)
+            if (j + 32 * u < nv) acc.template add_n<8>(v[u].v);
+        }
       }
       // tail
       const int64_t done = head + (nv << 3);
-      if (done + lane < len) acc.add(p[done + lane]);
+      if (done + lane < len) acc.add(to_f(p[done + lane]));
     }
   };
   if (cta_combine) {
@@ -713,8 +753,8 @@ __global__ void __launch_bounds__(QSB_THREADS, kTileCtasPerSm)
 // warp still reads consecutive memory; the row lanes are then combined through shared
 // memory in lane order (deterministic) and row lane 0 writes the partial.
 // ---------------------------------------------------------------------------
-template <int WHAT, int V>
-__device__ __forceinline__ void reduce_cols_body(const float *__restrict__ x, int64_t nrows, int64_t ncols,
+template <int WHAT, int V, class T>
+__device__ __forceinline__ void reduce_cols_body(const T *__restrict__ x, int64_t nrows, int64_t ncols,
                                                  int64_t rows_per_chunk, int tpr, Partials P) {
   pdl_wait();
   pdl_trigger();
@@ -728,7 +768,7 @@ __device__ __forceinline__ void reduce_cols_body(const float *__restrict__ x, in
   const int64_t r1 = (r0 + rows_per_chunk < nrows) ? r0 + rows_per_chunk : nrows;
   Acc<WHAT> acc[V];
   if (live) {
-    const float *p = x + vc * V;
+    const T *p = x + vc * V;
     int64_t r = r0 + rl;
     for (; r + 3 * (int64_t)rpb < r1; r += 4 * (int64_t)rpb) {
       VecF<V> v[4];
@@ -803,14 +843,14 @@ __device__ __forceinline__ void reduce_cols_body(const float *__restrict__ x, in
   }
 }
 
-template <int WHAT, int V, class Tail>
+template <int WHAT, int V, class Tail, class T>
 __global__ void __launch_bounds__(QSB_THREADS)
-    reduce_cols_kernel(const float *__restrict__ x, int64_t nrows, int64_t ncols,
+    reduce_cols_kernel(const T *__restrict__ x, int64_t nrows, int64_t ncols,
                        int64_t rows_per_chunk, int tpr, Partials P, const __grid_constant__ Tail tail) {
   extern __shared__ __align__(16) unsigned char qsb_dyn_smem[];
   if constexpr (std::is_same<Tail, StepTail>::value) pdl_wait();  // the old state may have been written by the kernel just before
   const StepPrefetch pre = fused_step_begin(tail);
-  reduce_cols_body<WHAT, V>(x, nrows, ncols, rows_per_chunk, tpr, P);
+  reduce_cols_body<WHAT, V, T>(x, nrows, ncols, rows_per_chunk, tpr, P);
   if constexpr (Tail::kFused) fused_tail<WHAT>(tail, P, qsb_dyn_smem, pre);
 }
 
@@ -1080,7 +1120,7 @@ void set_reduce_col_tpr_wide(int v) { g_col_tpr_wide = (v == 32 || v == 64 || v 
 void set_reduce_seg_min(int v) { g_reduce_seg_min = v >= 256 ? v : 256; }
 
 ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner,
-                            const float *x) {
+                            const void *x, int x_bytes) {
   ReducePlan p{};
   p.row_variant = row_variant_for(inner);
   const int64_t warps_phys =
@@ -1158,7 +1198,7 @@ ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner,
     p.row_mode = false;
     p.nrows = outer;
     p.ncols = channels * inner;
-    p.vcol = (p.ncols % 4 == 0 && (x == nullptr || aligned_to(x, 16))) ? 4 : 1;
+    p.vcol = (p.ncols % 4 == 0 && (x == nullptr || aligned_to(x, 4 * x_bytes))) ? 4 : 1;
     // The grid is planned for the vector width the SHAPE allows, whatever the alignment of x: the row
     // bands (and with them the partial layout that qsb_prune_quant_step_params re-derives without x)
     // must not depend on the pointer; an unaligned x only gets 4x more CTAs along the row.
@@ -1225,21 +1265,26 @@ Partials partials_from_workspace(void *workspace, int64_t n_partials) {
   return P;
 }
 
-template <int WHAT, class Tail = NoTail>
-static int run_reduce(const float *x, const ReducePlan &pl, int64_t channels,
+template <int WHAT, class Tail = NoTail, class T = float>
+static int run_reduce(const T *x, const ReducePlan &pl, int64_t channels,
                       int64_t inner, const Partials &P, const FinalOut &out,
                       cudaStream_t stream, bool finalize = true, const Tail &tail = Tail{}) {
   // dynamic shared memory of the fused parameter step (the tile kernel re-uses its tile buffer)
   const size_t dyn = std::is_same<Tail, StepTail>::value ? step_smem_bytes((int)channels) : 0;
   if (pl.row_mode && pl.tile_rows > 0) {
-    const int64_t grid = (pl.vwarps + pl.tile_rows - 1) / pl.tile_rows;
-    auto go = [&](auto kernel) {
-      return launch_k(kernel, dim3((unsigned)grid), dim3(QSB_THREADS), 0, stream, x, pl.rows, (int)inner,
-                      pl.tile_rows, pl.tile_spans, pl.tile_span_stride, pl.vwarps, P, tail);
-    };
-    if (inner <= 64) QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 4, 16, Tail>));
-    else if (inner <= 128) QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 8, 16, Tail>));
-    else QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 8, 32, Tail>));
+    // the tile kernel (only reachable through tuning key 20) stages fp32 sectors: fp32 input only
+    if constexpr (is_half16<T>) {
+      return QSB_E_UNSUPPORTED;
+    } else {
+      const int64_t grid = (pl.vwarps + pl.tile_rows - 1) / pl.tile_rows;
+      auto go = [&](auto kernel) {
+        return launch_k(kernel, dim3((unsigned)grid), dim3(QSB_THREADS), 0, stream, x, pl.rows, (int)inner,
+                        pl.tile_rows, pl.tile_spans, pl.tile_span_stride, pl.vwarps, P, tail);
+      };
+      if (inner <= 64) QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 4, 16, Tail>));
+      else if (inner <= 128) QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 8, 16, Tail>));
+      else QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 8, 32, Tail>));
+    }
   } else if (pl.row_mode) {
     constexpr int kWarps = QSB_THREADS / 32;
     int64_t grid = (int64_t)device_props().sm_count * row_ctas_per_sm(pl.row_variant);
@@ -1249,16 +1294,21 @@ static int run_reduce(const float *x, const ReducePlan &pl, int64_t channels,
       return launch_k(kernel, dim3((unsigned)grid), dim3(QSB_THREADS), dyn, stream, x, pl.rows, inner, pl.seg,
                       pl.segs_per_row, pl.vwarps, P, pl.cta_combine, (int)channels, tail);
     };
-    if (pl.row_variant == 2) QSB_CUDA_TRY(go(reduce_rows_kernel<WHAT, 8, 2, Tail>));
-    else QSB_CUDA_TRY(go(reduce_rows_kernel<WHAT, 4, 4, Tail>));
+    if (!is_half16<T> || aligned_to(x, 16)) {
+      if (pl.row_variant == 2) QSB_CUDA_TRY(go(reduce_rows_kernel<WHAT, 8, 2, Tail, T>));
+      else QSB_CUDA_TRY(go(reduce_rows_kernel<WHAT, 4, 4, Tail, T>));
+    } else if constexpr (is_half16<T>) {
+      if (pl.row_variant == 2) QSB_CUDA_TRY(go(reduce_rows_kernel<WHAT, 8, 2, Tail, T, false>));
+      else QSB_CUDA_TRY(go(reduce_rows_kernel<WHAT, 4, 4, Tail, T, false>));
+    }
   } else {
     const int64_t threads = pl.ncols / pl.vcol;
     dim3 grid((unsigned)((threads + pl.tpr - 1) / pl.tpr), (unsigned)pl.chunks);
     if (pl.vcol == 4)
-      QSB_CUDA_TRY(launch_k(reduce_cols_kernel<WHAT, 4, Tail>, grid, dim3(QSB_THREADS), dyn, stream, x, pl.nrows,
+      QSB_CUDA_TRY(launch_k(reduce_cols_kernel<WHAT, 4, Tail, T>, grid, dim3(QSB_THREADS), dyn, stream, x, pl.nrows,
                             pl.ncols, pl.rows_per_chunk, pl.tpr, P, tail));
     else
-      QSB_CUDA_TRY(launch_k(reduce_cols_kernel<WHAT, 1, Tail>, grid, dim3(QSB_THREADS), dyn, stream, x, pl.nrows,
+      QSB_CUDA_TRY(launch_k(reduce_cols_kernel<WHAT, 1, Tail, T>, grid, dim3(QSB_THREADS), dyn, stream, x, pl.nrows,
                             pl.ncols, pl.rows_per_chunk, pl.tpr, P, tail));
   }
   QSB_LAUNCH_CHECK();
@@ -1299,19 +1349,20 @@ extern "C" int64_t qsb_reduce_workspace_bytes(int64_t outer, int64_t channels,
   return partial_bytes(pl.n_partials) + 256 + stat_row_bytes(channels);
 }
 
-static int reduce_stats_impl(const float *x, int what, int64_t outer, int64_t channels, int64_t inner,
+template <class T>
+static int reduce_stats_impl(const T *x, int what, int64_t outer, int64_t channels, int64_t inner,
                              float *absmax, float *mn, float *mx, double *abssum, double *nnz,
                              float *tensor_min, void *workspace, int64_t workspace_bytes,
                              unsigned int *arrival, void *stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
   if (!x || !workspace) return QSB_E_BADARG;
-  if (!aligned_to(x, 4)) return QSB_E_ALIGN;
+  if (!aligned_to(x, sizeof(T))) return QSB_E_ALIGN;
   if ((what & ~(QSB_STAT_ABSMAX | QSB_STAT_MINMAX | QSB_STAT_ABSSUM |
                 QSB_STAT_NNZ)) || what == 0)
     return QSB_E_BADARG;
   if ((what & QSB_STAT_NNZ) && !(what & QSB_STAT_ABSSUM)) return QSB_E_BADARG;
-  const ReducePlan pl = make_plan(outer, channels, inner, x);
+  const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
   if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
   const Partials P = partials_from_workspace(workspace, pl.n_partials);
   FinalOut out{absmax, mn, mx, abssum, nnz};
@@ -1319,11 +1370,18 @@ static int reduce_stats_impl(const float *x, int what, int64_t outer, int64_t ch
   // small partial arrays: the last-arriving CTA of stage 1 finalizes (one launch instead of two)
   const bool fuse_final = arrival != nullptr && final_tail_ok(channels, pl.fin_count, pl.fin_q);
   const FinalTail ft{out, arrival, channels, pl.fin_count, pl.fin_q, step_group_for(channels, QSB_THREADS)};
+  // the one-launch finalize is only offered for fp32 x (qsb_reduce_stats_fused); no 16-bit instantiation of it
+  auto go = [&](auto w) {
+    constexpr int W = decltype(w)::value;
+    if constexpr (!is_half16<T>) {
+      if (fuse_final) return run_reduce<W, FinalTail, T>(x, pl, channels, inner, P, out, stream, false, ft);
+    }
+    return run_reduce<W, NoTail, T>(x, pl, channels, inner, P, out, stream);
+  };
   switch (what) {
-#define QSB_CASE(W)                                                                                       \
-  case W:                                                                                                 \
-    rc = fuse_final ? run_reduce<W, FinalTail>(x, pl, channels, inner, P, out, stream, false, ft)         \
-                    : run_reduce<W>(x, pl, channels, inner, P, out, stream);                              \
+#define QSB_CASE(W)                                  \
+  case W:                                            \
+    rc = go(std::integral_constant<int, W>{});       \
     break;
     QSB_CASE(QSB_STAT_ABSMAX)
     QSB_CASE(QSB_STAT_MINMAX)
@@ -1333,12 +1391,9 @@ static int reduce_stats_impl(const float *x, int what, int64_t outer, int64_t ch
     QSB_CASE(QSB_STAT_ABSSUM | QSB_STAT_NNZ | QSB_STAT_ABSMAX)
     QSB_CASE(QSB_STAT_ABSMAX | QSB_STAT_MINMAX)
 #undef QSB_CASE
-    default: {
+    default:
       // any other combination: everything in one pass
-      constexpr int kAll = QSB_STAT_ABSMAX | QSB_STAT_MINMAX | QSB_STAT_ABSSUM | QSB_STAT_NNZ;
-      rc = fuse_final ? run_reduce<kAll, FinalTail>(x, pl, channels, inner, P, out, stream, false, ft)
-                      : run_reduce<kAll>(x, pl, channels, inner, P, out, stream);
-    }
+      rc = go(std::integral_constant<int, QSB_STAT_ABSMAX | QSB_STAT_MINMAX | QSB_STAT_ABSSUM | QSB_STAT_NNZ>{});
   }
   if (rc) return rc;
   if ((what & QSB_STAT_NNZ) && tensor_min) {
@@ -1359,6 +1414,16 @@ extern "C" int qsb_reduce_stats(const float *x, int what, int64_t outer, int64_t
                            workspace_bytes, nullptr, stream);
 }
 
+extern "C" int qsb_reduce_stats_dt(const void *x, int x_dtype, int what, int64_t outer, int64_t channels,
+                                   int64_t inner, float *absmax, float *mn, float *mx, double *abssum, double *nnz,
+                                   float *tensor_min, void *workspace, int64_t workspace_bytes, void *stream) {
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    return reduce_stats_impl(static_cast<const T *>(x), what, outer, channels, inner, absmax, mn, mx, abssum, nnz,
+                             tensor_min, workspace, workspace_bytes, nullptr, stream);
+  });
+}
+
 // The same in ONE launch whenever the partial array is small (channels x entries <= 16 Ki): the
 // last-arriving CTA of stage 1 combines the partials itself.  arrival_counter_dev as in
 // qsb_reduce_prune_quant_step (one zeroed uint32 per stream, left zero).
@@ -1374,19 +1439,29 @@ extern "C" int qsb_reduce_stats_fused(const float *x, int what, int64_t outer, i
 
 // Stage 1 only: leaves the per-virtual-warp partials of sum|x| and max|x| in the
 // workspace for qsb_prune_quant_step_params, which finalizes them itself.
-extern "C" int qsb_reduce_partials(const float *x, int64_t outer, int64_t channels,
-                                   int64_t inner, void *workspace,
-                                   int64_t workspace_bytes, void *stream_) {
+extern "C" int qsb_reduce_partials_dt(const void *x_, int x_dtype, int64_t outer, int64_t channels,
+                                      int64_t inner, void *workspace,
+                                      int64_t workspace_bytes, void *stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
+  if (!dtype_ok(x_dtype)) return QSB_E_BADARG;
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
-  if (!x || !workspace) return QSB_E_BADARG;
-  if (!aligned_to(x, 4)) return QSB_E_ALIGN;
-  const ReducePlan pl = make_plan(outer, channels, inner, x);
-  if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
-  const Partials P = partials_from_workspace(workspace, pl.n_partials);
-  FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
-  return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX>(x, pl, channels, inner, P, out,
-                                                      stream, /*finalize=*/false);
+  if (!x_ || !workspace) return QSB_E_BADARG;
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    const T *x = static_cast<const T *>(x_);
+    if (!aligned_to(x, sizeof(T))) return QSB_E_ALIGN;
+    const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
+    if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
+    const Partials P = partials_from_workspace(workspace, pl.n_partials);
+    FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
+    return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, NoTail, T>(x, pl, channels, inner, P, out,
+                                                                   stream, /*finalize=*/false);
+  });
+}
+
+extern "C" int qsb_reduce_partials(const float *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+                                   int64_t workspace_bytes, void *stream) {
+  return qsb_reduce_partials_dt(x, QSB_DTYPE_F32, outer, channels, inner, workspace, workspace_bytes, stream);
 }
 
 // the last-arriving CTA finalizes channels x fin_count partials; beyond this many a second, parallel
@@ -1397,8 +1472,9 @@ constexpr int64_t kStepTailMaxEntries = 12288;
 // prune -> pow2 quantize training step: the stage-1 reduction of sum|x| / max|x| whose
 // last-arriving CTA finalizes, exchanges the statistics row with the peer GPUs and derives
 // magnitude EMA / threshold / mask / scale / decimal (step_epilogue.cuh).
-extern "C" int qsb_reduce_prune_quant_step(
-    const float *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+template <class T>
+static int reduce_prune_quant_step_impl(
+    const T *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
     int64_t workspace_bytes, unsigned int *arrival_counter_dev, float *magnitude, uint8_t *mask,
     float *scale, float *decimal_out, qsb_p2p_group *group, int64_t step_stamp, double count,
     int64_t t_prune, int update_magnitude, int refresh_mask, int64_t k, int bits, int64_t t_quant,
@@ -1408,13 +1484,13 @@ extern "C" int qsb_reduce_prune_quant_step(
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
   if (channels > kStepFusedMaxChannels) return QSB_E_UNSUPPORTED;
   if (!x || !workspace || !arrival_counter_dev) return QSB_E_BADARG;
-  if (!aligned_to(x, 4) || !aligned_to(arrival_counter_dev, 4)) return QSB_E_ALIGN;
+  if (!aligned_to(x, sizeof(T)) || !aligned_to(arrival_counter_dev, 4)) return QSB_E_ALIGN;
   StepTail tail;
   const int rc = fill_step_args(tail.a, magnitude, mask, scale, decimal_out, channels, group, step_stamp, count,
                                 t_prune, update_magnitude, refresh_mask, k, bits, t_quant, update_scale,
                                 abssum_out, absmax_out, stats_local, step_counter_dev, QSB_THREADS);
   if (rc) return rc;
-  const ReducePlan pl = make_plan(outer, channels, inner, x);
+  const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
   if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
   if (pl.fin_count > 0x7fffffffLL || pl.fin_q > 0x7fffffffLL) return QSB_E_UNSUPPORTED;
   const Partials P = partials_from_workspace(workspace, pl.n_partials);
@@ -1427,7 +1503,7 @@ extern "C" int qsb_reduce_prune_quant_step(
     double *row_sum = reinterpret_cast<double *>(row);
     float *row_max = reinterpret_cast<float *>(row + (channels * 8 + 255) / 256 * 256);
     FinalOut out{row_max, nullptr, nullptr, row_sum, nullptr};
-    const int rc2 = run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX>(x, pl, channels, inner, P, out, stream);
+    const int rc2 = run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, NoTail, T>(x, pl, channels, inner, P, out, stream);
     if (rc2) return rc2;
     tail.a.timing = nullptr;
     return launch_step_kernel_on_rows(tail.a, row_sum, row_max, stream);
@@ -1441,6 +1517,36 @@ extern "C" int qsb_reduce_prune_quant_step(
   // the forward pass (only meaningful for a per-channel mask in row mode)
   tail.keep_hint = (g_keep_hint && pl.row_mode && pl.tile_rows == 0 && channels > 1) ? mask : nullptr;
   FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
-  return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, StepTail>(x, pl, channels, inner, P, out, stream,
-                                                                 /*finalize=*/false, tail);
+  return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, StepTail, T>(x, pl, channels, inner, P, out, stream,
+                                                                    /*finalize=*/false, tail);
+}
+
+extern "C" int qsb_reduce_prune_quant_step_dt(
+    const void *x, int x_dtype, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+    int64_t workspace_bytes, unsigned int *arrival_counter_dev, float *magnitude, uint8_t *mask,
+    float *scale, float *decimal_out, qsb_p2p_group *group, int64_t step_stamp, double count,
+    int64_t t_prune, int update_magnitude, int refresh_mask, int64_t k, int bits, int64_t t_quant,
+    int update_scale, double *abssum_out, float *absmax_out, int stats_local,
+    int64_t *step_counter_dev, uint64_t *timing_out_dev, void *stream) {
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    return reduce_prune_quant_step_impl(static_cast<const T *>(x), outer, channels, inner, workspace,
+                                        workspace_bytes, arrival_counter_dev, magnitude, mask, scale, decimal_out,
+                                        group, step_stamp, count, t_prune, update_magnitude, refresh_mask, k, bits,
+                                        t_quant, update_scale, abssum_out, absmax_out, stats_local,
+                                        step_counter_dev, timing_out_dev, stream);
+  });
+}
+
+extern "C" int qsb_reduce_prune_quant_step(
+    const float *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+    int64_t workspace_bytes, unsigned int *arrival_counter_dev, float *magnitude, uint8_t *mask,
+    float *scale, float *decimal_out, qsb_p2p_group *group, int64_t step_stamp, double count,
+    int64_t t_prune, int update_magnitude, int refresh_mask, int64_t k, int bits, int64_t t_quant,
+    int update_scale, double *abssum_out, float *absmax_out, int stats_local,
+    int64_t *step_counter_dev, uint64_t *timing_out_dev, void *stream) {
+  return reduce_prune_quant_step_impl(x, outer, channels, inner, workspace, workspace_bytes, arrival_counter_dev,
+                                      magnitude, mask, scale, decimal_out, group, step_stamp, count, t_prune,
+                                      update_magnitude, refresh_mask, k, bits, t_quant, update_scale, abssum_out,
+                                      absmax_out, stats_local, step_counter_dev, timing_out_dev, stream);
 }

@@ -34,7 +34,9 @@ void set_reduce_col_tpr_wide(int v);
 void set_reduce_row_variant(int v);
 void set_reduce_keep_hint(int v);
 void set_reduce_col_max_inner(int v);
-ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner, const float *x);
+// x (element size x_bytes) only decides the column kernel's vector width; the plan's partial layout and
+// summation order depend on the shape alone
+ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner, const void *x, int x_bytes = 4);
 int64_t partial_bytes(int64_t n);
 // carve the five partial arrays out of a caller workspace (256-byte aligned)
 Partials partials_from_workspace(void *workspace, int64_t n_partials);

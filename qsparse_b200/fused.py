@@ -36,11 +36,12 @@ class _PruneQuantizeFn(torch.autograd.Function):
     def forward(ctx, x, layer):
         ctx.layer = layer
         ctx.layout = layer._layout(x)
+        ctx.x_dtype = N.as_native(x).dtype
         return layer._forward_impl(x, ctx.layout)
 
     @staticmethod
     def backward(ctx, grad_output):
-        return ctx.layer.backward_kernel(grad_output, ctx.layout), None
+        return ctx.layer.backward_kernel(grad_output, ctx.layout, ctx.x_dtype), None
 
 
 class PruneQuantize(nn.Module):
@@ -96,7 +97,7 @@ class PruneQuantize(nn.Module):
 
     def _forward_impl(self, x, layout):
         outer, ch, inner = layout
-        xs = N.as_f32_contiguous(x.detach())
+        xs = N.as_native_contiguous(x.detach())   # bf16 / fp16 read natively, y is fp32
         if self._exchange is None:
             self._allocate(xs, ch)
         if self.training:
@@ -145,10 +146,11 @@ class PruneQuantize(nn.Module):
             self.t_quant += 1
         return ops.fq_pow2_fwd(xs, self.decimal, layout, mask=self.mask.data)
 
-    def backward_kernel(self, g, layout):
+    def backward_kernel(self, g, layout, x_dtype=torch.float32):
+        """gx in ``x_dtype`` (the input's dtype: bf16 / fp16 are written directly, rounded like autograd's cast)"""
         g = N.as_f32_contiguous(g)
         _, gx = ops.ste_bwd(g, self.decimal, True, self.bits, 0, layout, mask=self.mask.data,
-                            clamp_in_place=self.mutate_grad_output, want_gx=True)
+                            clamp_in_place=self.mutate_grad_output, want_gx=True, gx_dtype=x_dtype)
         return gx
 
     def forward(self, x):
@@ -167,6 +169,7 @@ class _FusedLayersFn(torch.autograd.Function):
         # param: the step's decimal (DecimalQuantizer) or the layer's scale itself (ScalerQuantizer)
         ctx.layout, ctx.mask, ctx.param, ctx.bits, ctx.notch = layout, mask, param, bits, notch
         ctx.is_decimal = is_decimal
+        ctx.x_dtype = xs.dtype     # bf16 / fp16 activations: gx is written in their dtype
         if is_decimal:
             return ops.fq_pow2_fwd(xs, param, layout, mask=mask).view(x.shape)
         return ops.fq_scaler_fwd(xs, param, layout, mask=mask).view(x.shape)
@@ -179,7 +182,7 @@ class _FusedLayersFn(torch.autograd.Function):
         if not g.is_contiguous():
             g = g.contiguous()
         _, gx = ops.ste_bwd(g, ctx.param, ctx.is_decimal, ctx.bits, ctx.notch, ctx.layout, mask=ctx.mask,
-                            clamp_in_place=True, want_gx=True)
+                            clamp_in_place=True, want_gx=True, gx_dtype=ctx.x_dtype)
         return (gx,) + (None,) * 7
 
 
@@ -244,7 +247,7 @@ class FusedPruneQuantSequential(nn.Sequential):
         cb, qcb = p.callback, q.callback
         layout = N.channel_layout(x.shape, 1)
         outer, ch, inner = layout
-        xs = N.as_f32_contiguous(x.detach())
+        xs = N.as_native_contiguous(x.detach())   # bf16 / fp16 read natively
         sparsity = p._s_mirror.get(p._cur_sparsity)
         t = cb._t()
         refresh = (t % cb.mask_refresh_interval == 0 and t <= cb.stop_mask_refresh) and \

@@ -112,27 +112,33 @@ def invert_perm(perm):
 
 
 # ----------------------------------------------------------------------------- K1
+def _f32_like(x):
+    """the fp32 output of a fake-quantizer (also for a 16-bit x, SURVEY Q6), in x's memory format"""
+    return torch.empty_like(x, dtype=torch.float32)
+
+
 def fq_pow2_fwd(x, decimal, layout: Layout, mask=None, out=None):
+    """x: fp32, bf16 or fp16 (read natively); the result is fp32."""
     N.require_cuda(x, "input")
     lib = N.load_library()
-    y = torch.empty_like(x) if out is None else out
+    y = _f32_like(x) if out is None else out
     dev, n, host = _dev_param(decimal, "decimal")
     mk = _mask_kind(mask, x.numel(), layout)
-    N.check(lib.qsb_fq_pow2_fwd(N.ptr(x), N.ptr(y), N.ptr(dev), c_int64(n), c_double(host), N.ptr(mask), c_int(mk),
-                                c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]), N.stream_ptr(x.device)),
-            "qsb_fq_pow2_fwd")
+    N.check(lib.qsb_fq_pow2_fwd_dt(N.ptr(x), c_int(N.dtype_code(x)), N.ptr(y), N.ptr(dev), c_int64(n), c_double(host),
+                                   N.ptr(mask), c_int(mk), c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]),
+                                   N.stream_ptr(x.device)), "qsb_fq_pow2_fwd_dt")
     return y
 
 
 def fq_scaler_fwd(x, scaler, layout: Layout, mask=None, out=None):
     N.require_cuda(x, "input")
     lib = N.load_library()
-    y = torch.empty_like(x) if out is None else out
+    y = _f32_like(x) if out is None else out
     dev, n, host = _dev_param(scaler, "scaler")
     mk = _mask_kind(mask, x.numel(), layout)
-    N.check(lib.qsb_fq_scaler_fwd(N.ptr(x), N.ptr(y), N.ptr(dev), c_int64(n), c_float(host), N.ptr(mask), c_int(mk),
-                                  c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]), N.stream_ptr(x.device)),
-            "qsb_fq_scaler_fwd")
+    N.check(lib.qsb_fq_scaler_fwd_dt(N.ptr(x), c_int(N.dtype_code(x)), N.ptr(y), N.ptr(dev), c_int64(n),
+                                     c_float(host), N.ptr(mask), c_int(mk), c_int64(layout[0]), c_int64(layout[1]),
+                                     c_int64(layout[2]), N.stream_ptr(x.device)), "qsb_fq_scaler_fwd_dt")
     return y
 
 
@@ -140,7 +146,7 @@ def fq_line_fwd(x, lines, bits: int, float_zero_point: bool, layout: Layout, mas
     """lines: CUDA float tensor [n, 2] (n == 1 or channels) or a (lo, hi) pair."""
     N.require_cuda(x, "input")
     lib = N.load_library()
-    y = torch.empty_like(x) if out is None else out
+    y = _f32_like(x) if out is None else out
     if isinstance(lines, torch.Tensor) and lines.is_cuda:
         dev = lines.detach()
         if dev.dtype != torch.float32 or not dev.is_contiguous():
@@ -152,28 +158,29 @@ def fq_line_fwd(x, lines, bits: int, float_zero_point: bool, layout: Layout, mas
             raise RuntimeError("multi-row `lines` must be a CUDA tensor; qsparse_b200 is CUDA-only")
         dev, n, lo, hi = None, 1, float(flat[0]), float(flat[1])
     mk = _mask_kind(mask, x.numel(), layout)
-    N.check(lib.qsb_fq_line_fwd(N.ptr(x), N.ptr(y), N.ptr(dev), c_int64(n), c_float(lo), c_float(hi), c_int(bits),
-                                c_int(1 if float_zero_point else 0), N.ptr(mask), c_int(mk), c_int64(layout[0]),
-                                c_int64(layout[1]), c_int64(layout[2]), N.stream_ptr(x.device)),
-            "qsb_fq_line_fwd")
+    N.check(lib.qsb_fq_line_fwd_dt(N.ptr(x), c_int(N.dtype_code(x)), N.ptr(y), N.ptr(dev), c_int64(n), c_float(lo),
+                                   c_float(hi), c_int(bits), c_int(1 if float_zero_point else 0), N.ptr(mask),
+                                   c_int(mk), c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]),
+                                   N.stream_ptr(x.device)), "qsb_fq_line_fwd_dt")
     return y
 
 
 # ----------------------------------------------------------------------------- K2
 def ste_bwd(g, scale, is_decimal: bool, bits: int, notch: int, layout: Layout, mask=None, clamp_in_place=True,
-            want_gx=False):
+            want_gx=False, gx_dtype=torch.float32):
     """Returns (g_clamped or None, gx or None).  clamp_in_place reproduces the
-    reference's in-place `grad_output.clamp_` (quantize.py:72)."""
+    reference's in-place `grad_output.clamp_` (quantize.py:72).  gx_dtype: bf16 / fp16 writes the input
+    gradient of a 16-bit x directly in its dtype (rounded like autograd's cast of the fp32 value)."""
     N.require_cuda(g, "grad_output")
     lib = N.load_library()
     dev, n, host = _dev_param(scale, "scale")
     mk = _mask_kind(mask, g.numel(), layout)
     gc = g if clamp_in_place else None
-    gx = torch.empty_like(g) if (want_gx or not clamp_in_place) else None
-    N.check(lib.qsb_ste_bwd(N.ptr(g), N.ptr(gc), N.ptr(gx), N.ptr(dev), c_int64(n), c_double(host),
-                            c_int(1 if is_decimal else 0), c_int(bits), c_int(notch), N.ptr(mask), c_int(mk),
-                            c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]), N.stream_ptr(g.device)),
-            "qsb_ste_bwd")
+    gx = torch.empty_like(g, dtype=gx_dtype) if (want_gx or not clamp_in_place) else None
+    N.check(lib.qsb_ste_bwd_dt(N.ptr(g), N.ptr(gc), N.ptr(gx), c_int(N.NATIVE_DTYPES[gx_dtype]), N.ptr(dev),
+                               c_int64(n), c_double(host), c_int(1 if is_decimal else 0), c_int(bits), c_int(notch),
+                               N.ptr(mask), c_int(mk), c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]),
+                               N.stream_ptr(g.device)), "qsb_ste_bwd_dt")
     return gc, gx
 
 
@@ -208,13 +215,16 @@ def quant_export_int8(x, kind: int, param, bits: int, layout: Layout, pack4: boo
 
 
 # ----------------------------------------------------------------------------- K6
-def mask_apply(x, mask, layout: Layout, out=None):
+def mask_apply(x, mask, layout: Layout, out=None, out_dtype=None):
+    """``x * mask``; x and the result may differ in dtype when one of them is fp32 and the other bf16 / fp16
+    (``out_dtype``, default x's dtype)."""
     N.require_cuda(x, "input")
     lib = N.load_library()
-    y = torch.empty_like(x) if out is None else out
+    y = torch.empty_like(x, dtype=out_dtype or x.dtype) if out is None else out
     mk = _mask_kind(mask, x.numel(), layout)
-    N.check(lib.qsb_mask_apply(N.ptr(x), N.ptr(y), N.ptr(mask), c_int(mk), c_int64(layout[0]), c_int64(layout[1]),
-                               c_int64(layout[2]), N.stream_ptr(x.device)), "qsb_mask_apply")
+    N.check(lib.qsb_mask_apply_dt(N.ptr(x), c_int(N.dtype_code(x)), N.ptr(y), c_int(N.dtype_code(y)), N.ptr(mask),
+                                  c_int(mk), c_int64(layout[0]), c_int64(layout[1]), c_int64(layout[2]),
+                                  N.stream_ptr(x.device)), "qsb_mask_apply_dt")
     return y
 
 
@@ -251,17 +261,18 @@ def reduce_stats(x, layout: Layout, absmax=False, minmax=False, abssum=False, nn
         res["tensor_min"] = torch.empty(1, dtype=torch.float32, device=dev)
     nbytes = lib.qsb_reduce_workspace_bytes(c_int64(outer), c_int64(ch), c_int64(inner))
     ws = N.workspace(dev, nbytes)
-    if FUSE_REDUCE_FINALIZE:
+    if FUSE_REDUCE_FINALIZE and x.dtype == torch.float32:
         N.check(lib.qsb_reduce_stats_fused(N.ptr(x), c_int(what), c_int64(outer), c_int64(ch), c_int64(inner),
                                            N.ptr(res.get("absmax")), N.ptr(res.get("min")), N.ptr(res.get("max")),
                                            N.ptr(res.get("abssum")), N.ptr(res.get("nnz")),
                                            N.ptr(res.get("tensor_min")), N.ptr(ws), c_int64(ws.numel()),
                                            N.ptr(arrival_counter(dev)), N.stream_ptr(dev)), "qsb_reduce_stats_fused")
         return res
-    N.check(lib.qsb_reduce_stats(N.ptr(x), c_int(what), c_int64(outer), c_int64(ch), c_int64(inner),
-                                 N.ptr(res.get("absmax")), N.ptr(res.get("min")), N.ptr(res.get("max")),
-                                 N.ptr(res.get("abssum")), N.ptr(res.get("nnz")), N.ptr(res.get("tensor_min")),
-                                 N.ptr(ws), c_int64(ws.numel()), N.stream_ptr(dev)), "qsb_reduce_stats")
+    N.check(lib.qsb_reduce_stats_dt(N.ptr(x), c_int(N.dtype_code(x)), c_int(what), c_int64(outer), c_int64(ch),
+                                    c_int64(inner), N.ptr(res.get("absmax")), N.ptr(res.get("min")),
+                                    N.ptr(res.get("max")), N.ptr(res.get("abssum")), N.ptr(res.get("nnz")),
+                                    N.ptr(res.get("tensor_min")), N.ptr(ws), c_int64(ws.numel()), N.stream_ptr(dev)),
+            "qsb_reduce_stats_dt")
     return res
 
 
@@ -565,8 +576,9 @@ def reduce_partials(x, layout: Layout):
     outer, ch, inner = layout
     nbytes = lib.qsb_reduce_workspace_bytes(c_int64(outer), c_int64(ch), c_int64(inner))
     ws = N.workspace(x.device, nbytes)
-    N.check(lib.qsb_reduce_partials(N.ptr(x), c_int64(outer), c_int64(ch), c_int64(inner), N.ptr(ws),
-                                    c_int64(ws.numel()), N.stream_ptr(x.device)), "qsb_reduce_partials")
+    N.check(lib.qsb_reduce_partials_dt(N.ptr(x), c_int(N.dtype_code(x)), c_int64(outer), c_int64(ch), c_int64(inner),
+                                       N.ptr(ws), c_int64(ws.numel()), N.stream_ptr(x.device)),
+            "qsb_reduce_partials_dt")
     return ws
 
 
@@ -617,13 +629,13 @@ def reduce_prune_quant_step(x, layout: Layout, magnitude, mask, scale, decimal_o
     outer, ch, inner = layout
     nbytes = lib.qsb_reduce_workspace_bytes(c_int64(outer), c_int64(ch), c_int64(inner))
     ws = N.workspace(x.device, nbytes)
-    N.check(lib.qsb_reduce_prune_quant_step(
-        N.ptr(x), c_int64(outer), c_int64(ch), c_int64(inner), N.ptr(ws), c_int64(ws.numel()),
+    N.check(lib.qsb_reduce_prune_quant_step_dt(
+        N.ptr(x), c_int(N.dtype_code(x)), c_int64(outer), c_int64(ch), c_int64(inner), N.ptr(ws), c_int64(ws.numel()),
         N.ptr(arrival if arrival is not None else arrival_counter(x.device)), N.ptr(magnitude), N.ptr(mask), N.ptr(scale), N.ptr(decimal_out), group,
         c_int64(step_stamp), c_double(count), c_int64(t_prune), c_int(update_magnitude), c_int(int(refresh_mask)),
         c_int64(k), c_int(bits), c_int64(t_quant), c_int(1 if update_scale else 0), N.ptr(abssum_out),
         N.ptr(absmax_out), c_int(1 if stats_local else 0), N.ptr(step_counter), N.ptr(timing),
-        N.stream_ptr(x.device)), "qsb_reduce_prune_quant_step")
+        N.stream_ptr(x.device)), "qsb_reduce_prune_quant_step_dt")
 
 
 def prune_quant_rows_step_params(magnitude, mask, scale, decimal_out, stats: dict, count: float, t_prune: int,

@@ -14,8 +14,10 @@ DecimalQuantizer       ``optimize``: abs-max + EMA             qsb_reduce_stats,
 AdaptiveQuantizer      ``optimize``: min/max + EMA             qsb_reduce_stats, qsb_lines_ema
 =====================  =====================================  ==================
 
-No CPU path: CPU tensors raise.  Inputs that are not fp32 are converted to fp32
-first (the reference's output is always fp32, SURVEY Q6).
+No CPU path: CPU tensors raise.  bf16 and fp16 activations are read natively by the
+kernels, which compute in fp32: outputs are fp32 (the reference's output is always fp32,
+SURVEY Q6) and equal bit for bit what the input converted to fp32 gives; input gradients
+come back in the input's dtype.  Other dtypes are converted to fp32 first.
 """
 from __future__ import annotations
 
@@ -73,10 +75,6 @@ def _broadcast_result(y: torch.Tensor, x_shape, param) -> torch.Tensor:
     return y
 
 
-def _to_f32(x: torch.Tensor) -> torch.Tensor:
-    return x if x.dtype == torch.float32 else x.float()
-
-
 def _grad_buffer(grad_output: torch.Tensor) -> torch.Tensor:
     """The STE clamp runs in place on grad_output (quantize.py:72).  A gradient that
     is not a dense fp32 buffer (e.g. the stride-0 expand of `.sum().backward()`, on
@@ -98,7 +96,8 @@ def _ste_prepare(ctx, input, bits, param, channel_index, backward_passthrough, f
     if channelwise:
         assert len(param) == input.shape[channel_index], \
             "channel of input and decimal must be equal in channel-wise quantization"
-    x, layout = _physical_layout(_to_f32(input.detach()), channel_index, channelwise)
+    x, layout = _physical_layout(N.as_native(input.detach()), channel_index, channelwise)
+    ctx.x_dtype, ctx.x_shape = x.dtype, tuple(input.shape)
     ctx.backward_passthrough = backward_passthrough
     ctx.notch = 1 if flip_axis else 0
     ctx.bits = bits
@@ -123,6 +122,12 @@ def _ste_backward(ctx, grad_output):
     g = _grad_buffer(grad_output)
     param = ctx.saved_tensors[0] if ctx.param_is_tensor else ctx.param_host
     _, layout = _physical_layout(g, ctx.channel_index, ctx.channelwise)
+    x_dtype = getattr(ctx, "x_dtype", torch.float32)
+    if x_dtype != torch.float32 and tuple(g.shape) == ctx.x_shape:
+        # a 16-bit input: clamp grad_output in place and write its input gradient in the input's dtype, one pass
+        _, gx = ops.ste_bwd(g, param, ctx.is_decimal, ctx.bits, ctx.notch, layout, clamp_in_place=True,
+                            want_gx=True, gx_dtype=x_dtype)
+        return gx
     ops.ste_bwd(g, param, ctx.is_decimal, ctx.bits, ctx.notch, layout, clamp_in_place=True)
     return g
 
@@ -181,7 +186,7 @@ class LineQuantization(torch.autograd.Function):
             assert x.shape[channel_index] == lines.shape[0]
         assert lines.shape[1] == 2
         channelwise = channel_index >= 0 and lines.shape[0] > 1
-        xs, layout = _physical_layout(_to_f32(x.detach()), channel_index, channelwise)
+        xs, layout = _physical_layout(N.as_native(x.detach()), channel_index, channelwise)
         if lines.is_cuda:
             l = lines.detach().reshape(-1, 2)
         else:
@@ -269,6 +274,7 @@ class _TensorFusedSte(torch.autograd.Function):
             y = ops.fq_pow2_fwd(xs, decimal, layout)
         else:
             y = ops.fq_scaler_fwd(xs, weight.data.view(-1), layout)
+        ctx.x_dtype, ctx.x_shape = xs.dtype, tuple(input.shape)
         ctx.backward_passthrough = quantizer.backward_passthrough
         ctx.notch = 1 if quantizer.flip_axis else 0
         ctx.bits = bits
@@ -393,7 +399,7 @@ class DecimalQuantizer(BaseQuantizer):
                 f"{max(int(x.shape[channel_index]) // int(x.shape[0]), 1)}: channel-wise Decimal/Scaler "
                 "estimation on batched activations only works for batch size 1 in qsparse 2.0.1")
         with torch.no_grad():
-            xs = N.as_f32_contiguous(x.detach())
+            xs = N.as_native_contiguous(x.detach())
             layout = N.channel_layout(xs.shape, channel_index)
             absmax = ops.reduce_stats(xs, layout, absmax=True)["absmax"]
             if weight is None:
@@ -420,7 +426,7 @@ class DecimalQuantizer(BaseQuantizer):
                 return None
             if tuple(weight.shape) != (1, 1):
                 return None
-            return _TensorFusedSte.apply(x, self, bits, weight, N.as_f32_contiguous(x.detach()))
+            return _TensorFusedSte.apply(x, self, bits, weight, N.as_native_contiguous(x.detach()))
         xs = _row_fusable(self, exact, x, weight, channel_index)
         if xs is None:
             return None
@@ -554,7 +560,7 @@ class AdaptiveQuantizer(DecimalQuantizer):
             raise RuntimeError("view size is not compatible with input tensor's size and stride (at least one "
                                "dimension spans across two contiguous subspaces). Use .reshape(...) instead.")
         with torch.no_grad():
-            xs = N.as_f32_contiguous(x.detach())
+            xs = N.as_native_contiguous(x.detach())
             # per-(sample, channel) min/max followed by min-of-mins / max-of-maxes over the
             # batch (quantize.py:396-418) == one per-channel reduction with outer = batch
             layout = N.channel_layout(xs.shape, channel_index)

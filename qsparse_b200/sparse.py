@@ -42,12 +42,14 @@ SELECT_HINTS = True
 class _MaskApply(torch.autograd.Function):
     """``x * mask`` (ref qsparse/sparse.py:66,116,122,263) and its gradient ``g * mask``.
 
-    ``precomputed`` lets the fused mask-build+apply kernel hand in the forward value."""
+    ``precomputed`` lets the fused mask-build+apply kernel hand in the forward value.  A bf16 / fp16 ``x`` is
+    read natively; the forward value is fp32 either way and the gradient comes back in x's dtype."""
 
     @staticmethod
     def forward(ctx, x, mask, precomputed=None):
         ctx.perm = ops.mask_perm(x.shape, mask.shape)
         ctx.mask = mask  # read at backward time, like the reference's saved Parameter
+        ctx.gx_dtype = torch.float32
         if ctx.perm is not None:            # kept axes not adjacent: transpose, same kernel, transpose back
             xs, mk = _canonical(x.detach(), mask.detach(), ctx.perm)
             _, ctx.layout = ops.mask_layout(xs.shape, mk.shape)
@@ -58,8 +60,9 @@ class _MaskApply(torch.autograd.Function):
         ctx.layout = layout
         if precomputed is not None:
             return precomputed
-        xs = N.as_f32_contiguous(x.detach())
-        return ops.mask_apply(xs, mask.detach(), layout)
+        xs = N.as_native_contiguous(x.detach())
+        ctx.gx_dtype = xs.dtype
+        return ops.mask_apply(xs, mask.detach(), layout, out_dtype=torch.float32)
 
     @staticmethod
     def backward(ctx, grad_output):
@@ -67,15 +70,16 @@ class _MaskApply(torch.autograd.Function):
             g, mk = _canonical(grad_output, ctx.mask.detach(), ctx.perm)
             return ops.mask_apply(g, mk, ctx.layout).permute(ops.invert_perm(ctx.perm)), None, None
         g = N.as_f32_contiguous(grad_output)
-        return ops.mask_apply(g, ctx.mask.detach(), ctx.layout), None, None
+        return ops.mask_apply(g, ctx.mask.detach(), ctx.layout, out_dtype=ctx.gx_dtype), None, None
 
 
-def _canonical(x, like, perm):
+def _canonical(x, like, perm, native=False):
     """(x transposed so that the kept axes of ``like`` are adjacent — a contiguous fp32 copy, the permuted VIEW of
     ``like``): the view shares storage with the mask / magnitude Parameter, whose non-singleton axes keep their
-    order, so the kernels' in-place updates land in the Parameter."""
+    order, so the kernels' in-place updates land in the Parameter.  ``native``: an x that needs no transpose
+    keeps a bf16 / fp16 dtype (for the channel statistics, which read 16-bit values natively)."""
     if perm is None:
-        return N.as_f32_contiguous(x), like
+        return (N.as_native_contiguous(x) if native else N.as_f32_contiguous(x)), like
     return N.as_f32_contiguous(x.permute(perm)), like.permute(perm)
 
 
@@ -142,10 +146,11 @@ class MagnitudePruningCallback(nn.Module):
         with torch.no_grad():
             N.require_cuda(x, "x")
             mag = self.magnitude.data
-            xs, mag = _canonical(x.detach(), mag, ops.mask_perm(x.shape, mag.shape))
+            xs, mag = _canonical(x.detach(), mag, ops.mask_perm(x.shape, mag.shape), native=True)
             t = self._t()
             kind, layout = ops.mask_layout(xs.shape, mag.shape)
             if kind == "element":
+                xs = N.as_f32_contiguous(xs)   # the full-size EMA reads fp32
                 tensor_min = None
                 if self.l0:  # `x.min() == 0` gate (sparse.py:85), evaluated on the device
                     tensor_min = ops.reduce_stats(xs, (1, 1, xs.numel()), nnz=True)["tensor_min"]
@@ -160,8 +165,10 @@ class MagnitudePruningCallback(nn.Module):
         N.require_cuda(x, "x")
         with torch.no_grad():
             perm = ops.mask_perm(x.shape, mask.shape)
-            xs, mask_c = _canonical(x.detach(), mask.data, perm)
+            xs, mask_c = _canonical(x.detach(), mask.data, perm, native=True)
             kind, layout = ops.mask_layout(xs.shape, mask_c.shape)
+            if kind == "element":
+                xs = N.as_f32_contiguous(xs)   # the element select / mask build read fp32
             n = mask.numel()
             k = kth_rank(sparsity, n)
             if k >= n:
@@ -233,7 +240,7 @@ class MagnitudePruningCallback(nn.Module):
         if kind != "channel" or ch != mask.numel() or ch < 2 or ch > 2048 or outer * inner < 64:
             return None
         with torch.no_grad():
-            xs = N.as_f32_contiguous(x.detach())
+            xs = N.as_native_contiguous(x.detach())
             k = kth_rank(sparsity, ch) if refresh else 0
             if refresh and k >= ch:
                 raise IndexError(f"index {k} is out of bounds for dimension 0 with size {ch}")
