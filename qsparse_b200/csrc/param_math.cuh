@@ -27,6 +27,12 @@ __device__ __forceinline__ float scale_to_decimal(float s) {
   return rintf(l);
 }
 
+// What a PRUNED channel with max|x| bits `b` adds to the abs-max of `x * mask` (ref sparse.py:66,
+// quantize.py:329-340): |x * 0| is 0 for finite x, but inf * 0 and NaN * 0 are NaN, which the max keeps.
+__device__ __forceinline__ uint32_t pruned_max_bits(uint32_t b) {
+  return b >= 0x7f800000u ? 0x7fffffffu : 0u;
+}
+
 // mag = (t * mag + m) / (t + 1)      ref qsparse/sparse.py:89
 __device__ __forceinline__ float magnitude_ema_step(float mag, float m,
                                                     int64_t t) {

@@ -188,14 +188,13 @@ __global__ void __launch_bounds__(1024)
   }
 
   // 3. abs-max of the pruned tensor = max over kept channels (pruned ones
-  //    contribute |0| = 0), scale EMA, decimal.
+  //    contribute |x * 0|, see pruned_max_bits), scale EMA, decimal.
   uint32_t am = 0;
   if (update_scale) {
     for (int c = tid; c < channels; c += blockDim.x) {
-      if (mask[c]) {
-        const uint32_t b = max_bits_of(c);
-        am = b > am ? b : am;
-      }
+      const uint32_t mb = max_bits_of(c);
+      const uint32_t b = mask[c] ? mb : pruned_max_bits(mb);
+      am = b > am ? b : am;
     }
     am = warp_reduce(am, [](uint32_t a, uint32_t b) { return a > b ? a : b; });
     if ((tid & 31) == 0) s_amax[tid >> 5] = am;

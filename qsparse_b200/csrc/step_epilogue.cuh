@@ -410,7 +410,10 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
     } else {
       keep = a.mask[c] != 0;
     }
-    if (keep && a.update_scale) am = sm.max[c] > am ? sm.max[c] : am;
+    if (a.update_scale) {
+      const uint32_t b = keep ? sm.max[c] : pruned_max_bits(sm.max[c]);
+      am = b > am ? b : am;
+    }
   }
   am = warp_reduce(am, [](uint32_t x, uint32_t y) { return x > y ? x : y; });
   if (lane == 0) sm.amax[warp] = am;

@@ -105,6 +105,8 @@ class PruneQuantize(nn.Module):
             refresh = (t % self.mask_refresh_interval == 0) and (t > 0 or not self.running_average)
             mode = 1 if self.running_average else 2
             k = kth_rank(self.sparsity, ch)
+            if refresh and k >= ch and not graphs.active():   # the reference indexes sorted()[k] on a refresh step
+                raise IndexError(f"index {k} is out of bounds for dimension 0 with size {ch}")
             if isinstance(self._exchange, StatExchange):
                 # NCCL fallback: finalize into the row, all-gather, combine rows in the kernel
                 graphs.require_eager("PruneQuantize over the NCCL all-gather fallback")

@@ -553,11 +553,19 @@ def mask_build_apply(importance, thr, x, mask_out, take_abs=False, out=None):
     return y
 
 
+PARAMS_KERNEL_MAX_CHANNELS = 4096   # shared-memory arrays of prune_quant_params_kernel (params.cu)
+
+
 def prune_quant_params(magnitude, mask, scale, decimal_out, stats: dict, count: float, t_prune: int,
                        update_magnitude: int, refresh_mask: bool, k: int, bits: int, t_quant: int,
                        update_scale: bool, n_rows: int = 1, row_stride_bytes: int = 0):
     """stats["abssum"] / stats["absmax"] point at row 0; further rows (ranks / chunks) follow
-    every row_stride_bytes and are combined inside the kernel in row order."""
+    every row_stride_bytes and are combined inside the kernel in row order.  Above
+    PARAMS_KERNEL_MAX_CHANNELS channels the same step runs as a sequence of launches."""
+    if mask.numel() > PARAMS_KERNEL_MAX_CHANNELS:
+        return _prune_quant_params_composed(magnitude, mask, scale, decimal_out, stats, count, t_prune,
+                                            update_magnitude, refresh_mask, k, bits, t_quant, update_scale,
+                                            n_rows, row_stride_bytes)
     lib = N.load_library()
     N.check(lib.qsb_prune_quant_params(N.ptr(magnitude), N.ptr(mask), N.ptr(scale), N.ptr(decimal_out),
                                        N.ptr(stats.get("abssum")), N.ptr(stats.get("absmax")),
@@ -566,6 +574,48 @@ def prune_quant_params(magnitude, mask, scale, decimal_out, stats: dict, count: 
                                        c_int(update_magnitude), c_int(1 if refresh_mask else 0), c_int64(k),
                                        c_int(bits), c_int64(t_quant), c_int(1 if update_scale else 0),
                                        N.stream_ptr(mask.device)), "qsb_prune_quant_params")
+
+
+def _prune_quant_params_composed(magnitude, mask, scale, decimal_out, stats, count, t_prune, update_magnitude,
+                                 refresh_mask, k, bits, t_quant, update_scale, n_rows, row_stride_bytes):
+    """``prune_quant_params`` for more channels than its one-CTA kernel holds in shared memory: the same
+    arithmetic in the same order, as magnitude EMA -> exact k-th value -> mask -> abs-max of the kept channels
+    -> scale EMA -> decimal launches."""
+    ch = mask.numel()
+    bad = (update_magnitude not in (0, 1, 2) or n_rows < 1 or (update_magnitude and not count > 0)
+           or (refresh_mask and not 0 <= k < ch))
+    if bad:
+        N.check(-1, "qsb_prune_quant_params")     # QSB_E_BADARG, as the kernel's entry point returns it
+    abssum, absmax = stats.get("abssum"), stats.get("absmax")
+    if n_rows > 1:
+        # rows of other ranks: combined in row order like the kernel (fp64 sums, NaN-propagating maxima)
+        def row(t, r):
+            off = r * row_stride_bytes
+            assert off % t.element_size() == 0
+            return torch.as_strided(t, (ch,), (1,), t.storage_offset() + off // t.element_size())
+        abssum = abssum.clone() if abssum is not None else None
+        absmax = absmax.clone() if absmax is not None else None
+        for r in range(1, n_rows):
+            if abssum is not None:
+                abssum += row(stats["abssum"], r)
+            if absmax is not None:
+                torch.maximum(absmax, row(stats["absmax"], r), out=absmax)
+    if update_magnitude == 2:
+        # this step's mean |x| itself: the EMA at t = 0 of a zeroed vector is (0 * 0 + m) / 1 = m
+        importance = torch.zeros(ch, dtype=torch.float32, device=mask.device)
+        magnitude_ema_reduced_(importance, {"abssum": abssum}, count, 0)
+    else:
+        importance = magnitude
+        if update_magnitude == 1:
+            magnitude_ema_reduced_(magnitude, {"abssum": abssum}, count, t_prune)
+    if refresh_mask:
+        mask_from_threshold(importance, kth_value(importance, k), mask)
+    if update_scale:
+        # abs-max of x * mask: a pruned channel counts |x * 0|, i.e. 0, or NaN where it holds an inf / NaN
+        kept = mask_apply(absmax, mask, (1, ch, 1))
+        scale_ema_(scale.view(-1), reduce_stats(kept, (1, 1, ch), absmax=True)["absmax"], bits, t_quant)
+    if decimal_out is not None:
+        decimal_out.view(-1).copy_(scale_to_decimal(scale.view(-1)))
 
 
 def reduce_partials(x, layout: Layout):
