@@ -500,6 +500,10 @@ int qsb_group_mean(const float *values, const int64_t *labels, float *out,
  * all-gather, or one per staged chunk of a host tensor), stat_row_stride_bytes
  * apart; they are combined in row order: SUM for abssum, MAX for absmax.
  * `count` is the number of elements per channel over ALL rows.
+ * Requires 1 <= channels <= 4096 and 1 <= n_stat_rows <= 4096.  abssum may be
+ * NULL, and `count` is not checked, when update_magnitude == 0; absmax may be
+ * NULL when update_scale == 0.  Runs the one-CTA kernel of
+ * qsb_prune_quant_rows_step_params with group == NULL.
  * ---------------------------------------------------------------------- */
 int qsb_prune_quant_params(float *magnitude, uint8_t *mask, float *scale,
                            float *decimal_out, const double *abssum,
@@ -523,7 +527,7 @@ int qsb_prune_quant_params(float *magnitude, uint8_t *mask, float *scale,
  * increase by one per step (two slots are used alternately).  `count` is the
  * number of elements per channel over ALL ranks.  abssum_out / absmax_out
  * (optional, both or neither) receive the combined statistics.
- * Requires channels <= 2048 and the same (outer, channels, inner) that was
+ * Requires channels <= 4096 and the same (outer, channels, inner) that was
  * passed to qsb_reduce_partials.
  * step_counter_dev (optional): a device int64 step index for CUDA-graph capture
  * (launch arguments of a captured graph are frozen).  When given, with t =
@@ -579,7 +583,8 @@ int qsb_prune_quant_step_params(float *magnitude, uint8_t *mask, float *scale,
 
 /* The same parameter step on FINALIZED statistics rows (as qsb_prune_quant_params takes
  * them: one row per staged chunk, combined in row order) with the peer exchange of
- * qsb_prune_quant_step_params — what the host-buffer pipeline runs at N > 1 GPUs.
+ * qsb_prune_quant_step_params — what the host-buffer pipeline runs.  Requires
+ * channels <= 4096, 1 <= n_stat_rows <= 4096 and both statistics pointers.
  * `count` is the number of elements per channel over ALL ranks. */
 int qsb_prune_quant_rows_step_params(float *magnitude, uint8_t *mask, float *scale,
                                      float *decimal_out, const double *abssum,

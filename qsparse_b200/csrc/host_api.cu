@@ -200,25 +200,18 @@ extern "C" int qsb_host_prune_quant_step_submit(
     QSB_CUDA_TRY(cudaEventRecord(sl.ev_g[i], c->s_h2d));
   }
   // ---- parameters from all chunks' statistics -------------------------------
+  // The chunk rows are summed in chunk order and, with N > 1 GPUs, exchanged with the peers over
+  // NVLink inside the same kernel and combined in rank order — the same computation as the
+  // resident path's fused step.
   {
     const double *abssum0 = reinterpret_cast<const double *>(c->d_stats);
     const float *absmax0 =
         reinterpret_cast<const float *>(c->d_stats + channels * sizeof(double));
-    if (group) {
-      // N > 1 GPUs: the chunk rows are summed in chunk order, exchanged with the peers over
-      // NVLink inside the same kernel and combined in rank order — the same computation as the
-      // resident path's fused step
-      rc = qsb_prune_quant_rows_step_params(
-          magnitude_dev, mask_dev, scale_dev, decimal_dev, abssum0, absmax0, n_chunks,
-          c->stats_row_bytes, channels, group, step_stamp,
-          (double)outer * (double)inner * (double)group->dev.world, t_prune, 1, t_prune > 0, k, bits,
-          t_quant, 1, c->s_comp);
-    } else {
-      rc = qsb_prune_quant_params(magnitude_dev, mask_dev, scale_dev, decimal_dev,
-                                  abssum0, absmax0, n_chunks, c->stats_row_bytes,
-                                  channels, (double)outer * (double)inner, t_prune,
-                                  1, t_prune > 0, k, bits, t_quant, 1, c->s_comp);
-    }
+    const double world = group ? (double)group->dev.world : 1.0;
+    rc = qsb_prune_quant_rows_step_params(
+        magnitude_dev, mask_dev, scale_dev, decimal_dev, abssum0, absmax0, n_chunks,
+        c->stats_row_bytes, channels, group, step_stamp, (double)outer * (double)inner * world, t_prune, 1,
+        t_prune > 0, k, bits, t_quant, 1, c->s_comp);
     if (rc) return rc;
   }
   // ---- forward apply per chunk, download y ---------------------------------

@@ -112,111 +112,10 @@ __global__ void __launch_bounds__(1024)
 }
 
 // ---------------------------------------------------------------------------
-// fused structured prune -> pow2 quantize parameter step (one CTA)
-// ---------------------------------------------------------------------------
-constexpr int kFusedMaxChannels = 4096;
-
-__global__ void __launch_bounds__(1024)
-    prune_quant_params_kernel(float *magnitude, uint8_t *mask, float *scale,
-                              float *decimal_out, const double *abssum,
-                              const float *absmax, int n_rows,
-                              int64_t row_stride_bytes, int channels,
-                              double count, int64_t t_prune,
-                              int update_magnitude, int refresh_mask, int64_t k,
-                              float limit, int64_t t_quant, int update_scale) {
-  __shared__ float s_imp[kFusedMaxChannels];
-  __shared__ uint32_t s_key[kFusedMaxChannels];
-  __shared__ float s_thr;
-  __shared__ uint32_t s_amax[32];
-  const int tid = threadIdx.x;
-  // statistics may arrive as several rows (one per rank / per staged chunk), each
-  // row_stride_bytes apart; they are combined here in row order (fixed order ->
-  // every rank computes bit-identical parameters).
-  auto sum_of = [&](int c) {
-    double sacc = 0.0;
-    for (int r = 0; r < n_rows; ++r)
-      sacc += *reinterpret_cast<const double *>(
-          reinterpret_cast<const char *>(abssum + c) + (int64_t)r * row_stride_bytes);
-    return sacc;
-  };
-  auto max_bits_of = [&](int c) {
-    uint32_t mb = 0;
-    for (int r = 0; r < n_rows; ++r) {
-      const float v = *reinterpret_cast<const float *>(
-          reinterpret_cast<const char *>(absmax + c) + (int64_t)r * row_stride_bytes);
-      const uint32_t b = __float_as_uint(v) & 0x7fffffffu;
-      mb = b > mb ? b : mb;
-    }
-    return mb;
-  };
-
-  // 1. importance: running-average magnitude (update_magnitude == 1), the
-  //    existing magnitude (0), or this step's mean |x| itself (2:
-  //    running_average=False, sparse.py:63-64).
-  for (int c = tid; c < channels; c += blockDim.x) {
-    float imp;
-    if (update_magnitude == 2) {
-      imp = (float)(sum_of(c) / count);
-    } else {
-      imp = magnitude[c];
-      if (update_magnitude == 1) {
-        imp = magnitude_ema_step(imp, (float)(sum_of(c) / count), t_prune);
-        magnitude[c] = imp;
-      }
-    }
-    s_imp[c] = imp;
-    s_key[c] = float_to_key(imp);
-  }
-  __syncthreads();
-
-  // 2. threshold = sorted(importance)[k]; mask = importance >= threshold
-  if (refresh_mask) {
-    for (int c = tid; c < channels; c += blockDim.x) {
-      const uint32_t kc = s_key[c];
-      int rank = 0;
-      for (int j = 0; j < channels; ++j) {
-        const uint32_t kj = s_key[j];
-        rank += (kj < kc) || (kj == kc && j < c);
-      }
-      if (rank == k) s_thr = s_imp[c];
-    }
-    __syncthreads();
-    const float thr = s_thr;
-    for (int c = tid; c < channels; c += blockDim.x)
-      mask[c] = (s_imp[c] >= thr) ? 1 : 0;
-    __syncthreads();
-  }
-
-  // 3. abs-max of the pruned tensor = max over kept channels (pruned ones
-  //    contribute |x * 0|, see pruned_max_bits), scale EMA, decimal.
-  uint32_t am = 0;
-  if (update_scale) {
-    for (int c = tid; c < channels; c += blockDim.x) {
-      const uint32_t mb = max_bits_of(c);
-      const uint32_t b = mask[c] ? mb : pruned_max_bits(mb);
-      am = b > am ? b : am;
-    }
-    am = warp_reduce(am, [](uint32_t a, uint32_t b) { return a > b ? a : b; });
-    if ((tid & 31) == 0) s_amax[tid >> 5] = am;
-  }
-  __syncthreads();
-  if (tid == 0) {
-    float s = scale[0];
-    if (update_scale) {
-      for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
-        am = s_amax[w] > am ? s_amax[w] : am;
-      s = scale_ema_step(s, __uint_as_float(am), limit, t_quant);
-      scale[0] = s;
-    }
-    if (decimal_out) decimal_out[0] = scale_to_decimal(s);
-  }
-}
-
-
-// ---------------------------------------------------------------------------
-// The parameter step as a stand-alone one-CTA launch (step_epilogue.cuh): used when the
-// statistics come as finalized rows (chunks of a host tensor), for > 1024 channels, or when
-// the caller ran qsb_reduce_partials itself.  The training step proper uses the fused form,
+// The fused structured prune -> pow2 quantize parameter step as a stand-alone one-CTA launch
+// (step_epilogue.cuh): used when the statistics come as finalized rows (reduce_stats output,
+// chunks of a host tensor, all-gathered ranks), for > 1024 channels, or when the caller ran
+// qsb_reduce_partials itself.  The training step proper uses the fused form,
 // qsb_reduce_prune_quant_step (reduce.cu), where the last CTA of the reduction does this.
 // ---------------------------------------------------------------------------
 constexpr int kStepKernelThreads = 512;  // 128 registers per thread: the batched peer poll keeps 24 packets in flight
@@ -224,16 +123,31 @@ __global__ void __launch_bounds__(kStepKernelThreads)
     prune_quant_step_kernel(const __grid_constant__ StepArgs a) {
   pdl_wait();     // the partials come from the reduction launched just before
   pdl_trigger();  // the forward kernel's CTAs may queue up behind this single CTA
-  __shared__ double s_sum[kStepMaxChannels];
-  __shared__ uint32_t s_max[kStepMaxChannels];
-  __shared__ float s_imp[kStepMaxChannels];
-  __shared__ uint32_t s_key[kStepMaxChannels];
-  __shared__ double s_psum[32];
-  __shared__ uint32_t s_pmax[32], s_amax[32];
-  __shared__ float s_thr;
-  __shared__ int s_flag;
-  const StepSmem sm{s_sum, s_max, s_imp, s_key, s_psum, s_pmax, s_amax, &s_thr, &s_flag};
-  step_epilogue(a, sm);
+  extern __shared__ __align__(16) unsigned char qsb_dyn_smem[];  // step_smem_bytes(a.channels)
+  step_epilogue(a, carve_step_smem(qsb_dyn_smem, a.channels));
+}
+
+// Above the 48 KB of dynamic shared memory any kernel may take (from ~2400 channels) the kernel needs
+// the opt-in, once per device.  cudaFuncSetAttribute is not a stream operation: it is legal while the
+// caller's stream is being captured.
+static cudaError_t step_kernel_smem_opt_in() {
+  static std::once_flag once[64];
+  static cudaError_t err[64];
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 64) dev = 0;
+  std::call_once(once[dev], [dev] {
+    err[dev] = cudaFuncSetAttribute(prune_quant_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)step_smem_bytes(kStepMaxChannels));
+  });
+  return err[dev];
+}
+
+static int launch_step_kernel(const StepArgs &a, cudaStream_t stream) {
+  const size_t smem = step_smem_bytes(a.channels);
+  if (smem > 48 * 1024) QSB_CUDA_TRY(step_kernel_smem_opt_in());
+  QSB_CUDA_TRY(launch_k(prune_quant_step_kernel, dim3(1), dim3(kStepKernelThreads), smem, stream, a));
+  return 0;
 }
 
 }  // namespace qsb
@@ -364,34 +278,29 @@ extern "C" int qsb_prune_quant_params(float *magnitude, uint8_t *mask,
                                       int refresh_mask, int64_t k, int bits,
                                       int64_t t_quant, int update_scale,
                                       void *stream) {
-  if (channels <= 0 || channels > kFusedMaxChannels) return QSB_E_UNSUPPORTED;
-  if (!mask || !scale) return QSB_E_BADARG;
-  if (update_magnitude < 0 || update_magnitude > 2) return QSB_E_BADARG;
-  if (update_magnitude != 2 && !magnitude) return QSB_E_BADARG;
+  if (channels <= 0 || channels > kStepMaxChannels) return QSB_E_UNSUPPORTED;
+  // a statistic the step does not use may be NULL here (qsb_prune_quant_rows_step_params requires both)
   if (update_magnitude && (!abssum || !(count > 0))) return QSB_E_BADARG;
   if (update_scale && !absmax) return QSB_E_BADARG;
-  if (refresh_mask && (k < 0 || k >= channels)) return QSB_E_BADARG;
   if (n_stat_rows < 1 || n_stat_rows > 4096) return QSB_E_BADARG;
-  const float limit = (float)pow(2.0, (double)bits - 1.0);
-  int threads = 32;
-  while (threads < channels && threads < 1024) threads <<= 1;
-  prune_quant_params_kernel<<<1, threads, 0, (cudaStream_t)stream>>>(
-      magnitude, mask, scale, decimal_out, abssum, absmax, (int)n_stat_rows,
-      stat_row_stride_bytes, (int)channels, count, t_prune, update_magnitude,
-      refresh_mask, k, limit, t_quant, update_scale);
-  QSB_LAUNCH_CHECK();
-  return 0;
+  StepArgs a;
+  // `count` only divides the sums of an updated magnitude: any value is accepted otherwise
+  const int rc = fill_step_args(a, magnitude, mask, scale, decimal_out, channels, nullptr, 0,
+                                update_magnitude ? count : 1.0, t_prune, update_magnitude, refresh_mask, k, bits,
+                                t_quant, update_scale, nullptr, nullptr, 0, nullptr, 1024);
+  if (rc) return rc;
+  return launch_step_kernel_on_rows(a, abssum, absmax, n_stat_rows, stat_row_stride_bytes, (cudaStream_t)stream);
 }
 
-// shared argument checks + StepArgs assembly of the three parameter-step entry points
+// shared argument checks + StepArgs assembly of the parameter-step entry points
 namespace qsb {
-int launch_step_kernel_on_rows(StepArgs a, const double *row_sum, const float *row_max, cudaStream_t stream) {
+int launch_step_kernel_on_rows(StepArgs a, const double *row_sum, const float *row_max, int64_t n_rows,
+                               int64_t row_stride, cudaStream_t stream) {
   a.row_sum = row_sum;
   a.row_max = row_max;
-  a.n_rows = 1;
-  a.row_stride = 0;
-  QSB_CUDA_TRY(launch_k(prune_quant_step_kernel, dim3(1), dim3(kStepKernelThreads), 0, stream, a));
-  return 0;
+  a.n_rows = (int)n_rows;
+  a.row_stride = row_stride;
+  return launch_step_kernel(a, stream);
 }
 
 int fill_step_args(qsb::StepArgs &a, float *magnitude, uint8_t *mask, float *scale, float *decimal_out,
@@ -456,8 +365,7 @@ extern "C" int qsb_prune_quant_step_params(
   a.P = partials_from_workspace(reduce_workspace, pl.n_partials);
   a.fin_count = (int)pl.fin_count;
   a.fin_q = (int)pl.fin_q;
-  QSB_CUDA_TRY(launch_k(prune_quant_step_kernel, dim3(1), dim3(kStepKernelThreads), 0, (cudaStream_t)stream, a));
-  return 0;
+  return launch_step_kernel(a, (cudaStream_t)stream);
 }
 
 // The same parameter step on FINALIZED statistics rows (one per staged chunk of a host
@@ -474,10 +382,5 @@ extern "C" int qsb_prune_quant_rows_step_params(
                                 t_prune, update_magnitude, refresh_mask, k, bits, t_quant, update_scale,
                                 nullptr, nullptr, 0, nullptr, 1024);
   if (rc) return rc;
-  a.row_sum = abssum;
-  a.row_max = absmax;
-  a.n_rows = (int)n_stat_rows;
-  a.row_stride = stat_row_stride_bytes;
-  QSB_CUDA_TRY(launch_k(prune_quant_step_kernel, dim3(1), dim3(kStepKernelThreads), 0, (cudaStream_t)stream, a));
-  return 0;
+  return launch_step_kernel_on_rows(a, abssum, absmax, n_stat_rows, stat_row_stride_bytes, (cudaStream_t)stream);
 }

@@ -1506,7 +1506,7 @@ static int reduce_prune_quant_step_impl(
     const int rc2 = run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, NoTail, T>(x, pl, channels, inner, P, out, stream);
     if (rc2) return rc2;
     tail.a.timing = nullptr;
-    return launch_step_kernel_on_rows(tail.a, row_sum, row_max, stream);
+    return launch_step_kernel_on_rows(tail.a, row_sum, row_max, 1, 0, stream);
   }
   tail.a.P = P;
   tail.a.fin_count = (int)pl.fin_count;

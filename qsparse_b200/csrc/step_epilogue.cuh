@@ -33,8 +33,9 @@
 
 namespace qsb {
 
-constexpr int kStepMaxChannels = 2048;      // stand-alone kernel (static shared memory)
-constexpr int kStepFusedMaxChannels = 1024; // fused tail (dynamic shared memory, 20 B / channel)
+// Both forms carve step_smem_bytes(channels) of dynamic shared memory (20 B / channel).
+constexpr int kStepMaxChannels = 4096;      // stand-alone kernel: ~82 KB, opted in above the 48 KB default
+constexpr int kStepFusedMaxChannels = 1024; // fused tail: shares the CTA with the reduction
 
 struct StepArgs {
   float *magnitude;
@@ -44,8 +45,8 @@ struct StepArgs {
   // local statistics, one of:
   Partials P;  // stage-1 partials, entry j of channel c at (j / fin_q) * (channels * fin_q) + c * fin_q + j % fin_q
   int fin_count, fin_q;
-  const double *row_sum;  // or n_rows finalized rows (chunks of a host tensor), row_stride bytes apart
-  const float *row_max;
+  const double *row_sum;  // or n_rows > 0 finalized rows (chunks of a host tensor), row_stride bytes apart;
+  const float *row_max;   // either may be NULL when the step does not use it (no magnitude / scale update)
   int n_rows;
   int64_t row_stride;
   int channels;
@@ -167,17 +168,20 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
   step_stamp_time(a, 1);
 
   // ---- 1. this GPU's statistics, fixed order ------------------------------------------
-  if (a.row_sum) {
+  if (a.n_rows) {
     for (int c = tid; c < channels; c += nthr) {
       double sum = 0.0;
       uint32_t mx = 0;
       for (int r = 0; r < a.n_rows; ++r) {
-        sum += *reinterpret_cast<const double *>(reinterpret_cast<const char *>(a.row_sum + c) +
-                                                 (int64_t)r * a.row_stride);
-        const float v = *reinterpret_cast<const float *>(reinterpret_cast<const char *>(a.row_max + c) +
-                                                         (int64_t)r * a.row_stride);
-        const uint32_t b = __float_as_uint(v) & 0x7fffffffu;
-        mx = b > mx ? b : mx;
+        if (a.row_sum)
+          sum += *reinterpret_cast<const double *>(reinterpret_cast<const char *>(a.row_sum + c) +
+                                                   (int64_t)r * a.row_stride);
+        if (a.row_max) {
+          const float v = *reinterpret_cast<const float *>(reinterpret_cast<const char *>(a.row_max + c) +
+                                                           (int64_t)r * a.row_stride);
+          const uint32_t b = __float_as_uint(v) & 0x7fffffffu;
+          mx = b > mx ? b : mx;
+        }
       }
       sm.sum[c] = sum;
       sm.max[c] = mx;
@@ -438,8 +442,9 @@ int fill_step_args(StepArgs &a, float *magnitude, uint8_t *mask, float *scale, f
                    int update_scale, double *abssum_out, float *absmax_out, int stats_local,
                    int64_t *step_counter_dev, int threads);
 
-// the stand-alone one-CTA launch of the parameter step on ONE finalized statistics row (params.cu)
-int launch_step_kernel_on_rows(StepArgs a, const double *row_sum, const float *row_max, cudaStream_t stream);
+// the stand-alone one-CTA launch of the parameter step on n_rows >= 1 finalized statistics rows (params.cu)
+int launch_step_kernel_on_rows(StepArgs a, const double *row_sum, const float *row_max, int64_t n_rows,
+                               int64_t row_stride, cudaStream_t stream);
 
 // threads per channel for a CTA of `threads` threads: the largest power of two
 // <= min(32, threads / channels); one channel: the whole CTA

@@ -90,10 +90,9 @@ class PruneQuantize(nn.Module):
         if multi:
             assert_equal_shards(x.numel() // channels, self.group)
         self._p2p = make_exchange(channels, dev, self.group, timeout_ms=self.exchange_timeout_ms) \
-            if channels <= 2048 else None
-        # NCCL all-gather path only when peer memory is unavailable (or > 2048 channels)
-        self._exchange = StatExchange(channels, dev, self.group) if (multi and self._p2p is None) or channels > 2048 \
-            else True
+            if channels <= ops.PARTIALS_ROUTE_MAX_CHANNELS else None
+        # NCCL all-gather path only when peer memory is unavailable (or takes more channels than it exchanges)
+        self._exchange = StatExchange(channels, dev, self.group) if multi and self._p2p is None else True
 
     def _forward_impl(self, x, layout):
         outer, ch, inner = layout
@@ -123,25 +122,18 @@ class PruneQuantize(nn.Module):
                 world = self._p2p.world if self._p2p is not None else 1
                 grp = self._p2p.handle if self._p2p is not None else None
                 stamp = self._p2p.next_stamp() if self._p2p is not None else 1
+                count = float(outer * inner * world)
                 if graphs.active():
                     # graph mode: the step index (and the exchange stamp) come from a device counter that the
                     # kernel reads and advances itself
-                    if ch > ops.FUSED_STEP_MAX_CHANNELS:
-                        raise graphs.NotCapturable(f"PruneQuantize with more than {ops.FUSED_STEP_MAX_CHANNELS} channels")
-                    ops.reduce_prune_quant_step(xs, layout, self.magnitude.data, self.mask.data, self.scale.data,
-                                                self.decimal, float(outer * inner * world), 0, mode,
-                                                self.mask_refresh_interval, k, self.bits, self.t_quant - t, True,
-                                                group=grp, step_counter=self._step_counter(xs.device))
-                elif ch <= ops.FUSED_STEP_MAX_CHANNELS:
-                    # ONE kernel: reduction whose last CTA finalizes, exchanges and derives the parameters
-                    ops.reduce_prune_quant_step(xs, layout, self.magnitude.data, self.mask.data, self.scale.data,
-                                                self.decimal, float(outer * inner * world), t, mode, refresh, k,
-                                                self.bits, self.t_quant, True, group=grp, step_stamp=stamp)
+                    ops.structured_prune_quant_step(xs, layout, self.magnitude.data, self.mask.data, self.scale.data,
+                                                    self.decimal, count, 0, mode, self.mask_refresh_interval, k,
+                                                    self.bits, self.t_quant - t, True, group=grp,
+                                                    step_counter=self._step_counter(xs.device))
                 else:
-                    ws = ops.reduce_partials(xs, layout)
-                    ops.prune_quant_step_params(self.magnitude.data, self.mask.data, self.scale.data, self.decimal,
-                                                ws, layout, float(outer * inner * world), t, mode, refresh, k,
-                                                self.bits, self.t_quant, True, group=grp, step_stamp=stamp)
+                    ops.structured_prune_quant_step(xs, layout, self.magnitude.data, self.mask.data, self.scale.data,
+                                                    self.decimal, count, t, mode, refresh, k, self.bits,
+                                                    self.t_quant, True, group=grp, step_stamp=stamp)
                 if self._p2p is not None and t % self.check_every == 0 and not graphs.active():
                     self._p2p.check()     # raises when an earlier step timed out waiting for a peer
             self.t_prune += 1
@@ -226,7 +218,7 @@ class FusedPruneQuantSequential(nn.Sequential):
             return False
         if p.dimensions != {1} or not p.initted or not q.initted or p.mask.numel() == 1:
             return False
-        if p.mask.numel() != x.shape[1] or p.mask.numel() > 2048:
+        if p.mask.numel() != x.shape[1] or p.mask.numel() > ops.PARTIALS_ROUTE_MAX_CHANNELS:
             return False
         n = p._n_mirror.get(p._n_updates)
         if n < p.start or n in p.schedules:
@@ -271,21 +263,16 @@ class FusedPruneQuantSequential(nn.Sequential):
             if graphs.active():
                 # graph mode: the step index is the prune callback's own `t` Parameter, read and advanced by the
                 # kernel; the quantizer's EMA index keeps its constant distance to it
-                if ch > ops.FUSED_STEP_MAX_CHANNELS or cb.stop_mask_refresh != float("inf"):
-                    raise graphs.NotCapturable("a fused site with more than "
-                                               f"{ops.FUSED_STEP_MAX_CHANNELS} channels or a stopping mask refresh")
-                ops.reduce_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data.view(-1),
-                                            decimal, float(outer * inner), 0, mode, cb.mask_refresh_interval,
-                                            kth_rank(sparsity, ch), q.bits, qcb.t - t, True,
-                                            step_counter=graphs.callback_counter(cb, x.device))
-            elif ch <= ops.FUSED_STEP_MAX_CHANNELS:
-                ops.reduce_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data.view(-1),
-                                            decimal, float(outer * inner), t, mode, refresh, k, q.bits, qcb.t, True)
-                cb.t.data.add_(1)
+                if cb.stop_mask_refresh != float("inf"):
+                    raise graphs.NotCapturable("a fused site with a stopping mask refresh")
+                ops.structured_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data.view(-1),
+                                                decimal, float(outer * inner), 0, mode, cb.mask_refresh_interval,
+                                                kth_rank(sparsity, ch), q.bits, qcb.t - t, True,
+                                                step_counter=graphs.callback_counter(cb, x.device))
             else:
-                ws = ops.reduce_partials(xs, layout)
-                ops.prune_quant_step_params(magnitude, p.mask.data.view(-1), q.weight.data.view(-1), decimal, ws,
-                                            layout, float(outer * inner), t, mode, refresh, k, q.bits, qcb.t, True)
+                ops.structured_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data.view(-1),
+                                                decimal, float(outer * inner), t, mode, refresh, k, q.bits, qcb.t,
+                                                True)
                 cb.t.data.add_(1)
             # the counters of the two layers and their callbacks, as their own forwards advance them
             cb._t_mirror.wrote(cb.t, t + 1)

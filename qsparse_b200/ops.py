@@ -12,6 +12,7 @@ from typing import Optional, Sequence, Tuple
 import torch
 
 from . import _native as N
+from . import graphs
 
 Layout = Tuple[int, int, int]
 
@@ -553,7 +554,12 @@ def mask_build_apply(importance, thr, x, mask_out, take_abs=False, out=None):
     return y
 
 
-PARAMS_KERNEL_MAX_CHANNELS = 4096   # shared-memory arrays of prune_quant_params_kernel (params.cu)
+FUSED_STEP_MAX_CHANNELS = 1024      # the reduction's last CTA runs the step (kStepFusedMaxChannels)
+STEP_KERNEL_MAX_CHANNELS = 4096     # the one-CTA step kernel's shared memory (kStepMaxChannels, step_epilogue.cuh)
+# A route choice, not a kernel limit: up to here the step kernel finalizes the reduction's partials itself (and
+# runs the peer exchange); above it the statistics are finalized first.  Moving it changes which launch sequence
+# runs for 2049-4096 channels, which has not been measured.
+PARTIALS_ROUTE_MAX_CHANNELS = 2048
 
 
 def prune_quant_params(magnitude, mask, scale, decimal_out, stats: dict, count: float, t_prune: int,
@@ -561,8 +567,8 @@ def prune_quant_params(magnitude, mask, scale, decimal_out, stats: dict, count: 
                        update_scale: bool, n_rows: int = 1, row_stride_bytes: int = 0):
     """stats["abssum"] / stats["absmax"] point at row 0; further rows (ranks / chunks) follow
     every row_stride_bytes and are combined inside the kernel in row order.  Above
-    PARAMS_KERNEL_MAX_CHANNELS channels the same step runs as a sequence of launches."""
-    if mask.numel() > PARAMS_KERNEL_MAX_CHANNELS:
+    STEP_KERNEL_MAX_CHANNELS channels the same step runs as a sequence of launches."""
+    if mask.numel() > STEP_KERNEL_MAX_CHANNELS:
         return _prune_quant_params_composed(magnitude, mask, scale, decimal_out, stats, count, t_prune,
                                             update_magnitude, refresh_mask, k, bits, t_quant, update_scale,
                                             n_rows, row_stride_bytes)
@@ -648,8 +654,6 @@ def prune_quant_step_params(magnitude, mask, scale, decimal_out, workspace, layo
         N.ptr(step_counter), N.stream_ptr(mask.device)), "qsb_prune_quant_step_params")
 
 
-FUSED_STEP_MAX_CHANNELS = 1024
-
 _arrival_counters = {}
 
 
@@ -686,6 +690,37 @@ def reduce_prune_quant_step(x, layout: Layout, magnitude, mask, scale, decimal_o
         c_int64(k), c_int(bits), c_int64(t_quant), c_int(1 if update_scale else 0), N.ptr(abssum_out),
         N.ptr(absmax_out), c_int(1 if stats_local else 0), N.ptr(step_counter), N.ptr(timing),
         N.stream_ptr(x.device)), "qsb_reduce_prune_quant_step_dt")
+
+
+def structured_prune_quant_step(x, layout: Layout, magnitude, mask, scale, decimal_out, count: float, t_prune: int,
+                                update_magnitude: int, refresh_mask, k: int, bits: int, t_quant: int,
+                                update_scale: bool, group=None, step_stamp: int = 1, step_counter=None):
+    """The structured prune -> pow2 quantize parameter step on x, by channel count:
+
+      <= FUSED_STEP_MAX_CHANNELS      reduce_prune_quant_step (one launch)
+      <= PARTIALS_ROUTE_MAX_CHANNELS  reduce_partials + prune_quant_step_params
+      otherwise                       reduce_stats + prune_quant_params (single GPU only)
+
+    Arguments as in ``reduce_prune_quant_step``.  ``step_counter`` (CUDA graphs) is taken by the one-launch
+    route only: with more channels this raises ``graphs.NotCapturable``."""
+    ch = layout[1]
+    if ch <= FUSED_STEP_MAX_CHANNELS:
+        reduce_prune_quant_step(x, layout, magnitude, mask, scale, decimal_out, count, t_prune, update_magnitude,
+                                refresh_mask, k, bits, t_quant, update_scale, group=group, step_stamp=step_stamp,
+                                step_counter=step_counter)
+    elif step_counter is not None:
+        raise graphs.NotCapturable(f"the structured prune -> quantize step with more than {FUSED_STEP_MAX_CHANNELS} "
+                                   "channels")
+    elif ch <= PARTIALS_ROUTE_MAX_CHANNELS:
+        ws = reduce_partials(x, layout)
+        prune_quant_step_params(magnitude, mask, scale, decimal_out, ws, layout, count, t_prune, update_magnitude,
+                                refresh_mask, k, bits, t_quant, update_scale, group=group, step_stamp=step_stamp)
+    elif group is not None:
+        raise ValueError(f"the peer exchange takes at most {PARTIALS_ROUTE_MAX_CHANNELS} channels")
+    else:
+        stats = reduce_stats(x, layout, absmax=True, abssum=True)
+        prune_quant_params(magnitude, mask, scale, decimal_out, stats, count, t_prune, update_magnitude,
+                           refresh_mask, k, bits, t_quant, update_scale)
 
 
 def prune_quant_rows_step_params(magnitude, mask, scale, decimal_out, stats: dict, count: float, t_prune: int,

@@ -237,7 +237,8 @@ class MagnitudePruningCallback(nn.Module):
             return None                                   # non-adjacent kept axes: the transposing route
         kind, layout = ops.mask_layout(x.shape, mask.shape)
         outer, ch, inner = layout
-        if kind != "channel" or ch != mask.numel() or ch < 2 or ch > 2048 or outer * inner < 64:
+        if (kind != "channel" or ch != mask.numel() or ch < 2 or ch > ops.PARTIALS_ROUTE_MAX_CHANNELS
+                or outer * inner < 64):
             return None
         with torch.no_grad():
             xs = N.as_native_contiguous(x.detach())
@@ -252,18 +253,12 @@ class MagnitudePruningCallback(nn.Module):
             if counter is not None:
                 # graph mode: the kernel reads the step index from `counter` (the callback's own `t` Parameter),
                 # derives the refresh gate from it and advances it
-                if ch > ops.FUSED_STEP_MAX_CHANNELS:
-                    return None
-                ops.reduce_prune_quant_step(xs, layout, magnitude, mask.data.view(-1), dummy, None,
-                                            float(outer * inner), 0, mode, self.mask_refresh_interval,
-                                            kth_rank(sparsity, ch), 8, 0, False, step_counter=counter)
-            elif ch <= ops.FUSED_STEP_MAX_CHANNELS:
-                ops.reduce_prune_quant_step(xs, layout, magnitude, mask.data.view(-1), dummy, None,
-                                            float(outer * inner), t, mode, refresh, k, 8, 0, False)
+                ops.structured_prune_quant_step(xs, layout, magnitude, mask.data.view(-1), dummy, None,
+                                                float(outer * inner), 0, mode, self.mask_refresh_interval,
+                                                kth_rank(sparsity, ch), 8, 0, False, step_counter=counter)
             else:
-                ws = ops.reduce_partials(xs, layout)
-                ops.prune_quant_step_params(magnitude, mask.data.view(-1), dummy, None, ws, layout,
-                                            float(outer * inner), t, mode, refresh, k, 8, 0, False)
+                ops.structured_prune_quant_step(xs, layout, magnitude, mask.data.view(-1), dummy, None,
+                                                float(outer * inner), t, mode, refresh, k, 8, 0, False)
         return apply_mask(x, mask)
 
     def forward(self, x: torch.Tensor, sparsity: float, mask: torch.Tensor, name=""):

@@ -43,6 +43,17 @@ def test_argument_errors_without_gpu():
     assert lib.qsb_fq_pow2_fwd(null, null, null, 1, 5.0, null, 0, 1, 1, 8, null) == -1    # null pointers
     assert lib.qsb_kth_value(null, 0, 0, 0, null, null, 0, null) == -1
     assert lib.qsb_mask_apply(null, null, null, 0, 1, 1, 1, null) == -1                   # mask_kind none
+    # the structured prune -> quantize parameter step on statistics rows: host buffers, never dereferenced
+    c = 8
+    mag, amax, scale, dec = ((ctypes.c_float * c)() for _ in range(4))
+    mask, asum = (ctypes.c_uint8 * c)(), (ctypes.c_double * c)()
+
+    def params(channels, n_rows=1, k=2, refresh=1):
+        return lib.qsb_prune_quant_params(mag, mask, scale, dec, asum, amax, n_rows, 0, channels, 64.0, 1, 1,
+                                          refresh, k, 8, 1, 1, null)
+    assert params(0) == -4 and params(4097) == -4                                       # QSB_E_UNSUPPORTED
+    assert params(c, n_rows=0) == -1
+    assert params(c, k=c) == -1 and params(c, k=-1) == -1                               # k outside [0, C) on a refresh
 
 
 def test_product_fails_loudly_on_cpu_tensors():

@@ -6,8 +6,11 @@ channel count:
   one       C <= 1024, C * fin_count <= 12288   stage 1 whose last-arriving CTA runs the step (step_epilogue.cuh)
   three     C <= 1024, C * fin_count >  12288   stage 1 -> parallel finalize -> prune_quant_step_kernel
   partials  1024 < C <= 2048                    reduce_partials + prune_quant_step_kernel
-  params    2048 < C <= 4096                    reduce_stats + prune_quant_params_kernel
+  params    2048 < C <= 4096                    reduce_stats (stage 1 -> finalize) + prune_quant_step_kernel on rows
   composed  C > 4096                            reduce_stats + EMA / k-th value / mask / abs-max / scale launches
+
+(ops.structured_prune_quant_step picks among one, partials, params and composed by C; the partials entry point
+itself takes up to 4096 channels, and the table covers that too.)
 
 Every case names the route and the stage-1 kernel it is meant to reach, and a profiler recording of one step checks
 that it does, so a dispatch change fails here instead of leaving a route untested.  The reference is the oracle's
@@ -226,16 +229,17 @@ CASES = [
     ("f32-rows4-offset", (4, 32, 323), (4, 32, 323), "one", "rows4", F32, True, TIES),
 ]
 # channel counts at the steps of the tail's threads per channel (32 ... 1 at C = 9, 17, 33, 65, 129, 257) and at
-# the route limits, as [16, C] with the channel last (column mode)
+# the route limits, as [16, C] with the channel last (column mode); the partials entry point up to its own limit
 for _c, _route in [(2, "one"), (8, "one"), (9, "one"), (16, "one"), (17, "one"), (33, "one"), (65, "one"),
                    (129, "one"), (256, "one"), (257, "one"), (1000, "one"), (1024, "one"), (1025, "partials"),
-                   (2048, "partials"), (2049, "params"), (4096, "params")]:
-    CASES.append((f"C{_c}", (16, _c), (16, _c, 1), _route, "cols4" if _c % 4 == 0 else "cols1", F32, False,
+                   (2048, "partials"), (2049, "params"), (4096, "params"), (2049, "partials"), (4096, "partials")]:
+    _id = f"C{_c}-{_route}" if _c > 2048 else f"C{_c}"     # above 2048 channels both routes are covered
+    CASES.append((_id, (16, _c), (16, _c, 1), _route, "cols4" if _c % 4 == 0 else "cols1", F32, False,
                   FULL if _c in (9, 257, 1024, 1025, 2049, 4096) else TIES))
 # more channels than the fused tail holds, in row mode (the partials / params routes read row-mode partials too)
 CASES += [
     ("C1025-rows4", (2, 1025, 320), (2, 1025, 320), "partials", "rows4", F32, False, TIES),
-    ("C2049-rows4", (2, 2049, 320), (2, 2049, 320), "params", "rows4", F32, False, TIES),
+    ("C2049-rows4-params", (2, 2049, 320), (2, 2049, 320), "params", "rows4", F32, False, TIES),
     ("C2048-bf16-offset", (16, 2048), (16, 2048, 1), "partials", "cols1", BF16, True, TIES),
 ]
 
@@ -252,7 +256,7 @@ ROUTE_KERNELS = {
     "one": ([r"StepTail"], 1),
     "three": ([r"prune_quant_step_kernel", r"reduce_finalize"], 3),
     "partials": ([r"prune_quant_step_kernel"], 2),
-    "params": ([r"prune_quant_params_kernel", r"reduce_finalize"], 3),
+    "params": ([r"prune_quant_step_kernel", r"reduce_finalize"], 3),
 }
 
 
@@ -277,10 +281,10 @@ def check_route(route, stage1, names, what):
     assert any(re.search(STAGE1[stage1], n) for n in names), (what, stage1, names)
     for pat in extra:
         assert any(re.search(pat, n) for n in names), (what, pat, names)
-    if route != "params":
-        assert not any("prune_quant_params_kernel" in n for n in names), (what, names)
-    if route not in ("three", "partials"):
+    if route == "one":
         assert not any("prune_quant_step_kernel" in n for n in names), (what, names)
+    if route == "partials":
+        assert not any("reduce_finalize" in n for n in names), (what, names)
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
@@ -339,6 +343,33 @@ def test_sparsity_one_is_rejected_without_writing(route, layout):
     assert torch.equal(st.mask, before)
     with pytest.raises(IndexError):
         orc.mask_given_importance(np.arange(c, dtype=np.float32), 1.0)
+
+
+@pytest.mark.parametrize("c", [64, 2049, 4096, 4097])
+def test_params_takes_no_statistics_it_does_not_use(c):
+    """prune_quant_params with the magnitude kept (update_magnitude 0) takes no abssum and any count, and without a
+    scale update no absmax: the mask then comes from the stored magnitude (ties included), the scale stays"""
+    from qsparse_b200 import ops
+    st = State(c)
+    mag = np.abs(make_x((1, c, 1), "dup", 5, 0.5).reshape(-1))
+    st.mag.copy_(torch.from_numpy(mag))
+    st.scale.fill_(3.0)
+    k = _k(0.5, c)
+    ops.prune_quant_params(st.mag, st.mask, st.scale, st.dec, {}, 0.0, 1, 0, True, k, BITS, 1, False)
+    mask, _ = orc.mask_given_importance(mag, 0.5)
+    scale = np.array([3.0], np.float32)
+    assert np.array_equal(st.mask.cpu().numpy(), mask.astype(bool))
+    assert bits_equal(st.mag.cpu().numpy(), mag)
+    assert bits_equal(st.scale.cpu().numpy(), scale)
+    assert bits_equal(st.dec.cpu().numpy(), orc.scale_to_decimal(scale))
+    # the scale update on the stored mask, from absmax alone
+    amax = np.abs(make_x((1, c, 1), "rand", 6, 0.5).reshape(-1))
+    ops.prune_quant_params(st.mag, st.mask, st.scale, st.dec, {"absmax": torch.from_numpy(amax).cuda()}, 0.0, 1, 0,
+                           False, k, BITS, 1, True)
+    scale = orc.scale_ema(scale, np.array([np.max(amax * mask)], np.float32), BITS, 1)
+    assert np.array_equal(st.mask.cpu().numpy(), mask.astype(bool))
+    assert bits_equal(st.scale.cpu().numpy(), scale)
+    assert bits_equal(st.dec.cpu().numpy(), orc.scale_to_decimal(scale))
 
 
 # ----------------------------------------------------------------------------- module level
