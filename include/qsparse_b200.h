@@ -641,6 +641,57 @@ int qsb_reduce_prune_quant_step_dt(const void *x, int x_dtype, int64_t outer, in
                                    uint64_t *timing_out_dev, void *stream);
 
 /* ------------------------------------------------------------------------
+ * The line form of the structured prune -> quantize step, for an AdaptiveQuantizer
+ * (ref sparse.py:58-66,82-89 + util.py:79-117 + quantize.py:396-430): the same
+ * statistics reduction, finalize, magnitude EMA, threshold and mask as
+ * qsb_reduce_prune_quant_step (same plan, same summation order of sum|x|), then
+ * in place of abs-max -> scale -> decimal the (min, max) of x * mask and the
+ * lines EMA  lines = (lines * (t - 1) + new) / t  at the quantizer's 1-based call
+ * index t = t_line (t = 1 writes `new`, as qsb_lines_ema does).  A pruned channel
+ * adds min / max of x * 0: +-0 (the sign that min / max of the fp32 output of
+ * qsb_mask_apply_dt has), or NaN when it holds an inf or a NaN.
+ *   lines [n_lines, 2] (lo, hi): n_lines == 1 takes the NaN-propagating min / max
+ *   over all channels (per tensor), n_lines == channels each channel's own pair.
+ * Then qsb_fq_line_fwd_dt(mask, float_zero_point = 1) and qsb_mask_apply_dt(g).
+ * abssum_out / min_out / max_out (optional, each may be NULL) receive this step's
+ * sum|x|, min x and max x per channel (of x, not of x * mask).
+ * step_counter_dev (optional) as in qsb_prune_quant_step_params; the call index is
+ * then *step_counter_dev + t_line (t_line an offset) and the kernel advances the
+ * counter.  Without it t_line must be >= 1.
+ * Returns QSB_E_BADARG before any CUDA call for NULL x / workspace / arrival
+ * counter / mask / lines, n_lines not 1 or channels, t_line < 1 without a counter,
+ * k outside [0, channels) on a refresh, a bad update_magnitude or count, or any
+ * group (the line form runs on one GPU: group must be NULL).
+ *
+ * qsb_reduce_prune_line_step_dt: ONE launch (as qsb_reduce_prune_quant_step_dt,
+ * also its three-launch form for wide column-mode tensors).  Requires channels <=
+ * 1024 (QSB_E_UNSUPPORTED above).  No L2 residency hint: the line forward reads
+ * the pruned channels too.
+ * ---------------------------------------------------------------------- */
+int qsb_reduce_prune_line_step_dt(const void *x, int x_dtype, int64_t outer, int64_t channels,
+                                  int64_t inner, void *workspace, int64_t workspace_bytes,
+                                  unsigned int *arrival_counter_dev, float *magnitude,
+                                  uint8_t *mask, float *lines, int64_t n_lines,
+                                  qsb_p2p_group *group, double count, int64_t t_prune,
+                                  int update_magnitude, int refresh_mask, int64_t k,
+                                  int64_t t_line, double *abssum_out, float *min_out,
+                                  float *max_out, int64_t *step_counter_dev, void *stream);
+/* Stage 1 of sum|x| and min / max x only (plan and summation order as qsb_reduce_partials_dt);
+ * the partials stay in the workspace for qsb_prune_line_step_params. */
+int qsb_reduce_line_partials_dt(const void *x, int x_dtype, int64_t outer, int64_t channels,
+                                int64_t inner, void *workspace, int64_t workspace_bytes,
+                                void *stream);
+/* The line step as a one-CTA launch on the partials of qsb_reduce_line_partials_dt (same
+ * outer, channels, inner).  Requires channels <= 2048 (QSB_E_UNSUPPORTED above). */
+int qsb_prune_line_step_params(float *magnitude, uint8_t *mask, float *lines, int64_t n_lines,
+                               void *reduce_workspace, int64_t workspace_bytes, int64_t outer,
+                               int64_t channels, int64_t inner, qsb_p2p_group *group,
+                               double count, int64_t t_prune, int update_magnitude,
+                               int refresh_mask, int64_t k, int64_t t_line,
+                               double *abssum_out, float *min_out, float *max_out,
+                               int64_t *step_counter_dev, void *stream);
+
+/* ------------------------------------------------------------------------
  * Host-buffer entry points (what a host-side caller that keeps its tensors in
  * CPU memory binds to).  They stage through pinned memory owned by a context,
  * pipeline H2D / kernels / D2H over chunks on several streams, and return after

@@ -54,6 +54,12 @@ _SIGNATURES = {
     "qsb_reduce_prune_quant_step_dt": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, c_int64, _P, _P, _P, _P, _P,
                                                _P, c_int64, c_double, c_int64, c_int, c_int, c_int64, c_int, c_int64,
                                                c_int, _P, _P, c_int, _P, _P, _P]),
+    "qsb_reduce_prune_line_step_dt": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, c_int64, _P, _P, _P, _P,
+                                              c_int64, _P, c_double, c_int64, c_int, c_int, c_int64, c_int64, _P, _P,
+                                              _P, _P, _P]),
+    "qsb_reduce_line_partials_dt": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, c_int64, _P]),
+    "qsb_prune_line_step_params": (c_int, [_P, _P, _P, c_int64, _P, c_int64, c_int64, c_int64, c_int64, _P, c_double,
+                                           c_int64, c_int, c_int, c_int64, c_int64, _P, _P, _P, _P, _P]),
     "qsb_reduce_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64]),
     "qsb_reduce_stats": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P]),
     "qsb_reduce_stats_fused": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P,

@@ -33,6 +33,24 @@ __device__ __forceinline__ uint32_t pruned_max_bits(uint32_t b) {
   return b >= 0x7f800000u ? 0x7fffffffu : 0u;
 }
 
+// What channel c of `x * mask` adds to the (min, max) of the line quantizer's statistics (ref sparse.py:66,
+// quantize.py:396-418), from the channel's own min / max of x (both NaN when it holds a NaN).  A kept channel adds
+// them unchanged.  A pruned one adds min / max over x * 0: NaN when it holds an inf or a NaN (inf * 0, NaN * 0),
+// otherwise only zeros, each carrying the sign of its x.  min / max (fminf / fmaxf, the FMNMX instruction) order
+// -0 below +0, so the reduction over those zeros gives -0 for the min iff some x has its sign bit set — iff the
+// channel's own min does — and +0 for the max iff some x has it clear — iff the channel's own max does.  The
+// signs are then exactly what reduce_stats(minmax) computes on the fp32 output of mask_apply, whatever its order.
+__device__ __forceinline__ void masked_line(bool keep, float mn, float mx, float &lo, float &hi) {
+  if (keep) {
+    lo = mn, hi = mx;
+  } else if (mn != mn || isinf(mn) || isinf(mx)) {
+    lo = hi = __uint_as_float(0x7fc00000u);
+  } else {
+    lo = signbit(mn) ? -0.0f : 0.0f;
+    hi = signbit(mx) ? -0.0f : 0.0f;
+  }
+}
+
 // mag = (t * mag + m) / (t + 1)      ref qsparse/sparse.py:89
 __device__ __forceinline__ float magnitude_ema_step(float mag, float m,
                                                     int64_t t) {

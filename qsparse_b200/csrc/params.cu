@@ -119,17 +119,20 @@ __global__ void __launch_bounds__(1024)
 // qsb_reduce_prune_quant_step (reduce.cu), where the last CTA of the reduction does this.
 // ---------------------------------------------------------------------------
 constexpr int kStepKernelThreads = 512;  // 128 registers per thread: the batched peer poll keeps 24 packets in flight
+// LINES: the line form (a.lines != NULL)
+template <bool LINES>
 __global__ void __launch_bounds__(kStepKernelThreads)
     prune_quant_step_kernel(const __grid_constant__ StepArgs a) {
   pdl_wait();     // the partials come from the reduction launched just before
   pdl_trigger();  // the forward kernel's CTAs may queue up behind this single CTA
-  extern __shared__ __align__(16) unsigned char qsb_dyn_smem[];  // step_smem_bytes(a.channels)
-  step_epilogue(a, carve_step_smem(qsb_dyn_smem, a.channels));
+  extern __shared__ __align__(16) unsigned char qsb_dyn_smem[];  // step_smem_bytes(a.channels, LINES)
+  step_epilogue<LINES>(a, carve_step_smem(qsb_dyn_smem, a.channels));
 }
 
 // Above the 48 KB of dynamic shared memory any kernel may take (from ~2400 channels) the kernel needs
 // the opt-in, once per device.  cudaFuncSetAttribute is not a stream operation: it is legal while the
 // caller's stream is being captured.
+template <bool LINES>
 static cudaError_t step_kernel_smem_opt_in() {
   static std::once_flag once[64];
   static cudaError_t err[64];
@@ -137,17 +140,22 @@ static cudaError_t step_kernel_smem_opt_in() {
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64) dev = 0;
   std::call_once(once[dev], [dev] {
-    err[dev] = cudaFuncSetAttribute(prune_quant_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)step_smem_bytes(kStepMaxChannels));
+    err[dev] = cudaFuncSetAttribute(prune_quant_step_kernel<LINES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)step_smem_bytes(LINES ? kLineStepMaxChannels : kStepMaxChannels, LINES));
   });
   return err[dev];
 }
 
-static int launch_step_kernel(const StepArgs &a, cudaStream_t stream) {
-  const size_t smem = step_smem_bytes(a.channels);
-  if (smem > 48 * 1024) QSB_CUDA_TRY(step_kernel_smem_opt_in());
-  QSB_CUDA_TRY(launch_k(prune_quant_step_kernel, dim3(1), dim3(kStepKernelThreads), smem, stream, a));
+template <bool LINES>
+static int launch_step_kernel_form(const StepArgs &a, cudaStream_t stream) {
+  const size_t smem = step_smem_bytes(a.channels, LINES);
+  if (smem > 48 * 1024) QSB_CUDA_TRY(step_kernel_smem_opt_in<LINES>());
+  QSB_CUDA_TRY(launch_k(prune_quant_step_kernel<LINES>, dim3(1), dim3(kStepKernelThreads), smem, stream, a));
   return 0;
+}
+
+static int launch_step_kernel(const StepArgs &a, cudaStream_t stream) {
+  return a.lines ? launch_step_kernel_form<true>(a, stream) : launch_step_kernel_form<false>(a, stream);
 }
 
 }  // namespace qsb
@@ -343,6 +351,28 @@ int fill_step_args(qsb::StepArgs &a, float *magnitude, uint8_t *mask, float *sca
   a.step_counter = reinterpret_cast<long long *>(step_counter_dev);
   return 0;
 }
+
+int fill_line_step_args(StepArgs &a, float *magnitude, uint8_t *mask, float *lines, int64_t n_lines,
+                        int64_t channels, qsb_p2p_group *group, double count, int64_t t_prune, int update_magnitude,
+                        int refresh_mask, int64_t k, int64_t t_line, double *abssum_out, float *min_out,
+                        float *max_out, int64_t *step_counter_dev) {
+  if (!lines || group) return QSB_E_BADARG;  // the line form runs on one GPU
+  if (n_lines != 1 && n_lines != channels) return QSB_E_BADARG;
+  if (!step_counter_dev && t_line < 1) return QSB_E_BADARG;
+  // the pow2 checks and fields; `lines` stands in for the scale, which the line form never touches
+  const int rc = fill_step_args(a, magnitude, mask, lines, nullptr, channels, nullptr, 0, count, t_prune,
+                                update_magnitude, refresh_mask, k, 8, 0, 0, nullptr, nullptr, 0, step_counter_dev,
+                                256);
+  if (rc) return rc;
+  a.scale = nullptr;
+  a.lines = lines;
+  a.n_lines = (int)n_lines;
+  a.t_line = t_line;
+  a.abssum_out = abssum_out;
+  a.min_out = min_out;
+  a.max_out = max_out;
+  return 0;
+}
 }  // namespace qsb
 
 extern "C" int qsb_prune_quant_step_params(
@@ -383,4 +413,26 @@ extern "C" int qsb_prune_quant_rows_step_params(
                                 nullptr, nullptr, 0, nullptr, 1024);
   if (rc) return rc;
   return launch_step_kernel_on_rows(a, abssum, absmax, n_stat_rows, stat_row_stride_bytes, (cudaStream_t)stream);
+}
+
+// The line form on the partials of qsb_reduce_line_partials_dt (1025 - 2048 channels).
+extern "C" int qsb_prune_line_step_params(
+    float *magnitude, uint8_t *mask, float *lines, int64_t n_lines, void *reduce_workspace, int64_t workspace_bytes,
+    int64_t outer, int64_t channels, int64_t inner, qsb_p2p_group *group, double count, int64_t t_prune,
+    int update_magnitude, int refresh_mask, int64_t k, int64_t t_line, double *abssum_out, float *min_out,
+    float *max_out, int64_t *step_counter_dev, void *stream) {
+  if (outer <= 0 || channels <= 0 || inner <= 0 || !reduce_workspace) return QSB_E_BADARG;
+  if (channels > kLineStepMaxChannels) return QSB_E_UNSUPPORTED;
+  StepArgs a;
+  const int rc = fill_line_step_args(a, magnitude, mask, lines, n_lines, channels, group, count, t_prune,
+                                     update_magnitude, refresh_mask, k, t_line, abssum_out, min_out, max_out,
+                                     step_counter_dev);
+  if (rc) return rc;
+  const ReducePlan pl = make_plan(outer, channels, inner, nullptr);
+  if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
+  if (pl.fin_count > 0x7fffffffLL || pl.fin_q > 0x7fffffffLL) return QSB_E_UNSUPPORTED;
+  a.P = partials_from_workspace(reduce_workspace, pl.n_partials);
+  a.fin_count = (int)pl.fin_count;
+  a.fin_q = (int)pl.fin_q;
+  return launch_step_kernel(a, (cudaStream_t)stream);
 }

@@ -193,6 +193,12 @@ struct StepTail {
   const uint8_t *keep_hint;  // optional channel mask of the previous step (L2 residency hint)
 };
 
+// the statistics a stage-1 kernel gathers decide the form of its parameter step: sum|x| + max|x| the pow2 form,
+// sum|x| + min / max x the line form (AdaptiveQuantizer)
+template <int WHAT>
+constexpr bool kLineStep = (WHAT & QSB_STAT_MINMAX) != 0;
+
+template <bool LINES>
 __device__ __forceinline__ void fused_step_tail(const StepTail &t, unsigned char *smem, const StepPrefetch &pre) {
   __shared__ int s_last;
   // The CTA barrier orders every thread's partial stores before thread 0's fence + atomic (the grid-sync
@@ -211,16 +217,16 @@ __device__ __forceinline__ void fused_step_tail(const StepTail &t, unsigned char
   }
   __syncthreads();
   if (!s_last) return;
-  step_epilogue(t.a, carve_step_smem(smem, t.a.channels), pre);
+  step_epilogue<LINES>(t.a, carve_step_smem(smem, t.a.channels), pre);
 }
 
 // kernel start: the old state into registers (StepPrefetch) and, for the bench's evidence, the earliest
 // start time of any CTA
-template <class Tail>
+template <int WHAT, class Tail>
 __device__ __forceinline__ StepPrefetch fused_step_begin(const Tail &tail) {
   if constexpr (std::is_same<Tail, StepTail>::value) {
     if (tail.a.timing && threadIdx.x == 0) atomicMin(tail.a.timing, global_ns());
-    return step_prefetch(tail.a);
+    return step_prefetch<kLineStep<WHAT>>(tail.a);
   } else {
     return StepPrefetch{false, 0.f, 0.f, 0};
   }
@@ -433,7 +439,7 @@ __device__ __forceinline__ void fused_tail(const FinalTail &t, const Partials &P
 template <int WHAT>
 __device__ __forceinline__ void fused_tail(const StepTail &t, const Partials &, unsigned char *smem,
                                            const StepPrefetch &pre) {
-  fused_step_tail(t, smem, pre);
+  fused_step_tail<kLineStep<WHAT>>(t, smem, pre);
 }
 
 // 256-bit load with a run-time L2 eviction policy (createpolicy): kept channels of the previous
@@ -477,7 +483,7 @@ __global__ void __launch_bounds__(QSB_THREADS, MINB)
   pdl_wait();
   pdl_trigger();
   extern __shared__ __align__(16) unsigned char qsb_dyn_smem[];
-  const StepPrefetch pre = fused_step_begin(tail);
+  const StepPrefetch pre = fused_step_begin<WHAT>(tail);
   if constexpr (std::is_same<Tail, StepTail>::value) ktime_begin(0);
   const int lane = threadIdx.x & 31;
   const int64_t warps_phys = (int64_t)gridDim.x * (QSB_THREADS / 32);
@@ -633,7 +639,7 @@ __global__ void __launch_bounds__(QSB_THREADS, kTileCtasPerSm)
                        int span_stride, int64_t vwarps, Partials P, const __grid_constant__ Tail tail) {
   pdl_wait();
   pdl_trigger();
-  const StepPrefetch pre = fused_step_begin(tail);
+  const StepPrefetch pre = fused_step_begin<WHAT>(tail);
   __shared__ __align__(32) float tile[kTileFloats];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t slot0 = (int64_t)blockIdx.x * tile_rows;
@@ -849,7 +855,7 @@ __global__ void __launch_bounds__(QSB_THREADS)
                        int64_t rows_per_chunk, int tpr, Partials P, const __grid_constant__ Tail tail) {
   extern __shared__ __align__(16) unsigned char qsb_dyn_smem[];
   if constexpr (std::is_same<Tail, StepTail>::value) pdl_wait();  // the old state may have been written by the kernel just before
-  const StepPrefetch pre = fused_step_begin(tail);
+  const StepPrefetch pre = fused_step_begin<WHAT>(tail);
   reduce_cols_body<WHAT, V, T>(x, nrows, ncols, rows_per_chunk, tpr, P);
   if constexpr (Tail::kFused) fused_tail<WHAT>(tail, P, qsb_dyn_smem, pre);
 }
@@ -1242,9 +1248,10 @@ ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner,
   return p;
 }
 
-// a finalized statistics row in a workspace: fp64 sums and fp32 maxima, each 256-byte aligned
+// a finalized statistics row in a workspace: fp64 sums, fp32 maxima and fp32 minima (line form), each 256-byte
+// aligned
 static inline int64_t stat_row_bytes(int64_t channels) {
-  return (channels * 8 + 255) / 256 * 256 + (channels * 4 + 255) / 256 * 256;
+  return (channels * 8 + 255) / 256 * 256 + 2 * ((channels * 4 + 255) / 256 * 256);
 }
 
 int64_t partial_bytes(int64_t n) {
@@ -1270,7 +1277,7 @@ static int run_reduce(const T *x, const ReducePlan &pl, int64_t channels,
                       int64_t inner, const Partials &P, const FinalOut &out,
                       cudaStream_t stream, bool finalize = true, const Tail &tail = Tail{}) {
   // dynamic shared memory of the fused parameter step (the tile kernel re-uses its tile buffer)
-  const size_t dyn = std::is_same<Tail, StepTail>::value ? step_smem_bytes((int)channels) : 0;
+  const size_t dyn = std::is_same<Tail, StepTail>::value ? step_smem_bytes((int)channels, kLineStep<WHAT>) : 0;
   if (pl.row_mode && pl.tile_rows > 0) {
     // the tile kernel (only reachable through tuning key 20) stages fp32 sectors: fp32 input only
     if constexpr (is_half16<T>) {
@@ -1437,11 +1444,11 @@ extern "C" int qsb_reduce_stats_fused(const float *x, int what, int64_t outer, i
                            workspace_bytes, arrival_counter_dev, stream);
 }
 
-// Stage 1 only: leaves the per-virtual-warp partials of sum|x| and max|x| in the
-// workspace for qsb_prune_quant_step_params, which finalizes them itself.
-extern "C" int qsb_reduce_partials_dt(const void *x_, int x_dtype, int64_t outer, int64_t channels,
-                                      int64_t inner, void *workspace,
-                                      int64_t workspace_bytes, void *stream_) {
+// Stage 1 only: leaves the per-virtual-warp partials of sum|x| and max|x| (WHAT: sum|x| and min / max x) in the
+// workspace for qsb_prune_quant_step_params (qsb_prune_line_step_params), which finalizes them itself.
+template <int WHAT>
+static int reduce_partials_impl(const void *x_, int x_dtype, int64_t outer, int64_t channels, int64_t inner,
+                                void *workspace, int64_t workspace_bytes, void *stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   if (!dtype_ok(x_dtype)) return QSB_E_BADARG;
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
@@ -1454,9 +1461,20 @@ extern "C" int qsb_reduce_partials_dt(const void *x_, int x_dtype, int64_t outer
     if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
     const Partials P = partials_from_workspace(workspace, pl.n_partials);
     FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
-    return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, NoTail, T>(x, pl, channels, inner, P, out,
-                                                                   stream, /*finalize=*/false);
+    return run_reduce<WHAT, NoTail, T>(x, pl, channels, inner, P, out, stream, /*finalize=*/false);
   });
+}
+
+extern "C" int qsb_reduce_partials_dt(const void *x, int x_dtype, int64_t outer, int64_t channels, int64_t inner,
+                                      void *workspace, int64_t workspace_bytes, void *stream) {
+  return reduce_partials_impl<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX>(x, x_dtype, outer, channels, inner, workspace,
+                                                                 workspace_bytes, stream);
+}
+
+extern "C" int qsb_reduce_line_partials_dt(const void *x, int x_dtype, int64_t outer, int64_t channels,
+                                           int64_t inner, void *workspace, int64_t workspace_bytes, void *stream) {
+  return reduce_partials_impl<QSB_STAT_ABSSUM | QSB_STAT_MINMAX>(x, x_dtype, outer, channels, inner, workspace,
+                                                                 workspace_bytes, stream);
 }
 
 extern "C" int qsb_reduce_partials(const float *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
@@ -1549,4 +1567,66 @@ extern "C" int qsb_reduce_prune_quant_step(
                                       magnitude, mask, scale, decimal_out, group, step_stamp, count, t_prune,
                                       update_magnitude, refresh_mask, k, bits, t_quant, update_scale, abssum_out,
                                       absmax_out, stats_local, step_counter_dev, timing_out_dev, stream);
+}
+
+// The line form of the same step (AdaptiveQuantizer): the stage-1 reduction gathers sum|x| and min / max x, the
+// last-arriving CTA runs finalize -> magnitude EMA -> threshold -> mask -> (min, max) of x * mask -> lines EMA.
+// Same reduction plan, same summation order of sum|x| (the magnitudes equal those of the pow2 step bit for bit).
+template <class T>
+static int reduce_prune_line_step_impl(const T *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+                                       int64_t workspace_bytes, unsigned int *arrival_counter_dev, const StepArgs &a,
+                                       cudaStream_t stream) {
+  constexpr int kWhat = QSB_STAT_ABSSUM | QSB_STAT_MINMAX;
+  if (!aligned_to(x, sizeof(T)) || !aligned_to(arrival_counter_dev, 4)) return QSB_E_ALIGN;
+  const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
+  if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
+  if (pl.fin_count > 0x7fffffffLL || pl.fin_q > 0x7fffffffLL) return QSB_E_UNSUPPORTED;
+  const Partials P = partials_from_workspace(workspace, pl.n_partials);
+  StepTail tail;
+  tail.a = a;
+  if (channels * pl.fin_count > kStepTailMaxEntries) {
+    // as the pow2 step: stage 1, a parallel finalize into a statistics row, the step kernel on that row
+    if (workspace_bytes < partial_bytes(pl.n_partials) + 256 + stat_row_bytes(channels)) return QSB_E_WORKSPACE;
+    unsigned char *row = reinterpret_cast<unsigned char *>(
+        (reinterpret_cast<uintptr_t>(workspace) + 255) / 256 * 256 + (uintptr_t)partial_bytes(pl.n_partials));
+    double *row_sum = reinterpret_cast<double *>(row);
+    float *row_max = reinterpret_cast<float *>(row + (channels * 8 + 255) / 256 * 256);
+    float *row_min = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(row_max) +
+                                               (channels * 4 + 255) / 256 * 256);
+    FinalOut out{nullptr, row_min, row_max, row_sum, nullptr};
+    const int rc = run_reduce<kWhat, NoTail, T>(x, pl, channels, inner, P, out, stream);
+    if (rc) return rc;
+    tail.a.row_min = row_min;
+    return launch_step_kernel_on_rows(tail.a, row_sum, row_max, 1, 0, stream);
+  }
+  tail.a.P = P;
+  tail.a.fin_count = (int)pl.fin_count;
+  tail.a.fin_q = (int)pl.fin_q;
+  tail.arrival = arrival_counter_dev;
+  // no L2 keep hint: the line forward reads the pruned channels too
+  tail.keep_hint = nullptr;
+  FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
+  return run_reduce<kWhat, StepTail, T>(x, pl, channels, inner, P, out, stream, /*finalize=*/false, tail);
+}
+
+extern "C" int qsb_reduce_prune_line_step_dt(
+    const void *x, int x_dtype, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+    int64_t workspace_bytes, unsigned int *arrival_counter_dev, float *magnitude, uint8_t *mask, float *lines,
+    int64_t n_lines, qsb_p2p_group *group, double count, int64_t t_prune, int update_magnitude, int refresh_mask,
+    int64_t k, int64_t t_line, double *abssum_out, float *min_out, float *max_out, int64_t *step_counter_dev,
+    void *stream) {
+  if (!dtype_ok(x_dtype)) return QSB_E_BADARG;
+  if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
+  if (!x || !workspace || !arrival_counter_dev) return QSB_E_BADARG;
+  if (channels > kStepFusedMaxChannels) return QSB_E_UNSUPPORTED;
+  StepArgs a;
+  const int rc = fill_line_step_args(a, magnitude, mask, lines, n_lines, channels, group, count, t_prune,
+                                     update_magnitude, refresh_mask, k, t_line, abssum_out, min_out, max_out,
+                                     step_counter_dev);
+  if (rc) return rc;
+  return dispatch_dtype(x_dtype, [&](auto *tx) {
+    using T = std::remove_pointer_t<decltype(tx)>;
+    return reduce_prune_line_step_impl(static_cast<const T *>(x), outer, channels, inner, workspace,
+                                       workspace_bytes, arrival_counter_dev, a, (cudaStream_t)stream);
+  });
 }

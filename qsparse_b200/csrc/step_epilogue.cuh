@@ -33,9 +33,10 @@
 
 namespace qsb {
 
-// Both forms carve step_smem_bytes(channels) of dynamic shared memory (20 B / channel).
+// Both forms carve step_smem_bytes(channels) of dynamic shared memory (20 B / channel; the line form 28).
 constexpr int kStepMaxChannels = 4096;      // stand-alone kernel: ~82 KB, opted in above the 48 KB default
 constexpr int kStepFusedMaxChannels = 1024; // fused tail: shares the CTA with the reduction
+constexpr int kLineStepMaxChannels = 2048;  // line form, stand-alone kernel (partials route)
 
 struct StepArgs {
   float *magnitude;
@@ -66,6 +67,13 @@ struct StepArgs {
   int stats_local;
   long long *step_counter;  // optional device step index (CUDA graphs)
   unsigned long long *timing;  // optional: %globaltimer stamps of the phases (development / bench evidence)
+  // line form (step_epilogue<true>, AdaptiveQuantizer): in place of abs-max -> scale -> decimal, the (min, max)
+  // of x * mask -> lines EMA.  The statistics are sum|x| and min / max x (row_max then holds max x, not max|x|).
+  float *lines;           // [n_lines, 2], n_lines == 1 (per tensor) or channels
+  int n_lines;
+  int64_t t_line;         // the quantizer's 1-based call index (an offset to *step_counter when that is given)
+  const float *row_min;
+  float *min_out, *max_out;  // optional, like abssum_out: this step's min / max x per channel
 };
 
 struct StepSmem {
@@ -78,10 +86,11 @@ struct StepSmem {
   uint32_t *amax; // [32]
   float *thr;     // [1]
   int *flag;      // [1]
+  float *mn, *mx; // [channels] each, line form only (min / max x, NaN when the channel holds a NaN)
 };
 
-__host__ __device__ inline size_t step_smem_bytes(int channels) {
-  return (size_t)channels * 20 + 32 * 8 + 32 * 4 + 32 * 4 + 16;
+__host__ __device__ inline size_t step_smem_bytes(int channels, bool lines = false) {
+  return (size_t)channels * 20 + 32 * 8 + 32 * 4 + 32 * 4 + 16 + (lines ? (size_t)channels * 8 : 0);
 }
 __device__ __forceinline__ StepSmem carve_step_smem(unsigned char *base, int channels) {
   StepSmem s;
@@ -94,6 +103,8 @@ __device__ __forceinline__ StepSmem carve_step_smem(unsigned char *base, int cha
   s.amax = s.pmax + 32;
   s.thr = reinterpret_cast<float *>(s.amax + 32);
   s.flag = reinterpret_cast<int *>(s.thr + 1);
+  s.mn = reinterpret_cast<float *>(base + step_smem_bytes(channels));
+  s.mx = s.mn + channels;
   return s;
 }
 
@@ -122,6 +133,7 @@ struct StepPrefetch {
   long long t;          // *step_counter (every thread)
 };
 
+template <bool LINES = false>
 __device__ __forceinline__ StepPrefetch step_prefetch(const StepArgs &a) {
   StepPrefetch p;
   const int tid = threadIdx.x, nthr = blockDim.x;
@@ -132,7 +144,7 @@ __device__ __forceinline__ StepPrefetch step_prefetch(const StepArgs &a) {
   if (!p.valid) return p;
   const int c = tid / a.group;
   if (tid % a.group == 0 && c < a.channels && a.update_magnitude != 2) p.mag_old = a.magnitude[c];
-  if (tid == 0) p.scale_old = a.scale[0];
+  if (!LINES && tid == 0) p.scale_old = a.scale[0];
   if (a.step_counter) p.t = *a.step_counter;
   return p;
 }
@@ -142,6 +154,8 @@ __device__ __forceinline__ void step_stamp_time(const StepArgs &a, int slot) {
 }
 
 // Runs on every thread of ONE CTA (blockDim.x a multiple of 32).  sm: shared memory of that CTA.
+// LINES: the line form (StepArgs::lines); it takes no peer group.
+template <bool LINES = false>
 __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem &sm,
                                               const StepPrefetch pre = StepPrefetch{false, 0.f, 0.f, 0}) {
   int64_t t_prune = a.t_prune, t_quant = a.t_quant;
@@ -163,7 +177,7 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
   const int channels = a.channels, group = a.group;
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5;
   const int gl = tid % group, gc = tid / group, cpp = nthr / group;
-  const float scale_old = pre.valid ? pre.scale_old : ((tid == 0) ? a.scale[0] : 0.0f);  // prefetch
+  const float scale_old = LINES ? 0.0f : pre.valid ? pre.scale_old : ((tid == 0) ? a.scale[0] : 0.0f);  // prefetch
   if (tid == 0) *sm.flag = 0;
   step_stamp_time(a, 1);
 
@@ -172,11 +186,20 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
     for (int c = tid; c < channels; c += nthr) {
       double sum = 0.0;
       uint32_t mx = 0;
+      float cmin = INFINITY, cmax = -INFINITY;  // line form: min / max x
+      bool nan = false;
       for (int r = 0; r < a.n_rows; ++r) {
         if (a.row_sum)
           sum += *reinterpret_cast<const double *>(reinterpret_cast<const char *>(a.row_sum + c) +
                                                    (int64_t)r * a.row_stride);
-        if (a.row_max) {
+        if constexpr (LINES) {
+          const int64_t off = (int64_t)r * a.row_stride;
+          const float l = *reinterpret_cast<const float *>(reinterpret_cast<const char *>(a.row_min + c) + off);
+          const float h = *reinterpret_cast<const float *>(reinterpret_cast<const char *>(a.row_max + c) + off);
+          nan = nan || l != l || h != h;
+          cmin = fminf(cmin, l);
+          cmax = fmaxf(cmax, h);
+        } else if (a.row_max) {
           const float v = *reinterpret_cast<const float *>(reinterpret_cast<const char *>(a.row_max + c) +
                                                            (int64_t)r * a.row_stride);
           const uint32_t b = __float_as_uint(v) & 0x7fffffffu;
@@ -184,7 +207,12 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
         }
       }
       sm.sum[c] = sum;
-      sm.max[c] = mx;
+      if constexpr (LINES) {
+        sm.mn[c] = nan ? nan_poison() : cmin;
+        sm.mx[c] = nan ? nan_poison() : cmax;
+      } else {
+        sm.max[c] = mx;
+      }
       sm.imp[c] = (a.update_magnitude != 2) ? a.magnitude[c] : 0.0f;
     }
   } else {
@@ -198,6 +226,8 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
       if (!pre.valid && act && gl == 0 && a.update_magnitude != 2) mag_old = a.magnitude[c];  // prefetch
       double sum = 0.0;
       uint32_t mx = 0;
+      float cmin = INFINITY, cmax = -INFINITY;  // line form: min / max x, NaN-propagating through `nan`
+      bool nan = false;
       if (act) {
         // kFinBatch independent loads per thread in flight (L2 hits): the C2 plan has 9 entries per
         // thread, i.e. ONE round trip; the additions run in ascending j whatever the batch size
@@ -205,6 +235,7 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
         for (int j0 = gl; j0 < a.fin_count; j0 += kFinBatch * group) {
           double v[kFinBatch];
           uint32_t b[kFinBatch];
+          float l[kFinBatch], h[kFinBatch];
 #pragma unroll
           for (int u = 0; u < kFinBatch; ++u) {
             const int j = j0 + u * group;
@@ -213,45 +244,91 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
             const int64_t idx =
                 (int64_t)hi * ((int64_t)channels * a.fin_q) + (int64_t)c * a.fin_q + (ok ? j - hi * a.fin_q : 0);
             v[u] = ok ? __ldcg(a.P.asum + idx) : 0.0;
-            b[u] = ok ? __ldcg(a.P.amax + idx) : 0u;
+            if constexpr (LINES) {
+              l[u] = ok ? __ldcg(a.P.mn + idx) : INFINITY;
+              h[u] = ok ? __ldcg(a.P.mx + idx) : -INFINITY;
+            } else {
+              b[u] = ok ? __ldcg(a.P.amax + idx) : 0u;
+            }
           }
 #pragma unroll
           for (int u = 0; u < kFinBatch; ++u) {
             sum += v[u];
-            mx = b[u] > mx ? b[u] : mx;
+            if constexpr (LINES) {
+              nan = nan || l[u] != l[u] || h[u] != h[u];
+              cmin = fminf(cmin, l[u]);
+              cmax = fmaxf(cmax, h[u]);
+            } else {
+              mx = b[u] > mx ? b[u] : mx;
+            }
           }
         }
       }
       for (int o = (group < 32 ? group : 32) >> 1; o > 0; o >>= 1) {
         sum += __shfl_xor_sync(0xffffffffu, sum, o);
-        const uint32_t other = __shfl_xor_sync(0xffffffffu, mx, o);
-        mx = other > mx ? other : mx;
+        if constexpr (LINES) {
+          nan = __shfl_xor_sync(0xffffffffu, (int)nan, o) || nan;
+          cmin = fminf(cmin, __shfl_xor_sync(0xffffffffu, cmin, o));
+          cmax = fmaxf(cmax, __shfl_xor_sync(0xffffffffu, cmax, o));
+        } else {
+          const uint32_t other = __shfl_xor_sync(0xffffffffu, mx, o);
+          mx = other > mx ? other : mx;
+        }
+      }
+      if constexpr (LINES) {
+        if (nan) cmin = cmax = nan_poison();
       }
       if (group > 32) {
         // one channel, the whole CTA (per-tensor statistics): combine the warps of the group
-        // through shared memory, in warp order
+        // through shared memory, in warp order (line form: min / max bits in pmax / amax)
         if (lane == 0) {
           sm.psum[warp] = sum;
-          sm.pmax[warp] = mx;
+          if constexpr (LINES) {
+            sm.pmax[warp] = __float_as_uint(cmin);
+            sm.amax[warp] = __float_as_uint(cmax);
+          } else {
+            sm.pmax[warp] = mx;
+          }
         }
         __syncthreads();
         if (gl == 0)
           for (int w = 1; w < group / 32; ++w) {
             sum += sm.psum[warp + w];
-            mx = sm.pmax[warp + w] > mx ? sm.pmax[warp + w] : mx;
+            if constexpr (LINES) {
+              const float l = __uint_as_float(sm.pmax[warp + w]), h = __uint_as_float(sm.amax[warp + w]);
+              nan = nan || l != l || h != h;
+              cmin = fminf(cmin, l);
+              cmax = fmaxf(cmax, h);
+            } else {
+              mx = sm.pmax[warp + w] > mx ? sm.pmax[warp + w] : mx;
+            }
           }
+        if constexpr (LINES) {
+          if (nan) cmin = cmax = nan_poison();
+        }
         __syncthreads();
       }
       if (act && gl == 0) {
         sm.sum[c] = sum;
-        sm.max[c] = mx;
+        if constexpr (LINES) {
+          sm.mn[c] = cmin;
+          sm.mx[c] = cmax;
+        } else {
+          sm.max[c] = mx;
+        }
         sm.imp[c] = mag_old;
       }
     }
   }
   __syncthreads();
   step_stamp_time(a, 2);
-  if (a.abssum_out && a.stats_local) {
+  if constexpr (LINES) {
+    for (int c = tid; c < channels; c += nthr) {
+      if (a.abssum_out) a.abssum_out[c] = sm.sum[c];
+      if (a.min_out) a.min_out[c] = sm.mn[c];
+      if (a.max_out) a.max_out[c] = sm.mx[c];
+    }
+  } else if (a.abssum_out && a.stats_local) {
     for (int c = tid; c < channels; c += nthr) {
       a.abssum_out[c] = sm.sum[c];
       a.absmax_out[c] = __uint_as_float(sm.max[c]);
@@ -259,7 +336,7 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
   }
 
   // ---- 2. exchange with the peers (weak scaling over the batch) -------------------------
-  if (a.px.world > 1) {
+  if (!LINES && a.px.world > 1) {
     const P2PDev &px = a.px;
     const int parity = (int)(stamp & 1ull);
     const uint32_t flag = (uint32_t)(stamp & 0x7fffffffull) | 0x80000000u;
@@ -360,7 +437,7 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
   // ---- 3. importance (magnitude EMA) -----------------------------------------------------
   step_stamp_time(a, 3);
   for (int c = tid; c < channels; c += nthr) {
-    if (a.abssum_out && !a.stats_local) {
+    if (!LINES && a.abssum_out && !a.stats_local) {
       a.abssum_out[c] = sm.sum[c];
       a.absmax_out[c] = __uint_as_float(sm.max[c]);
     }
@@ -405,6 +482,57 @@ __device__ __forceinline__ void step_epilogue(const StepArgs &a, const StepSmem 
   // ---- 5. mask, abs-max of the kept channels, scale EMA, decimal ---------------------------
   step_stamp_time(a, 5);
   const float thr = refresh_mask ? *sm.thr : 0.0f;
+  if constexpr (LINES) {
+    // line form: (min, max) of x * mask per channel or over the tensor (quantize.py:396-418) -> lines EMA
+    // (quantize.py:428-430) at the quantizer's call index
+    const int64_t tl = a.step_counter ? t_counter + a.t_line : a.t_line;
+    const float tm1 = (float)(tl - 1), tf = (float)tl;
+    float lo = INFINITY, hi = -INFINITY;
+    bool nan = false;
+    for (int c = tid; c < channels; c += nthr) {
+      bool keep;
+      if (refresh_mask) {
+        keep = sm.imp[c] >= thr;
+        a.mask[c] = keep ? 1 : 0;
+      } else {
+        keep = a.mask[c] != 0;
+      }
+      float l, h;
+      masked_line(keep, sm.mn[c], sm.mx[c], l, h);
+      if (a.n_lines == 1) {
+        nan = nan || l != l;
+        lo = fminf(lo, l);
+        hi = fmaxf(hi, h);
+      } else {
+        a.lines[2 * c] = lines_ema_step(a.lines[2 * c], l, tm1, tf);
+        a.lines[2 * c + 1] = lines_ema_step(a.lines[2 * c + 1], h, tm1, tf);
+      }
+    }
+    if (a.n_lines == 1) {
+      lo = warp_reduce(lo, [](float x, float y) { return fminf(x, y); });
+      hi = warp_reduce(hi, [](float x, float y) { return fmaxf(x, y); });
+      if (lane == 0) {
+        sm.pmax[warp] = __float_as_uint(lo);
+        sm.amax[warp] = __float_as_uint(hi);
+      }
+      if (nan) *sm.flag = 1;
+      __syncthreads();
+      if (tid == 0) {
+        for (int w = 1; w < (nthr >> 5); ++w) {
+          lo = fminf(lo, __uint_as_float(sm.pmax[w]));
+          hi = fmaxf(hi, __uint_as_float(sm.amax[w]));
+        }
+        if (*sm.flag) lo = hi = nan_poison();
+        a.lines[0] = lines_ema_step(a.lines[0], lo, tm1, tf);
+        a.lines[1] = lines_ema_step(a.lines[1], hi, tm1, tf);
+      }
+    }
+    if (tid == 0) {
+      if (a.step_counter) *a.step_counter = t_counter + 1;
+      if (a.timing) a.timing[6] = global_ns();
+    }
+    return;
+  }
   uint32_t am = 0;
   for (int c = tid; c < channels; c += nthr) {
     bool keep;
@@ -441,6 +569,11 @@ int fill_step_args(StepArgs &a, float *magnitude, uint8_t *mask, float *scale, f
                    int update_magnitude, int refresh_mask, int64_t k, int bits, int64_t t_quant,
                    int update_scale, double *abssum_out, float *absmax_out, int stats_local,
                    int64_t *step_counter_dev, int threads);
+// the same for the line form (no scale, no group): lines [n_lines, 2], n_lines 1 or channels
+int fill_line_step_args(StepArgs &a, float *magnitude, uint8_t *mask, float *lines, int64_t n_lines,
+                        int64_t channels, qsb_p2p_group *group, double count, int64_t t_prune, int update_magnitude,
+                        int refresh_mask, int64_t k, int64_t t_line, double *abssum_out, float *min_out,
+                        float *max_out, int64_t *step_counter_dev);
 
 // the stand-alone one-CTA launch of the parameter step on n_rows >= 1 finalized statistics rows (params.cu)
 int launch_step_kernel_on_rows(StepArgs a, const double *row_sum, const float *row_max, int64_t n_rows,

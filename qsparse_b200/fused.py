@@ -1,4 +1,4 @@
-"""Fused structured prune -> pow2 quantize (K7): the training step of
+"""Fused structured prune -> quantize (K7): the training step of
 ``Sequential(PruneLayer(dimensions={channel}), QuantizeLayer(channelwise=-1,
 callback=DecimalQuantizer()))`` (the adjacency ``convert()`` creates,
 ref qsparse/convert.py:214-217) in three launches and 20 B/elem:
@@ -16,6 +16,16 @@ step counters are host integers, every derived scalar stays on the device.  With
 process group the statistics row is exchanged over peer memory inside that kernel
 (parallel.P2PExchange; NCCL all-gather + a parameter kernel when peer mapping is
 unavailable) and combined in rank order, so every rank derives identical parameters.
+
+The fusion pass (``FusedPruneQuantSequential``) also takes an ``AdaptiveQuantizer`` site (per-tensor lines, or
+per-channel lines on the prune axis), on one GPU, in the same three launches and bytes:
+
+    forward   reduce_prune_line_step(x)  4 B/elem   sum|x| and min / max x; the last CTA derives magnitude EMA,
+                                                    threshold, mask, the (min, max) of x * mask and the lines EMA
+              fq_line_fwd(x, mask)       8 B/elem   y = Q_lines(x * mask), float zero point
+    backward  mask_apply(g, mask)        8 B/elem   gx = g * mask (identity STE: grad_output is not written)
+
+(bf16 / fp16 x: 2 B/elem less for each read of x and the write of gx, 14 B/elem in all.)
 """
 from __future__ import annotations
 
@@ -180,6 +190,22 @@ class _FusedLayersFn(torch.autograd.Function):
         return (gx,) + (None,) * 7
 
 
+class _FusedLineLayersFn(torch.autograd.Function):
+    """the same for an AdaptiveQuantizer: y = Q_lines(x * mask) with the float zero point of a training step,
+    gx = g * mask.  The line quantizer's backward is the identity (ref quantize.py:134-185, SURVEY Q9), so
+    grad_output is read, never written."""
+
+    @staticmethod
+    def forward(ctx, x, xs, layout, mask, lines, bits):
+        ctx.layout, ctx.mask, ctx.x_dtype = layout, mask, xs.dtype
+        return ops.fq_line_fwd(xs, lines, bits, True, layout, mask=mask).view(x.shape)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        g = N.as_f32_contiguous(grad_output)
+        return (ops.mask_apply(g, ctx.mask, ctx.layout, out_dtype=ctx.x_dtype),) + (None,) * 5
+
+
 class FusedPruneQuantSequential(nn.Sequential):
     """``Sequential(Sequential(act, PruneLayer), QuantizeLayer)`` (what two ``convert()`` calls build around
     an activation, ref qsparse/convert.py:214-217) or ``Sequential(PruneLayer, QuantizeLayer)``, with the
@@ -189,8 +215,9 @@ class FusedPruneQuantSequential(nn.Sequential):
 
     A step is fused only when it is provably the plain case: both layers initialised, training, structured
     channel prune (``dimensions={1}``) by the stock ``MagnitudePruningCallback`` (no gradient / l0 / hook
-    variants), pruning started and the sparsity not changing at this step, per-tensor stock
-    ``DecimalQuantizer`` or ``ScalerQuantizer`` (``quantize()``'s default callback) past its timeout.  Every other step (warm-up, ramp steps, eval, other callbacks,
+    variants), pruning started and the sparsity not changing at this step, past the quantizer's timeout, with
+    a per-tensor stock ``DecimalQuantizer`` or ``ScalerQuantizer`` (``quantize()``'s default callback) or a
+    stock ``AdaptiveQuantizer`` (per tensor, or per channel on the prune axis) after its first estimate.  Every other step (warm-up, ramp steps, eval, other callbacks,
     non-contiguous inputs) runs the two layers one after the other, exactly as before.  Counters and
     parameters advance identically either way, so the two routes can alternate freely."""
 
@@ -203,7 +230,7 @@ class FusedPruneQuantSequential(nn.Sequential):
         return None, first, q
 
     def _fusable(self, p, q, x):
-        from .quantize import DecimalQuantizer, QuantizeLayer, ScalerQuantizer
+        from .quantize import AdaptiveQuantizer, DecimalQuantizer, QuantizeLayer, ScalerQuantizer
         from .sparse import MagnitudePruningCallback, PruneLayer
 
         if not (isinstance(p, PruneLayer) and isinstance(q, QuantizeLayer) and self.training and p.training
@@ -212,7 +239,8 @@ class FusedPruneQuantSequential(nn.Sequential):
         if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dim() >= 2 and x.is_contiguous()):
             return False
         cb, qcb = p.callback, q.callback
-        if type(cb) is not MagnitudePruningCallback or type(qcb) not in (DecimalQuantizer, ScalerQuantizer):
+        if type(cb) is not MagnitudePruningCallback or type(qcb) not in (DecimalQuantizer, ScalerQuantizer,
+                                                                         AdaptiveQuantizer):
             return False
         if cb.use_gradient or cb.l0 or cb.forward_hook is not None or not cb.training or not qcb.training:
             return False
@@ -227,17 +255,27 @@ class FusedPruneQuantSequential(nn.Sequential):
             return False
         if cb.running_average and not hasattr(cb, "magnitude"):
             return False
-        if q.channelwise >= 0 or q.timeout <= 0 or q._t_mirror.get(q._n_updates) < q.timeout:
+        if q.timeout <= 0 or q._t_mirror.get(q._n_updates) < q.timeout or qcb.group_num > 0:
             return False
-        if qcb.backward_passthrough or qcb.use_uint or qcb.group_num > 0:
+        if p._s_mirror.get(p._cur_sparsity) < 0:
+            return False
+        if type(qcb) is AdaptiveQuantizer:
+            # lines per tensor or per channel of the prune axis; not before the first optimize(), which may
+            # re-create `t` (like _fused_weight_step)
+            rows = 1 if q.channelwise < 0 else p.mask.numel()
+            if q.channelwise >= 0 and q.channelwise != 1:
+                return False
+            if tuple(q.weight.shape) != (rows, 2) or not q.weight.is_contiguous():
+                return False
+            return isinstance(qcb.t, torch.Tensor) or qcb.t != 0
+        if q.channelwise >= 0 or qcb.backward_passthrough or qcb.use_uint:
             return False
         if qcb.use_float_scaler != (type(qcb) is ScalerQuantizer):
             return False
-        if tuple(q.weight.shape) != (1, 1) or p._s_mirror.get(p._cur_sparsity) < 0:
-            return False
-        return True
+        return tuple(q.weight.shape) == (1, 1)
 
     def _fused_step(self, p, q, x):
+        from .quantize import AdaptiveQuantizer
         cb, qcb = p.callback, q.callback
         layout = N.channel_layout(x.shape, 1)
         outer, ch, inner = layout
@@ -251,7 +289,8 @@ class FusedPruneQuantSequential(nn.Sequential):
             raise IndexError(f"index {k} is out of bounds for dimension 0 with size {ch}")
         if not refresh:
             k = min(k, ch - 1)
-        is_decimal = not qcb.use_float_scaler
+        line = type(qcb) is AdaptiveQuantizer
+        is_decimal = not line and not qcb.use_float_scaler
         # DecimalQuantizer: this step's decimal (a fresh tensor: the backward must see THIS step's value);
         # ScalerQuantizer: the quantize kernels read the layer's scale itself, like the reference's saved tensor
         decimal = torch.empty(1, dtype=torch.float32, device=x.device) if is_decimal else None
@@ -260,31 +299,46 @@ class FusedPruneQuantSequential(nn.Sequential):
                 magnitude, mode = cb.magnitude.data.view(-1), 1
             else:
                 magnitude, mode = torch.empty(ch, dtype=torch.float32, device=x.device), 2
+            # AdaptiveQuantizer: this call's 1-based index; also advances its device `t` when it has one
+            t_line = qcb._next_t() if line else 0
             if graphs.active():
                 # graph mode: the step index is the prune callback's own `t` Parameter, read and advanced by the
                 # kernel; the quantizer's EMA index keeps its constant distance to it
                 if cb.stop_mask_refresh != float("inf"):
                     raise graphs.NotCapturable("a fused site with a stopping mask refresh")
-                ops.structured_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data.view(-1),
-                                                decimal, float(outer * inner), 0, mode, cb.mask_refresh_interval,
-                                                kth_rank(sparsity, ch), q.bits, qcb.t - t, True,
-                                                step_counter=graphs.callback_counter(cb, x.device))
+                counter = graphs.callback_counter(cb, x.device)
+                if line:
+                    ops.structured_prune_line_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data,
+                                                   float(outer * inner), 0, mode, cb.mask_refresh_interval,
+                                                   kth_rank(sparsity, ch), t_line - t, step_counter=counter)
+                else:
+                    ops.structured_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1),
+                                                    q.weight.data.view(-1), decimal, float(outer * inner), 0, mode,
+                                                    cb.mask_refresh_interval, kth_rank(sparsity, ch), q.bits,
+                                                    qcb.t - t, True, step_counter=counter)
             else:
-                ops.structured_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data.view(-1),
-                                                decimal, float(outer * inner), t, mode, refresh, k, q.bits, qcb.t,
-                                                True)
+                if line:
+                    ops.structured_prune_line_step(xs, layout, magnitude, p.mask.data.view(-1), q.weight.data,
+                                                   float(outer * inner), t, mode, refresh, k, t_line)
+                else:
+                    ops.structured_prune_quant_step(xs, layout, magnitude, p.mask.data.view(-1),
+                                                    q.weight.data.view(-1), decimal, float(outer * inner), t, mode,
+                                                    refresh, k, q.bits, qcb.t, True)
                 cb.t.data.add_(1)
             # the counters of the two layers and their callbacks, as their own forwards advance them
             cb._t_mirror.wrote(cb.t, t + 1)
             n = p._n_mirror.get(p._n_updates)
             p._n_updates.data.add_(1)
             p._n_mirror.wrote(p._n_updates, n + 1)
-            qcb.t += 1
+            if not line:
+                qcb.t += 1
             q._quantized = True
             tq = q._t_mirror.get(q._n_updates)
             q._n_updates.data.add_(1)
             q._t_mirror.wrote(q._n_updates, tq + 1)
         self.fused_steps += 1
+        if line:
+            return _FusedLineLayersFn.apply(x, xs, layout, p.mask.data.view(-1), q.weight.data, q.bits)
         return _FusedLayersFn.apply(x, xs, layout, p.mask.data.view(-1),
                                     decimal if is_decimal else q.weight.data.view(-1), q.bits,
                                     1 if qcb.flip_axis else 0, is_decimal)

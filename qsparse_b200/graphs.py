@@ -16,7 +16,8 @@ Capturable routes: every stock quantizer (Decimal / Scaler / Adaptive / Percenti
 row-resident weight kernel, the fused weight chain), the stock magnitude prune callback with a channel mask or a
 full-size mask (the one-pass step K9, per layer or batched by ``WeightSetPruner``) or a frozen mask, and fused
 prune -> quantize activation sites
-(``convert(..., fuse=True)``), past their timeouts and schedules, with the default mask refresh (every step, never
+(``convert(..., fuse=True)``; Decimal / Scaler, and Adaptive whose lines index keeps a constant offset to the prune
+callback's counter, up to 1 024 channels), past their timeouts and schedules, with the default mask refresh (every step, never
 stopping).  Every other stateful route (gradient / l0 importance, sparser refresh intervals on full-size masks,
 group-wise scale sharing before its clustering step, ...) raises ``NotCapturable`` while graph mode
 is on rather than silently freezing a step index."""

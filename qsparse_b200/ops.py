@@ -692,26 +692,39 @@ def reduce_prune_quant_step(x, layout: Layout, magnitude, mask, scale, decimal_o
         N.stream_ptr(x.device)), "qsb_reduce_prune_quant_step_dt")
 
 
+def _step_route(channels: int, step_counter=None) -> str:
+    """The route of the structured prune -> quantize step by channel count (pow2 and line form alike):
+
+      <= FUSED_STEP_MAX_CHANNELS      "one"       stage 1 whose last-arriving CTA runs the step (one launch)
+      <= PARTIALS_ROUTE_MAX_CHANNELS  "partials"  stage 1 + the one-CTA step kernel on its partials
+      otherwise                       "stats"     finalized statistics + the step on rows (pow2 form only)
+
+    A device ``step_counter`` (CUDA graphs) is taken by the one-launch route only: with more channels this raises
+    ``graphs.NotCapturable``."""
+    if channels <= FUSED_STEP_MAX_CHANNELS:
+        return "one"
+    if step_counter is not None:
+        raise graphs.NotCapturable(f"the structured prune -> quantize step with more than {FUSED_STEP_MAX_CHANNELS} "
+                                   "channels")
+    return "partials" if channels <= PARTIALS_ROUTE_MAX_CHANNELS else "stats"
+
+
 def structured_prune_quant_step(x, layout: Layout, magnitude, mask, scale, decimal_out, count: float, t_prune: int,
                                 update_magnitude: int, refresh_mask, k: int, bits: int, t_quant: int,
                                 update_scale: bool, group=None, step_stamp: int = 1, step_counter=None):
-    """The structured prune -> pow2 quantize parameter step on x, by channel count:
+    """The structured prune -> pow2 quantize parameter step on x, by channel count (``_step_route``):
 
-      <= FUSED_STEP_MAX_CHANNELS      reduce_prune_quant_step (one launch)
-      <= PARTIALS_ROUTE_MAX_CHANNELS  reduce_partials + prune_quant_step_params
-      otherwise                       reduce_stats + prune_quant_params (single GPU only)
+      one       reduce_prune_quant_step
+      partials  reduce_partials + prune_quant_step_params
+      stats     reduce_stats + prune_quant_params (single GPU only)
 
-    Arguments as in ``reduce_prune_quant_step``.  ``step_counter`` (CUDA graphs) is taken by the one-launch
-    route only: with more channels this raises ``graphs.NotCapturable``."""
-    ch = layout[1]
-    if ch <= FUSED_STEP_MAX_CHANNELS:
+    Arguments as in ``reduce_prune_quant_step``."""
+    route = _step_route(layout[1], step_counter)
+    if route == "one":
         reduce_prune_quant_step(x, layout, magnitude, mask, scale, decimal_out, count, t_prune, update_magnitude,
                                 refresh_mask, k, bits, t_quant, update_scale, group=group, step_stamp=step_stamp,
                                 step_counter=step_counter)
-    elif step_counter is not None:
-        raise graphs.NotCapturable(f"the structured prune -> quantize step with more than {FUSED_STEP_MAX_CHANNELS} "
-                                   "channels")
-    elif ch <= PARTIALS_ROUTE_MAX_CHANNELS:
+    elif route == "partials":
         ws = reduce_partials(x, layout)
         prune_quant_step_params(magnitude, mask, scale, decimal_out, ws, layout, count, t_prune, update_magnitude,
                                 refresh_mask, k, bits, t_quant, update_scale, group=group, step_stamp=step_stamp)
@@ -721,6 +734,75 @@ def structured_prune_quant_step(x, layout: Layout, magnitude, mask, scale, decim
         stats = reduce_stats(x, layout, absmax=True, abssum=True)
         prune_quant_params(magnitude, mask, scale, decimal_out, stats, count, t_prune, update_magnitude,
                            refresh_mask, k, bits, t_quant, update_scale)
+
+
+# ----------------------------------------------------------------------------- the line form (AdaptiveQuantizer)
+def reduce_prune_line_step(x, layout: Layout, magnitude, mask, lines, count: float, t_prune: int,
+                           update_magnitude: int, refresh_mask, k: int, t_line: int, abssum_out=None, min_out=None,
+                           max_out=None, step_counter=None, arrival=None):
+    """ONE launch: sum|x| / min / max reduction of x whose last-arriving CTA updates magnitude / mask and the
+    ``lines`` [n, 2] (n == 1 or channels) of an AdaptiveQuantizer from the (min, max) of x * mask, at its call index
+    ``t_line`` (1-based; an offset to ``*step_counter`` when that is given).  Up to FUSED_STEP_MAX_CHANNELS."""
+    N.require_cuda(x, "input")
+    if step_counter is not None:
+        N.require_cuda(step_counter, "step_counter")
+    lib = N.load_library()
+    outer, ch, inner = layout
+    ws = N.workspace(x.device, lib.qsb_reduce_workspace_bytes(c_int64(outer), c_int64(ch), c_int64(inner)))
+    N.check(lib.qsb_reduce_prune_line_step_dt(
+        N.ptr(x), c_int(N.dtype_code(x)), c_int64(outer), c_int64(ch), c_int64(inner), N.ptr(ws), c_int64(ws.numel()),
+        N.ptr(arrival if arrival is not None else arrival_counter(x.device)), N.ptr(magnitude), N.ptr(mask),
+        N.ptr(lines), c_int64(lines.numel() // 2), None, c_double(count), c_int64(t_prune), c_int(update_magnitude),
+        c_int(int(refresh_mask)), c_int64(k), c_int64(t_line), N.ptr(abssum_out), N.ptr(min_out), N.ptr(max_out),
+        N.ptr(step_counter), N.stream_ptr(x.device)), "qsb_reduce_prune_line_step_dt")
+
+
+def reduce_line_partials(x, layout: Layout):
+    """Stage 1 of the sum|x| / min / max reduction only; the partials stay in the returned workspace for
+    ``prune_line_step_params``."""
+    N.require_cuda(x, "input")
+    lib = N.load_library()
+    outer, ch, inner = layout
+    ws = N.workspace(x.device, lib.qsb_reduce_workspace_bytes(c_int64(outer), c_int64(ch), c_int64(inner)))
+    N.check(lib.qsb_reduce_line_partials_dt(N.ptr(x), c_int(N.dtype_code(x)), c_int64(outer), c_int64(ch),
+                                            c_int64(inner), N.ptr(ws), c_int64(ws.numel()), N.stream_ptr(x.device)),
+            "qsb_reduce_line_partials_dt")
+    return ws
+
+
+def prune_line_step_params(magnitude, mask, lines, workspace, layout: Layout, count: float, t_prune: int,
+                           update_magnitude: int, refresh_mask, k: int, t_line: int, abssum_out=None, min_out=None,
+                           max_out=None, step_counter=None):
+    """the line step as one one-CTA kernel on the partials of ``reduce_line_partials`` (up to 2048 channels)"""
+    lib = N.load_library()
+    outer, ch, inner = layout
+    N.check(lib.qsb_prune_line_step_params(
+        N.ptr(magnitude), N.ptr(mask), N.ptr(lines), c_int64(lines.numel() // 2), N.ptr(workspace),
+        c_int64(workspace.numel()), c_int64(outer), c_int64(ch), c_int64(inner), None, c_double(count),
+        c_int64(t_prune), c_int(update_magnitude), c_int(int(refresh_mask)), c_int64(k), c_int64(t_line),
+        N.ptr(abssum_out), N.ptr(min_out), N.ptr(max_out), N.ptr(step_counter), N.stream_ptr(mask.device)),
+        "qsb_prune_line_step_params")
+
+
+def structured_prune_line_step(x, layout: Layout, magnitude, mask, lines, count: float, t_prune: int,
+                               update_magnitude: int, refresh_mask, k: int, t_line: int, step_counter=None):
+    """The structured prune -> AdaptiveQuantizer parameter step on x, on the route ``_step_route`` picks:
+
+      one       reduce_prune_line_step
+      partials  reduce_line_partials + prune_line_step_params
+
+    Above PARTIALS_ROUTE_MAX_CHANNELS channels there is no line route: ``ValueError``."""
+    route = _step_route(layout[1], step_counter)
+    if route == "one":
+        reduce_prune_line_step(x, layout, magnitude, mask, lines, count, t_prune, update_magnitude, refresh_mask, k,
+                               t_line, step_counter=step_counter)
+    elif route == "partials":
+        ws = reduce_line_partials(x, layout)
+        prune_line_step_params(magnitude, mask, lines, ws, layout, count, t_prune, update_magnitude, refresh_mask, k,
+                               t_line)
+    else:
+        raise ValueError(f"the structured prune -> line quantize step takes at most {PARTIALS_ROUTE_MAX_CHANNELS} "
+                         "channels")
 
 
 def prune_quant_rows_step_params(magnitude, mask, scale, decimal_out, stats: dict, count: float, t_prune: int,
