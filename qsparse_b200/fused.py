@@ -38,20 +38,33 @@ from . import _native as N
 from . import graphs
 from . import ops
 from .parallel import StatExchange, make_exchange
+from .quantize import _grad_buffer, _physical_layout
 from .util import kth_rank
+
+
+def _walked(t, axis):
+    """(t, (outer, C, inner) of its memory around ``axis``; axis < 0: per tensor): a contiguous or 4-D channels_last
+    tensor as it is (the result keeps its memory format), anything else as a contiguous copy"""
+    return _physical_layout(t, axis, axis >= 0)
+
+
+def _grad_walked(grad_output, axis):
+    """grad_output as the backward kernels read it: fp32, and, unless it is contiguous or 4-D channels_last, a
+    contiguous copy; with its (outer, C, inner) around ``axis``"""
+    return _walked(_grad_buffer(grad_output), axis)
 
 
 class _PruneQuantizeFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, layer):
         ctx.layer = layer
-        ctx.layout = layer._layout(x)
-        ctx.x_dtype = N.as_native(x).dtype
-        return layer._forward_impl(x, ctx.layout)
+        xs, layout = _walked(N.as_native(x.detach()), layer.channel_index)
+        ctx.x_dtype = xs.dtype
+        return layer._forward_impl(xs, layout)
 
     @staticmethod
     def backward(ctx, grad_output):
-        return ctx.layer.backward_kernel(grad_output, ctx.layout, ctx.x_dtype), None
+        return ctx.layer.backward_kernel(grad_output, ctx.x_dtype), None
 
 
 class PruneQuantize(nn.Module):
@@ -74,9 +87,6 @@ class PruneQuantize(nn.Module):
         self.t_prune = 0   # MagnitudePruningCallback.t
         self.t_quant = 0   # DecimalQuantizer.t
         self._exchange: Optional[StatExchange] = None
-
-    def _layout(self, x):
-        return N.channel_layout(x.shape, self.channel_index)
 
     def _step_counter(self, device):
         """device twin of ``t_prune`` for graph mode (created outside capture by ``GraphedTrainStep``)"""
@@ -104,9 +114,9 @@ class PruneQuantize(nn.Module):
         # NCCL all-gather path only when peer memory is unavailable (or takes more channels than it exchanges)
         self._exchange = StatExchange(channels, dev, self.group) if multi and self._p2p is None else True
 
-    def _forward_impl(self, x, layout):
+    def _forward_impl(self, xs, layout):
+        """xs: x as ``_walked`` returns it (bf16 / fp16 read natively, y is fp32 in xs's memory format)"""
         outer, ch, inner = layout
-        xs = N.as_native_contiguous(x.detach())   # bf16 / fp16 read natively, y is fp32
         if self._exchange is None:
             self._allocate(xs, ch)
         if self.training:
@@ -150,9 +160,10 @@ class PruneQuantize(nn.Module):
             self.t_quant += 1
         return ops.fq_pow2_fwd(xs, self.decimal, layout, mask=self.mask.data)
 
-    def backward_kernel(self, g, layout, x_dtype=torch.float32):
-        """gx in ``x_dtype`` (the input's dtype: bf16 / fp16 are written directly, rounded like autograd's cast)"""
-        g = N.as_f32_contiguous(g)
+    def backward_kernel(self, g, x_dtype=torch.float32):
+        """gx in ``x_dtype`` (the input's dtype: bf16 / fp16 are written directly, rounded like autograd's cast) and
+        in g's memory format"""
+        g, layout = _grad_walked(g, self.channel_index)
         _, gx = ops.ste_bwd(g, self.decimal, True, self.bits, 0, layout, mask=self.mask.data,
                             clamp_in_place=self.mutate_grad_output, want_gx=True, gx_dtype=x_dtype)
         return gx
@@ -163,15 +174,28 @@ class PruneQuantize(nn.Module):
 
 
 # ----------------------------------------------------------------------------- fusion pass (SURVEY §8 f-1)
+def _site_layout(x, d):
+    """(outer, C, inner) of x's memory around the prune axis ``d`` when the fused step walks x without a copy:
+    contiguous with ``1 <= d < x.dim()`` (the last axis gives [rows, C, 1]), or 4-D channels_last with ``d == 1``
+    ([N*H*W, C, 1]); None for every other layout"""
+    if not 1 <= d < x.dim():
+        return None
+    if x.is_contiguous() or (d == 1 and x.dim() == 4 and x.is_contiguous(memory_format=torch.channels_last)):
+        return _physical_layout(x, d, True)[1]
+    return None
+
+
 class _FusedLayersFn(torch.autograd.Function):
     """forward value and backward of ``QuantizeLayer(PruneLayer(x))`` in its steady state, on the two
     layers' own state tensors: y = Q(x * mask), gx = clamp(g) * mask (grad_output clamped in place, like
-    DecimalQuantization.backward does, ref quantize.py:65-77, sparse.py backward of x * mask)."""
+    DecimalQuantization.backward does, ref quantize.py:65-77, sparse.py backward of x * mask).  xs is walked in
+    ``layout`` (its memory around the prune axis ``axis``), so y keeps x's memory format; the backward walks
+    grad_output in its own memory, so gx keeps g's."""
 
     @staticmethod
-    def forward(ctx, x, xs, layout, mask, param, bits, notch, is_decimal):
+    def forward(ctx, x, xs, layout, axis, mask, param, bits, notch, is_decimal):
         # param: the step's decimal (DecimalQuantizer) or the layer's scale itself (ScalerQuantizer)
-        ctx.layout, ctx.mask, ctx.param, ctx.bits, ctx.notch = layout, mask, param, bits, notch
+        ctx.axis, ctx.mask, ctx.param, ctx.bits, ctx.notch = axis, mask, param, bits, notch
         ctx.is_decimal = is_decimal
         ctx.x_dtype = xs.dtype     # bf16 / fp16 activations: gx is written in their dtype
         if is_decimal:
@@ -180,14 +204,10 @@ class _FusedLayersFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_output):
-        g = grad_output
-        if g.dtype != torch.float32:
-            g = g.float()
-        if not g.is_contiguous():
-            g = g.contiguous()
-        _, gx = ops.ste_bwd(g, ctx.param, ctx.is_decimal, ctx.bits, ctx.notch, ctx.layout, mask=ctx.mask,
+        g, layout = _grad_walked(grad_output, ctx.axis)
+        _, gx = ops.ste_bwd(g, ctx.param, ctx.is_decimal, ctx.bits, ctx.notch, layout, mask=ctx.mask,
                             clamp_in_place=True, want_gx=True, gx_dtype=ctx.x_dtype)
-        return (gx,) + (None,) * 7
+        return (gx,) + (None,) * 8
 
 
 class _FusedLineLayersFn(torch.autograd.Function):
@@ -196,14 +216,14 @@ class _FusedLineLayersFn(torch.autograd.Function):
     grad_output is read, never written."""
 
     @staticmethod
-    def forward(ctx, x, xs, layout, mask, lines, bits):
-        ctx.layout, ctx.mask, ctx.x_dtype = layout, mask, xs.dtype
+    def forward(ctx, x, xs, layout, axis, mask, lines, bits):
+        ctx.axis, ctx.mask, ctx.x_dtype = axis, mask, xs.dtype
         return ops.fq_line_fwd(xs, lines, bits, True, layout, mask=mask).view(x.shape)
 
     @staticmethod
     def backward(ctx, grad_output):
-        g = N.as_f32_contiguous(grad_output)
-        return (ops.mask_apply(g, ctx.mask, ctx.layout, out_dtype=ctx.x_dtype),) + (None,) * 5
+        g, layout = _grad_walked(grad_output, ctx.axis)
+        return (ops.mask_apply(g, ctx.mask, layout, out_dtype=ctx.x_dtype),) + (None,) * 6
 
 
 class FusedPruneQuantSequential(nn.Sequential):
@@ -214,12 +234,15 @@ class FusedPruneQuantSequential(nn.Sequential):
     the mask folded in: 20 B/elem with the backward, instead of ~60 + 16).
 
     A step is fused only when it is provably the plain case: both layers initialised, training, structured
-    channel prune (``dimensions={1}``) by the stock ``MagnitudePruningCallback`` (no gradient / l0 / hook
-    variants), pruning started and the sparsity not changing at this step, past the quantizer's timeout, with
-    a per-tensor stock ``DecimalQuantizer`` or ``ScalerQuantizer`` (``quantize()``'s default callback) or a
-    stock ``AdaptiveQuantizer`` (per tensor, or per channel on the prune axis) after its first estimate.  Every other step (warm-up, ramp steps, eval, other callbacks,
-    non-contiguous inputs) runs the two layers one after the other, exactly as before.  Counters and
-    parameters advance identically either way, so the two routes can alternate freely."""
+    prune along one axis ``d`` (``dimensions={d}``) by the stock ``MagnitudePruningCallback`` (no gradient / l0 /
+    hook variants), pruning started and the sparsity not changing at this step, past the quantizer's timeout,
+    with a per-tensor stock ``DecimalQuantizer`` or ``ScalerQuantizer`` (``quantize()``'s default callback) or a
+    stock ``AdaptiveQuantizer`` (per tensor, or per channel on the prune axis) after its first estimate, on an
+    input the kernels walk without a copy (``_site_layout``): contiguous with ``d >= 1`` (``[N, C, H, W]`` on
+    axis 1, ``[tokens, hidden]`` or ``[B, T, H]`` on the last axis) or a 4-D ``channels_last`` tensor with
+    ``d == 1``.  Every other step (warm-up, ramp steps, eval, other callbacks, other layouts) runs the two layers
+    one after the other, exactly as before.  Counters and parameters advance identically either way, so the two
+    routes can alternate freely."""
 
     fused_steps = 0  # how many forwards took the fused route (per instance once incremented)
 
@@ -236,7 +259,10 @@ class FusedPruneQuantSequential(nn.Sequential):
         if not (isinstance(p, PruneLayer) and isinstance(q, QuantizeLayer) and self.training and p.training
                 and q.training):
             return False
-        if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dim() >= 2 and x.is_contiguous()):
+        if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dim() >= 2 and len(p.dimensions) == 1):
+            return False
+        d = next(iter(p.dimensions))
+        if _site_layout(x, d) is None:
             return False
         cb, qcb = p.callback, q.callback
         if type(cb) is not MagnitudePruningCallback or type(qcb) not in (DecimalQuantizer, ScalerQuantizer,
@@ -244,9 +270,9 @@ class FusedPruneQuantSequential(nn.Sequential):
             return False
         if cb.use_gradient or cb.l0 or cb.forward_hook is not None or not cb.training or not qcb.training:
             return False
-        if p.dimensions != {1} or not p.initted or not q.initted or p.mask.numel() == 1:
+        if not p.initted or not q.initted or p.mask.numel() == 1:
             return False
-        if p.mask.numel() != x.shape[1] or p.mask.numel() > ops.PARTIALS_ROUTE_MAX_CHANNELS:
+        if p.mask.numel() != x.shape[d] or p.mask.numel() > ops.PARTIALS_ROUTE_MAX_CHANNELS:
             return False
         n = p._n_mirror.get(p._n_updates)
         if n < p.start or n in p.schedules:
@@ -263,7 +289,7 @@ class FusedPruneQuantSequential(nn.Sequential):
             # lines per tensor or per channel of the prune axis; not before the first optimize(), which may
             # re-create `t` (like _fused_weight_step)
             rows = 1 if q.channelwise < 0 else p.mask.numel()
-            if q.channelwise >= 0 and q.channelwise != 1:
+            if q.channelwise >= 0 and q.channelwise != d:
                 return False
             if tuple(q.weight.shape) != (rows, 2) or not q.weight.is_contiguous():
                 return False
@@ -277,9 +303,10 @@ class FusedPruneQuantSequential(nn.Sequential):
     def _fused_step(self, p, q, x):
         from .quantize import AdaptiveQuantizer
         cb, qcb = p.callback, q.callback
-        layout = N.channel_layout(x.shape, 1)
+        axis = next(iter(p.dimensions))
+        layout = _site_layout(x, axis)
         outer, ch, inner = layout
-        xs = N.as_native_contiguous(x.detach())   # bf16 / fp16 read natively
+        xs = N.as_native(x.detach())   # bf16 / fp16 read natively, in x's memory format
         sparsity = p._s_mirror.get(p._cur_sparsity)
         t = cb._t()
         refresh = (t % cb.mask_refresh_interval == 0 and t <= cb.stop_mask_refresh) and \
@@ -338,8 +365,8 @@ class FusedPruneQuantSequential(nn.Sequential):
             q._t_mirror.wrote(q._n_updates, tq + 1)
         self.fused_steps += 1
         if line:
-            return _FusedLineLayersFn.apply(x, xs, layout, p.mask.data.view(-1), q.weight.data, q.bits)
-        return _FusedLayersFn.apply(x, xs, layout, p.mask.data.view(-1),
+            return _FusedLineLayersFn.apply(x, xs, layout, axis, p.mask.data.view(-1), q.weight.data, q.bits)
+        return _FusedLayersFn.apply(x, xs, layout, axis, p.mask.data.view(-1),
                                     decimal if is_decimal else q.weight.data.view(-1), q.bits,
                                     1 if qcb.flip_axis else 0, is_decimal)
 
