@@ -40,14 +40,11 @@ ops.magnitude_ema_full_(magf, wt, 3)
 thr = ops.kth_value(magf, n4 // 2)
 mk = torch.empty(n4, dtype=torch.bool, device=dev)
 ops.mask_build_apply(magf, thr, wt, mk)
-# config 3 through the row-resident fused kernel (register and TMA variants)
+# config 3 through the row-resident fused kernel
 lines2 = torch.zeros(4096, 2, device=dev)
 ops.row_quant_fused_(w, lines2, ops.ROW_LINE, 4, 1, True)
 sc2 = torch.zeros(4096, 1, device=dev)
 ops.row_quant_fused_(w, sc2, ops.ROW_SCALER, 4, 0)
-ops.set_tuning(9, 1)
-ops.row_quant_fused_(w, lines2, ops.ROW_LINE, 4, 2, True)
-ops.set_tuning(9, 0)
 # config 4 as a weight set: multi-tensor EMA, batched select, multi-tensor mask build + apply
 del wt, magf, mk
 from qsparse_b200 import parallel  # noqa: E402

@@ -21,14 +21,11 @@ ops.kth_value(v[: 100003], 5000)
 ops.kth_value(v[1: 70001], 5000)
 vs = [torch.randn(s, device=dev, generator=g) for s in (200_000, 131_072, 999, 300_000)]
 ops.kth_value_batched(vs, [s.numel() // 2 for s in vs])
-# row-resident kernels: warp per row, CTA per row, TMA variant
+# row-resident kernels: warp per row, CTA per row
 for shape in ((33, 8), (64, 288), (130, 1024), (48, 4096), (3, 8200), (2, 16384)):
     x = torch.randn(shape, device=dev, generator=g)
     for kind, w in ((ops.ROW_LINE, 2), (ops.ROW_SCALER, 1), (ops.ROW_DECIMAL, 1)):
-        for variant in (0, 1):
-            ops.set_tuning(9, variant)
-            ops.row_quant_fused_(x, torch.zeros(shape[0], w, device=dev), kind, 4, 1 if kind == ops.ROW_LINE else 0)
-ops.set_tuning(9, 0)
+        ops.row_quant_fused_(x, torch.zeros(shape[0], w, device=dev), kind, 4, 1 if kind == ops.ROW_LINE else 0)
 # multi-tensor EMA / mask, weight-set step
 shapes = [(64, 32, 3, 3), (40, 1000), (7, 13, 5), (256, 64, 3, 3)]
 ws = [torch.randn(s, device=dev, generator=g) for s in shapes]
@@ -62,8 +59,8 @@ ops.fq_line_fwd(x, torch.tensor([[-0.1, 0.9]] * 16, device=dev), 8, True, layout
 ops.fq_scaler_fwd(x, 0.037, (1, 1, x.numel()))
 ops.quant_export_int8(x, ops.EXPORT_DECIMAL, 4.0, 8, (1, 1, x.numel()))
 ops.quant_export_int8(x, ops.EXPORT_LINE, torch.tensor([[-0.1, 0.9]] * 16, device=dev), 8, layout)
-# short-row / channel-last layouts: tile reduction (several visits, ragged tiles, 4-byte-aligned view), transposed
-# finalize, row-lane column reduction, group-resident channel-last maps, straddling vectors, packed int4 export
+# short-row / channel-last layouts: column reduction (4-byte-aligned views), transposed finalize, row-lane column
+# reduction, group-resident channel-last maps, straddling vectors, packed int4 export
 for lay, off in (((300, 24, 196), 0), ((40, 96, 64), 3), ((9, 700, 100), 1), ((2100, 8, 255), 5), ((5000, 24, 1), 0),
                  ((600, 1000, 1), 0), ((64, 96, 49), 0)):
     n_ = lay[0] * lay[1] * lay[2]

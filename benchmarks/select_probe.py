@@ -61,15 +61,7 @@ for name, v, take_abs in cases():
         if ref is not None:
             got = ops.kth_value(v, k, take_abs=take_abs)
             ok = bool((got == ref[k]).item())
-        res = {}
-        for per in (1, 2, 4):
-            ops.set_tuning(7, per)
-            res[per] = timed(lambda: ops.kth_value(v, k, take_abs=take_abs))[0]
-        ops.set_tuning(7, 4)
-        ops.set_tuning(8, 0)
-        med2 = timed(lambda: ops.kth_value(v, k, take_abs=take_abs))[0]
-        ops.set_tuning(8, 1)
-        print(json.dumps(dict(case=name, frac=frac, ok=ok, us_8k=round(res[1], 2), us_16k=round(res[2], 2),
-                              us_32k=round(res[4], 2), us_32k_nopdl=round(med2, 2),
-                              gbs=round(4 * n / res[4] / 1e3, 1))), flush=True)
+        med = timed(lambda: ops.kth_value(v, k, take_abs=take_abs))[0]
+        print(json.dumps(dict(case=name, frac=frac, ok=ok, us_32k=round(med, 2), gbs=round(4 * n / med / 1e3, 1))),
+              flush=True)
     del ref

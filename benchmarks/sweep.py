@@ -4,7 +4,7 @@
 
 Times every hot-path kernel with CUDA events on the launching stream; between timed
 launches a 512 MB buffer is rewritten to flush the 126 MB L2.  GB/s = algorithmic bytes
-(SURVEY §8d table) / time.  Also sweeps the grid policy knob (qsb_set_tuning key 0).
+(SURVEY §8d table) / time.
 """
 import argparse
 import json
@@ -74,26 +74,17 @@ def main():
     emask = torch.rand(shape, device=dev) > 0.5
 
     report("torch_copy", 8 * n, lambda: y.copy_(x))
-    for tune in ([0] if args.quick else [0, 4, 8]):      # per-tensor grid policy (key 0)
-        ops.set_tuning(0, tune)
-        report("fq_pow2_tensor", 8 * n, lambda: ops.fq_pow2_fwd(x, dec1, (1, 1, n), out=y), tune0=tune)
-        report("ste_bwd_inplace", 8 * n, lambda: ops.ste_bwd(g, dec1, True, 8, 0, (1, 1, n)), tune0=tune)
-    ops.set_tuning(0, 0)
-    for tune in ([0] if args.quick else [0, -1, 3, 8]):   # per-channel grid policy (key 1)
-        ops.set_tuning(1, tune)
-        report("fq_pow2_chdec", 8 * n, lambda: ops.fq_pow2_fwd(x, decC, layout, out=y), tune1=tune)
-        report("fq_pow2_chmask0", 8 * n, lambda: ops.fq_pow2_fwd(x, dec1, layout, mask=mask0, out=y), tune1=tune)
-        report("fq_pow2_chmask75", 8 * n, lambda: ops.fq_pow2_fwd(x, dec1, layout, mask=mask75, out=y), tune1=tune,
-               note="dense-algorithmic bytes; 75% of reads skipped")
-    ops.set_tuning(1, 0)
+    report("fq_pow2_tensor", 8 * n, lambda: ops.fq_pow2_fwd(x, dec1, (1, 1, n), out=y))
+    report("ste_bwd_inplace", 8 * n, lambda: ops.ste_bwd(g, dec1, True, 8, 0, (1, 1, n)))
+    report("fq_pow2_chdec", 8 * n, lambda: ops.fq_pow2_fwd(x, decC, layout, out=y))
+    report("fq_pow2_chmask0", 8 * n, lambda: ops.fq_pow2_fwd(x, dec1, layout, mask=mask0, out=y))
+    report("fq_pow2_chmask75", 8 * n, lambda: ops.fq_pow2_fwd(x, dec1, layout, mask=mask75, out=y),
+           note="dense-algorithmic bytes; 75% of reads skipped")
     report("fq_pow2_emask", 9 * n, lambda: ops.fq_pow2_fwd(x, dec1, (1, 1, n), mask=emask, out=y))
     report("fq_scaler_tensor", 8 * n, lambda: ops.fq_scaler_fwd(x, 0.037, (1, 1, n), out=y))
     report("fq_line_tensor", 8 * n, lambda: ops.fq_line_fwd(x, (-0.1, 0.9), 8, True, (1, 1, n), out=y))
     lines64 = torch.tensor([[-0.1, 0.9]] * 64, device=dev)
-    for tune in (0, -1):
-        ops.set_tuning(1, tune)
-        report("fq_line_ch", 8 * n, lambda: ops.fq_line_fwd(x, lines64, 8, True, layout, out=y), tune1=tune)
-    ops.set_tuning(1, 0)
+    report("fq_line_ch", 8 * n, lambda: ops.fq_line_fwd(x, lines64, 8, True, layout, out=y))
 
     def bwd_fused():
         lib_gx = ops.N.load_library()
@@ -101,10 +92,7 @@ def main():
         ops.N.check(lib_gx.qsb_ste_bwd(ops.N.ptr(g), ops.N.ptr(None), ops.N.ptr(gx), ops.N.ptr(dec1), c_int64(1),
                                        c_double(0), c_int(1), c_int(8), c_int(0), ops.N.ptr(mask75), c_int(1),
                                        c_int64(256), c_int64(64), c_int64(3136), ops.N.stream_ptr(dev)), "ste")
-    for tune in ([0] if args.quick else [0, -1, 8]):
-        ops.set_tuning(1, tune)
-        report("ste_bwd_fused_gx", 8 * n, bwd_fused, tune1=tune)
-    ops.set_tuning(1, 0)
+    report("ste_bwd_fused_gx", 8 * n, bwd_fused)
     report("export_int8_pow2_ch", 5 * n, lambda: ops.quant_export_int8(x, ops.EXPORT_DECIMAL, decC, 8, layout),
            note="4 B read + 1 B written per element")
     report("export_int4_pow2_ch", 4.5 * n,
@@ -169,11 +157,6 @@ def main():
     st = ops.reduce_stats(w, (1, 4096, 4096), minmax=True)
     ops.lines_ema_(lines, st["min"], st["max"], 1)
     report("c3_line_fwd", 8 * nw, lambda: ops.fq_line_fwd(w, lines, 4, True, (1, 4096, 4096), out=wy))
-    for seg in (512, 1024, 2048, 4096):
-        ops.set_tuning(3, seg)
-        report("c3_reduce_minmax", 4 * nw, lambda: ops.reduce_stats(w, (1, 4096, 4096), minmax=True), seg_min=seg)
-        report("reduce_abssum_absmax_ch", 4 * n, lambda: ops.reduce_stats(x, layout, abssum=True, absmax=True), seg_min=seg)
-    ops.set_tuning(3, 1024)
 
     def c3_access():      # the real weight access: reduce -> EMA -> line quant, back to back (W stays in L2)
         st_ = ops.reduce_stats(w, (1, 4096, 4096), minmax=True)
@@ -187,15 +170,6 @@ def main():
            note="8 B/elem actual traffic")
     report("c3_weight_access_fused_alg12", 12 * nw,
            lambda: ops.row_quant_fused_(w, lines2, ops.ROW_LINE, 4, 2, True), note="12 B/elem dense-algorithmic")
-    ops.set_tuning(9, 1)
-    for per_sm, stages in ((3, 4), (6, 2)):
-        ops.set_tuning(10, per_sm)
-        ops.set_tuning(11, stages)
-        report("c3_weight_access_fused", 8 * nw, lambda: ops.row_quant_fused_(w, lines2, ops.ROW_LINE, 4, 2, True),
-               variant="TMA-pipelined persistent", ctas_per_sm=per_sm, stages=stages)
-    ops.set_tuning(10, 0)
-    ops.set_tuning(11, 0)
-    ops.set_tuning(9, 0)
     sc2 = torch.zeros(4096, 1, device=dev)
     report("c3_weight_access_fused_scaler", 8 * nw, lambda: ops.row_quant_fused_(w, sc2, ops.ROW_SCALER, 4, 1))
     report("c3_weight_access_fused_decimal", 8 * nw, lambda: ops.row_quant_fused_(w, sc2, ops.ROW_DECIMAL, 4, 1))

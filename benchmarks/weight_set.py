@@ -11,7 +11,7 @@ from pathlib import Path
 import torch
 
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
-from qsparse_b200 import ops, parallel  # noqa: E402
+from qsparse_b200 import parallel  # noqa: E402
 
 dev = torch.device("cuda:0")
 torch.manual_seed(4)
@@ -49,14 +49,6 @@ def timed(fn, iters=8):
     return ts[len(ts) // 2]
 
 
-if "--tune" in sys.argv:
-    for per in (1, 2, 4):
-        for sig in (30, 35, 45):
-            ops.set_tuning(13, per)
-            ops.set_tuning(14, sig)
-            print(json.dumps(dict(kernel="c4_weight_set_step", samples_k=8 * per, sigma=sig / 10, us=round(timed(step), 1))))
-    ops.set_tuning(13, 4)
-    ops.set_tuning(14, 35)
 t_eager = timed(step)
 side = torch.cuda.Stream()
 side.wait_stream(torch.cuda.current_stream())

@@ -64,49 +64,27 @@ int qsb_device_info(int *sm_count, int64_t *l2_bytes);
  * otherwise reads 3 x 2 x 256 uint64 %globaltimer stamps [statistics / forward / backward kernel][first CTA
  * start, last CTA end][SM] — the in-situ durations of a graph-replayed step without event records. */
 int qsb_debug_kernel_times(unsigned long long *out_host, void *stream);
-/* Benchmark-only knobs; defaults are what the product uses.
- *   key 0: per-tensor streaming kernels: 0 = one CTA per tile (default),
- *          n > 0 = persistent grid of n CTAs per SM;
- *   key 1: per-channel streaming kernels: 0 = occupancy-derived persistent
- *          grid (default), n > 0 = n CTAs per SM;
+/* Benchmark knobs and one test hook; defaults are what the product uses.
  *   key 2: tile order of the one-CTA-per-tile kernels: 1 (default) = last tile first
  *          (re-reads the L2-resident tail of a just-touched tensor) except in the
  *          channel-masked kernels, which follow the fused statistics kernel and its
  *          L2 keep tags and measured faster first tile first; 2 = always last tile
  *          first; 0 = always first tile first;
- *   key 3: minimum segment length (elements) of the row reductions (default 1024);
- *   key 4: 1 = sampled-pivot ~1-pass route of qsb_kth_value for n >= 2^22
+ *   key 4: test hook: 1 = sampled-pivot ~1-pass route of qsb_kth_value for n >= 2^22
  *          (default), 0 = always the 3-pass radix select;
- *   key 6: 256-bit loads in flight per thread in the select's partition pass
- *          (2, 4 = default);
- *   key 7: samples per sampler thread of the select (1, 2, 4 = default ->
- *          8 Ki, 16 Ki, 32 Ki samples; 4 reads four neighbours per location);
- *   key 8: 1 = the kernels of one select are chained by programmatic dependent
- *          launch (default), 0 = ordinary stream order;
- *   key 9: qsb_row_quant_fused on rows of 1 Ki .. 16 Ki elements: 0 = register-
- *          resident one-CTA-per-row kernel (default), 1 = TMA-pipelined persistent kernel;
- *   key 10 / 11: persistent CTAs per SM (0 = up to 3) / ring stages (0 = auto) of the latter;
  *   key 12: 1 = the streaming, reduction and fused-parameter kernels are launched with
  *          programmatic stream serialization (each begins with griddepcontrol.wait, so
  *          stream order is unchanged; launch latency overlaps the predecessor's tail);
- *   key 13 / 14: fused prune step: samples per sampler thread (1, 2, 4 = default) / distance
- *          of the pivots from the estimated rank in tenths of a sigma (default 35);
- *   key 15: per-channel kernels on channel-last layouts (inner == 1, channels % 8 == 0):
- *          1 = a thread keeps one group of 8 channels in registers (default), 0 = table walk;
- *   key 16: column-mode reductions: most threads of a CTA along one row (32, 64 = default, 128, 256);
- *          the CTA's other threads walk interleaved rows and are combined in shared memory, so
- *          256 / value times fewer partials reach the finalize;
  *   key 17: row-mode statistics kernels: 2 = 8 x 256-bit loads in flight per lane, 2 CTAs / SM,
  *          0 = 4 loads, 4 CTAs / SM, any other value = by row length (default: 2 for rows of
  *          >= 2048 elements, else 0); the reduction plan — and with it the summation order — follows;
  *   key 18: 1 = qsb_reduce_prune_quant_step reads the channels the previous mask keeps with
  *          L2::evict_last (the forward pass re-reads exactly those next) and the rest with
  *          L2::evict_first (default), 0 = default policy for everything;
- *   key 20: statistics of rows up to this many elements use the column kernel on the
- *          [outer, channels * inner] view instead of the tile kernel (default 256; 0 = never);
  *   key 21: L2 set-aside for persisting accesses in MB (cudaLimitPersistingL2CacheSize, device-wide;
  *          untouched by default).  A development probe only: every set-aside >= 32 MB HALVED the
- *          speed of the streaming kernels on B200 (profiles/r02_l2_set_aside.jsonl). */
+ *          speed of the streaming kernels on B200 (profiles/r02_l2_set_aside.jsonl).
+ * Any other key returns QSB_E_BADARG. */
 int qsb_set_tuning(int key, int value);
 /* Test hook: compares the kernels' reciprocal-based exact division with
  * __fdiv_rn on n_threads * pairs_per_thread pseudo-random operand pairs and
@@ -266,8 +244,7 @@ int qsb_reduce_stats_fused(const float *x, int what, int64_t outer, int64_t chan
  * segments, row bands, vectors of 8, fp32 pre-sums and with them the summation order — is
  * the same function of the shape for every dtype (vectors are counted from x[0], i.e. as
  * for an fp32 x that starts on a 32-byte boundary), so a 16-bit x gives the statistics of
- * its fp32 copy bit for bit.  The tile kernel that tuning key 20 can select for short rows
- * is fp32 only: with it a 16-bit x returns QSB_E_UNSUPPORTED. */
+ * its fp32 copy bit for bit. */
 int qsb_reduce_stats_dt(const void *x, int x_dtype, int what, int64_t outer, int64_t channels,
                         int64_t inner, float *absmax, float *mn, float *mx,
                         double *abssum, double *nnz, float *tensor_min,

@@ -12,14 +12,6 @@
 #include "reduce_internal.cuh"
 namespace qsb {
 void set_select_fast(int v);
-void set_select_partition_u(int v);
-void set_select_sample_per(int v);
-void set_select_pdl(int v);
-void set_row_tma(int v);
-void set_row_ctas_per_sm(int v);
-void set_row_stages(int v);
-void set_step_sample_per(int v);
-void set_step_sigma10(int v);
 }
 
 namespace qsb {
@@ -36,9 +28,9 @@ int launch_map_big_out(const Op &op, const IO &io, const Layout &L, cudaStream_t
   return launch_map<Op, Hint::STREAM, Hint::KEEP>(op, io, L, stream);
 }
 
-MapTuning &map_tuning() {
-  static MapTuning t{0, 0, 1, 1};
-  return t;
+int &map_reverse_tiles() {
+  static int v = 1;
+  return v;
 }
 
 // ---------------------------------------------------------------------------
@@ -737,60 +729,16 @@ extern "C" int qsb_debug_kernel_times(unsigned long long *out_host, void *stream
 }
 
 extern "C" int qsb_set_tuning(int key, int value) {
-  if (key == 0) {
-    map_tuning().ctas_per_sm = value;
-    return 0;
-  }
-  if (key == 1) {
-    map_tuning().chan_ctas_per_sm = value;
-    return 0;
-  }
   if (key == 2) {
-    map_tuning().reverse_tiles = value;
-    return 0;
-  }
-  if (key == 3) {
-    set_reduce_seg_min(value);
+    map_reverse_tiles() = value;
     return 0;
   }
   if (key == 4) {
     set_select_fast(value);
     return 0;
   }
-  if (key == 6) {
-    set_select_partition_u(value);
-    return 0;
-  }
-  if (key == 7) {
-    set_select_sample_per(value);
-    return 0;
-  }
-  if (key == 8) {
-    set_select_pdl(value);
-    return 0;
-  }
-  if (key == 9) {
-    set_row_tma(value);
-    return 0;
-  }
-  if (key == 10) {
-    set_row_ctas_per_sm(value);
-    return 0;
-  }
-  if (key == 11) {
-    set_row_stages(value);
-    return 0;
-  }
   if (key == 12) {
     set_pdl_enabled(value);
-    return 0;
-  }
-  if (key == 15) {
-    map_tuning().lastdim = value;
-    return 0;
-  }
-  if (key == 16) {
-    set_reduce_col_tpr_wide(value);
     return 0;
   }
   if (key == 17) {
@@ -799,10 +747,6 @@ extern "C" int qsb_set_tuning(int key, int value) {
   }
   if (key == 18) {
     set_reduce_keep_hint(value);
-    return 0;
-  }
-  if (key == 20) {
-    set_reduce_col_max_inner(value);
     return 0;
   }
   if (key == 21) {
@@ -815,14 +759,6 @@ extern "C" int qsb_set_tuning(int key, int value) {
     size_t want = (size_t)(value < 0 ? 0 : value) << 20;
     if (want > (size_t)max_bytes) want = (size_t)max_bytes;
     QSB_CUDA_TRY(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want));
-    return 0;
-  }
-  if (key == 13) {
-    set_step_sample_per(value);
-    return 0;
-  }
-  if (key == 14) {
-    set_step_sigma10(value);
     return 0;
   }
   return QSB_E_BADARG;

@@ -18,10 +18,10 @@
 //                    MODE 0: inner % V == 0, a vector never straddles two rows;
 //                    MODE 1: a vector touches at most two channels.
 //   map_chan_kernel  rows shorter than a vector (inner < V, MODE 2: walk the
-//                    channels element by element) and unaligned pointers.
-//                    Persistent grid, full per-channel table in shared memory
-//                    when it fits, 32-bit (column, channel) bookkeeping advanced
-//                    by constants — no division in the loop.
+//                    channels element by element) and unaligned pointers (V = 1,
+//                    MODE 0).  Persistent grid, full per-channel table in shared
+//                    memory when it fits, 32-bit (column, channel) bookkeeping
+//                    advanced by constants — no division in the loop.
 #pragma once
 #include <type_traits>
 
@@ -102,26 +102,20 @@ __device__ __forceinline__ void store_outb(uint8_t *outb, int64_t e, const VecB<
   }
 }
 
-struct MapTuning {
-  int ctas_per_sm;   // per-tensor kernel: 0 = one CTA per tile (default); >0 persistent
-  int chan_ctas_per_sm;  // channel kernel: 0 = occupancy-derived persistent grid
-  // Tile order of the one-CTA-per-tile kernels.  1 (default): last tile first.  The
-  // tensor a streaming kernel reads was normally just produced / reduced front to
-  // back, so its TAIL is what still sits in the 126 MB L2; walking backwards turns
-  // up to ~100 MB of the second pass into L2 hits instead of HBM reads.
-  int reverse_tiles;
-  int lastdim;  // 1 (default): channel-last layouts use the group-resident kernel; 0: the MODE 2 walk
-};
-MapTuning &map_tuning();
+// Tile order of the one-CTA-per-tile kernels (tuning key 2).  1 (default): last tile first.  The
+// tensor a streaming kernel reads was normally just produced / reduced front to
+// back, so its TAIL is what still sits in the 126 MB L2; walking backwards turns
+// up to ~100 MB of the second pass into L2 hits instead of HBM reads.
+int &map_reverse_tiles();
 
-// reverse_tiles: 0 never, 1 (default) every map kernel EXCEPT the channel-masked ones, 2 always.  The masked
+// map_reverse_tiles(): 0 never, 1 (default) every map kernel EXCEPT the channel-masked ones, 2 always.  The masked
 // forward / backward follow the fused statistics kernel, which has already tagged the kept channels
 // L2::evict_last: there the natural order measured 3 us faster on the bench step (20.7 vs 25.5 MB of DRAM reads
 // in the forward, profiles/r02_tile_order.json), while the untagged pair {statistics -> quantize} gains 4 us
 // from walking backwards at every size above ~90 MB.
 template <class Op>
 inline int reverse_for() {
-  const int v = map_tuning().reverse_tiles;
+  const int v = map_reverse_tiles();
   return (v == 2 || (v == 1 && !Op::kCanSkip)) ? 1 : 0;
 }
 
@@ -189,11 +183,6 @@ int launch_map_tensor(const Op &op, const IO &io, int64_t n,
   constexpr int64_t kTile = (int64_t)QSB_THREADS * V * U;
   const int64_t tiles = (n + kTile - 1) / kTile;
   int64_t grid = tiles;
-  const int per_sm = map_tuning().ctas_per_sm;
-  if (per_sm > 0) {
-    grid = (int64_t)device_props().sm_count * per_sm;
-    if (grid > tiles) grid = tiles;
-  }
   if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;  // the kernel loops
   const int reverse = (grid == tiles && reverse_for<Op>()) ? 1 : 0;
   QSB_CUDA_TRY(launch_k(kern, dim3((unsigned)grid), dim3(QSB_THREADS), 0, stream, op, io, n, reverse));
@@ -365,14 +354,7 @@ __global__ void __launch_bounds__(QSB_THREADS)
       colu[u] = col;
       skipv[u] = false;
       if (e < n_main) {
-        if constexpr (Op::kCanSkip && MODE != 2) {
-          bool s = op.skip(param_of(c));
-          if (MODE == 1 && s && col + V > G.inner) {
-            const uint32_t c1 = (c + 1 >= G.channels) ? 0 : c + 1;
-            s = op.skip(param_of(c1));
-          }
-          skipv[u] = s;
-        }
+        if constexpr (Op::kCanSkip && MODE != 2) skipv[u] = op.skip(param_of(c));
         if (!skipv[u]) a[u] = ld_vec<V, LH>(io.in0 + e);
         if constexpr (Op::kIn1) b[u] = ld_vec<V, LH>(io.in1 + e);
         if constexpr (Op::kInB) mb[u] = ld_bytes<V>(io.inb + e);
@@ -400,35 +382,7 @@ __global__ void __launch_bounds__(QSB_THREADS)
             }
           }
         } else {
-          const P p0 = param_of(cu[u]);
-          const uint32_t left = G.inner - colu[u];  // elements left in this row
-          if (MODE == 0 || left >= (uint32_t)V) {
-            apply_vec<Op, V>(op, a[u], b[u], mb[u], skipv[u], p0, o0, o1, ob);
-          } else {
-            const uint32_t c1 = (cu[u] + 1 >= G.channels) ? 0 : cu[u] + 1;
-            const P p1 = param_of(c1);
-            // a vector across two rows: still the cheap arithmetic when both rows allow it (with
-            // 7x7 feature maps one vector in six straddles; the generic IEEE path on those alone
-            // made the line quantizer 2.4x slower than the pow2 one)
-            bool fast2 = Op::kHasFast;
-            if constexpr (Op::kHasFast)
-              fast2 = op.template fast<V>(p0, a[u].v) && op.template fast<V>(p1, a[u].v);
-            if (fast2) {
-              if constexpr (Op::kHasFast) {
-#pragma unroll
-                for (int j = 0; j < V; ++j)
-                  op.apply_fast(skipv[u] ? 0.f : a[u].v[j], Op::kIn1 ? b[u].v[j] : 0.f,
-                                Op::kInB ? mb[u].b[j] : (uint8_t)1,
-                                ((uint32_t)j < left) ? p0 : p1, o0.v[j], o1.v[j], ob.b[j]);
-              }
-            } else {
-#pragma unroll
-              for (int j = 0; j < V; ++j)
-                op.apply(skipv[u] ? 0.f : a[u].v[j], Op::kIn1 ? b[u].v[j] : 0.f,
-                         Op::kInB ? mb[u].b[j] : (uint8_t)1,
-                         ((uint32_t)j < left) ? p0 : p1, o0.v[j], o1.v[j], ob.b[j]);
-            }
-          }
+          apply_vec<Op, V>(op, a[u], b[u], mb[u], skipv[u], param_of(cu[u]), o0, o1, ob);
         }
         if constexpr (Op::kOut0) st_vec<V, SH>(io.out0 + e, o0);
         if constexpr (Op::kOut1) st_vec<V, SH>(io.out1 + e, o1);
@@ -547,7 +501,10 @@ __global__ void __launch_bounds__(QSB_THREADS)
         apply_vec<Op, V>(op, a[u], b[u], mb[u], skipv[u], p0, o0, o1, ob);
       } else {
         const P p1 = tab[ru[u] + (leftu[u] < (uint32_t)V ? 1 : 0)];
-        bool fast2 = Op::kHasFast;  // see map_chan_win_kernel: straddling vectors stay on the cheap path
+        // a vector across two rows: still the cheap arithmetic when both rows allow it (with 7x7 feature maps one
+        // vector in six straddles; the generic IEEE path on those alone made the line quantizer 2.4x slower than
+        // the pow2 one)
+        bool fast2 = Op::kHasFast;
         if constexpr (Op::kHasFast)
           fast2 = op.template fast<V>(p0, a[u].v) && op.template fast<V>(p1, a[u].v);
         if (fast2) {
@@ -621,10 +578,8 @@ int launch_map_chan_variant(const Op &op, const IO &io, int64_t n,
   QSB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern,
                                                              QSB_THREADS, smem));
   if (occ < 1) occ = 1;
-  const int per_sm = map_tuning().chan_ctas_per_sm;
   const int64_t tiles = (n + kTile - 1) / kTile;
-  int64_t grid = (int64_t)device_props().sm_count * (per_sm > 0 ? per_sm : occ);
-  if (per_sm < 0) grid = tiles;  // one CTA per tile
+  int64_t grid = (int64_t)device_props().sm_count * occ;
   if (grid > tiles) grid = tiles;
   if (grid < 1) grid = 1;
   if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
@@ -760,14 +715,9 @@ int launch_map(const Op &op, const IO &io, const Layout &L,
   }
   if (L.inner >= (1LL << 31) || L.channels >= (1LL << 31)) return QSB_E_UNSUPPORTED;
   if ((bits & 31) == 0) {
-    if (map_tuning().chan_ctas_per_sm == 0) {
-      if (L.inner % 8 == 0) return launch_map_chan_win<Op, 8, 2, 0, LH, SH, IO>(op, io, n, L, stream);
-      if (L.inner >= 8) return launch_map_chan_win<Op, 8, 2, 1, LH, SH, IO>(op, io, n, L, stream);
-    } else {  // benchmark knob: the persistent full-table kernel for every shape
-      if (L.inner % 8 == 0) return launch_map_chan_variant<Op, 8, 2, 0, LH, SH, IO>(op, io, n, L, stream);
-      if (L.inner >= 8) return launch_map_chan_variant<Op, 8, 2, 1, LH, SH, IO>(op, io, n, L, stream);
-    }
-    if (L.inner == 1 && L.channels % 8 == 0 && map_tuning().lastdim)
+    if (L.inner % 8 == 0) return launch_map_chan_win<Op, 8, 2, 0, LH, SH, IO>(op, io, n, L, stream);
+    if (L.inner >= 8) return launch_map_chan_win<Op, 8, 2, 1, LH, SH, IO>(op, io, n, L, stream);
+    if (L.inner == 1 && L.channels % 8 == 0)
       return launch_map_lastdim<Op, LH, SH, IO>(op, io, n, L, stream);
     return launch_map_chan_variant<Op, 8, 2, 2, LH, SH, IO>(op, io, n, L, stream);
   }

@@ -4,17 +4,14 @@
 // floating-point atomics).
 //
 // Stage 1 has two shapes:
-//   row mode    (inner >= 64): work items are (row, segment) pieces; a "virtual
+//   row mode    (inner > 256): work items are (row, segment) pieces; a "virtual
 //                warp" v owns items v, v + W, v + 2W, ... where W is a multiple of
 //                channels * segments_per_row, so all its items belong to ONE
 //                channel: it accumulates them in registers and writes a single
 //                partial at the end (W partials in total instead of one per item).
 //                256-bit loads, 4 in flight per lane, scalar head/tail peel for
 //                pieces that do not start on a 32-byte boundary;
-//   tile mode   (64 <= inner <= 256, short rows): same partial layout as row mode, but a
-//                CTA stages 32 consecutive rows per visit in shared memory with aligned,
-//                coalesced loads and a warp reduces a row from there (reduce_tile_kernel);
-//   column mode (inner  < 64): the tensor is [outer, channels*inner]; one
+//   column mode (inner <= 256): the tensor is [outer, channels*inner]; one
 //                thread per column (or 4 columns) walks a chunk of rows, so a
 //                warp still reads contiguous 128/512-byte lines.
 // Stage 2 (finalize) combines the partials of each channel in a fixed order (a transposed
@@ -37,7 +34,6 @@
 
 namespace qsb {
 
-constexpr int kRowModeMinInner = 64;
 constexpr int kRowCtasPerSm = 4;  // column mode / default row variant
 // row-kernel variant (tuning key 17): 0 = 4 x 256-bit loads per lane in flight, 4 CTAs / SM;
 // 2 = 8 loads, 2 CTAs / SM (default: half as many partials for the finalize / the fused tail).
@@ -53,14 +49,13 @@ static inline int row_variant_for(int64_t inner) {
   return inner >= 2048 ? 2 : 0;
 }
 static inline int row_ctas_per_sm(int variant) { return variant == 0 ? 4 : 2; }
-// tuning key 20: rows up to this many elements use the COLUMN kernel (the tensor seen as [outer, C * inner]:
-// vertical accumulation, perfectly coalesced, ~4 instructions per element) instead of the tile / row kernels
-// Measured (profiles/r02_colmode_probe_r2t.jsonl, sum|x| + max|x|, us): [256,256,14,14] 23.6 (tile kernel) -> 17.4,
+// Rows up to this many elements use the COLUMN kernel (the tensor seen as [outer, C * inner]: vertical
+// accumulation, perfectly coalesced, ~4 instructions per element).  Against the tile kernel that used to take rows
+// of 64..256 elements (profiles/r02_colmode_probe_r2t.jsonl, sum|x| + max|x|, us): [256,256,14,14] 23.6 -> 17.4,
 // [512,512,10,10] 35.8 -> 25.6, [256,512,16,16] 46.1 -> 29.7, [4096,64,14,14] 60.4 -> 39.9 (0.53 -> 0.80 of the copy
-// peak), [256,2048,8,8] 42.0 -> 27.6; rows of 784 elements and more are better off in the row kernel (23.6 vs 27.6).
-// Default: rows of up to 256 elements (what used to be the tile kernel's range); 63 restores the tile kernel.
-static int g_col_max_inner = 256;
-void set_reduce_col_max_inner(int v) { g_col_max_inner = v < 1 ? 256 : v; }
+// peak), [256,2048,8,8] 42.0 -> 27.6, so the tile kernel was removed; rows of 784 elements and more are better off in
+// the row kernel (23.6 vs 27.6).
+constexpr int64_t kColMaxInner = 256;
 // tuning key 18: the fused step reads the previous mask's kept channels with L2::evict_last
 static int g_keep_hint = 1;
 void set_reduce_keep_hint(int v) { g_keep_hint = v != 0; }
@@ -141,39 +136,6 @@ __device__ __forceinline__ void warp_store(const Acc<WHAT> &a_in, int lane,
   if constexpr (WHAT & QSB_STAT_NNZ) {
     a.nnz = warp_reduce(a.nnz, [](uint32_t x, uint32_t y) { return x + y; });
     if (lane == 0) P.nnz[item] = (double)a.nnz;
-  }
-}
-
-// the same over groups of LPR consecutive lanes (each group owns one partial; `item` and `live` are the group's)
-template <int WHAT, int LPR>
-__device__ __forceinline__ void group_store(const Acc<WHAT> &a_in, int lane, const Partials &P, int64_t item,
-                                            bool live) {
-  if constexpr (LPR == 32) {
-    if (live) warp_store<WHAT>(a_in, lane, P, item);  // live is warp-uniform here
-    return;
-  }
-  Acc<WHAT> a = a_in;
-  int nan = a.nan ? 1 : 0;
-#pragma unroll
-  for (int o = LPR / 2; o > 0; o >>= 1) {
-    if constexpr (WHAT & QSB_STAT_ABSMAX) {
-      const uint32_t t = __shfl_xor_sync(0xffffffffu, a.amax, o);
-      a.amax = t > a.amax ? t : a.amax;
-    }
-    if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ)) {
-      nan |= __shfl_xor_sync(0xffffffffu, nan, o);
-      a.mn = fminf(a.mn, __shfl_xor_sync(0xffffffffu, a.mn, o));
-    }
-    if constexpr (WHAT & QSB_STAT_MINMAX) a.mx = fmaxf(a.mx, __shfl_xor_sync(0xffffffffu, a.mx, o));
-    if constexpr (WHAT & QSB_STAT_ABSSUM) a.asum += __shfl_xor_sync(0xffffffffu, a.asum, o);
-    if constexpr (WHAT & QSB_STAT_NNZ) a.nnz += __shfl_xor_sync(0xffffffffu, a.nnz, o);
-  }
-  if (live && (lane & (LPR - 1)) == 0) {
-    if constexpr (WHAT & QSB_STAT_ABSMAX) P.amax[item] = a.amax;
-    if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ)) P.mn[item] = nan ? nan_f() : a.mn;
-    if constexpr (WHAT & QSB_STAT_MINMAX) P.mx[item] = nan ? nan_f() : a.mx;
-    if constexpr (WHAT & QSB_STAT_ABSSUM) P.asum[item] = a.asum;
-    if constexpr (WHAT & QSB_STAT_NNZ) P.nnz[item] = (double)a.nnz;
   }
 }
 
@@ -615,143 +577,6 @@ __global__ void __launch_bounds__(QSB_THREADS, MINB)
 }
 
 // ---------------------------------------------------------------------------
-// stage 1, short rows (kTileMinInner <= inner <= kTileMaxInner: 8x8 .. 16x16 feature maps).
-// A warp per row is one sub-KB request per DRAM round trip with rows that start mid-sector
-// (measured 0.21 of the copy peak on [256, 256, 14, 14]).  Here a CTA owns `tile_rows`
-// consecutive virtual warps ("slots"), i.e. tile_rows consecutive ROWS of every tile it visits
-// — one contiguous span of memory: it is read with aligned, fully coalesced 256-bit loads into
-// shared memory (the next tile's loads are already in flight in registers), then warp w reduces
-// rows w, w + 8, ... from shared memory, lane-strided, into one accumulator per slot.  The
-// partial layout (one entry per virtual warp, slot % channels == channel) is the row kernel's.
-// ---------------------------------------------------------------------------
-constexpr int kTileMinInner = 64;  // below: column mode (a warp per 7x7 row wastes lanes and issue slots: measured 2-3x slower)
-constexpr int kTileMaxInner = 256;
-constexpr int kTileFloats = 8192;  // 32 KB of shared memory; 4 vectors per thread
-constexpr int kTileRowsMax = 32;   // 4 slots per warp
-constexpr int kTileVpt = kTileFloats / 8 / QSB_THREADS;
-constexpr int kTileCtasPerSm = 3;  // 80 registers: 4 accumulators + a prefetched visit + a row in flight
-
-// LPR lanes share a row (32: a warp per row; 16: two rows per warp pass, for rows of <= 128 elements, where a
-// whole warp per 64-element row spent ~60 instructions of overhead per row); KI = loads per lane per row.
-template <int WHAT, int KI, int LPR, class Tail>
-__global__ void __launch_bounds__(QSB_THREADS, kTileCtasPerSm)
-    reduce_tile_kernel(const float *__restrict__ x, int64_t rows, int inner, int tile_rows, int spans,
-                       int span_stride, int64_t vwarps, Partials P, const __grid_constant__ Tail tail) {
-  pdl_wait();
-  pdl_trigger();
-  const StepPrefetch pre = fused_step_begin<WHAT>(tail);
-  __shared__ __align__(32) float tile[kTileFloats];
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int64_t slot0 = (int64_t)blockIdx.x * tile_rows;
-  const int nslots = (int)((vwarps - slot0 < tile_rows) ? vwarps - slot0 : tile_rows);
-  const int vps = span_stride >> 3;  // vectors per span
-  constexpr int G = 32 / LPR;                    // rows per warp pass
-  constexpr int kQ = kTileRowsMax / (8 * G);     // passes = accumulators per lane
-  const int gid = lane / LPR, gl = lane % LPR;
-  Acc<WHAT> acc[kQ];
-  VecF<8> r[kTileVpt];
-  unsigned have_next = 0;  // which r[i] hold data of the visit being fetched
-
-  // rows [base + g * vwarps, +nslots) for g < spans: `spans` contiguous pieces of memory, each
-  // copied to tile[g * span_stride ...] keeping its position inside a 32-byte sector
-  // which piece / vector of the piece this thread's i-th register vector is: the same for every visit
-  int gi[kTileVpt], vii[kTileVpt];
-#pragma unroll
-  for (int i = 0; i < kTileVpt; ++i) {
-    const int v = threadIdx.x + i * QSB_THREADS;
-    gi[i] = v / vps;
-    vii[i] = v - gi[i] * vps;
-  }
-  auto fetch = [&](int64_t base) {
-    have_next = 0;
-#pragma unroll
-    for (int i = 0; i < kTileVpt; ++i) {
-      const int g = gi[i], vi = vii[i];
-      if (g >= spans) continue;
-      const int64_t base_g = base + (int64_t)g * vwarps;
-      if (base_g >= rows) continue;
-      const int nr = (int)((rows - base_g < nslots) ? rows - base_g : nslots);
-      const float *S = x + base_g * inner;
-      const int a = (int)((reinterpret_cast<uintptr_t>(S) >> 2) & 7);
-      const float *A = S - a;  // 32-byte aligned
-      const int end = a + nr * inner;
-      if ((vi << 3) >= end) continue;
-      have_next |= 1u << i;
-      if ((vi > 0 || a == 0) && (vi << 3) + 8 <= end) {
-        r[i] = ld_vec<8, Hint::KEEP>(A + (vi << 3));
-      } else {  // first / last vector of a span: never touch memory outside it
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int e = (vi << 3) + j;
-          r[i].v[j] = (e >= a && e < end) ? A[e] : 0.f;
-        }
-      }
-    }
-  };
-
-  const int64_t visit = (int64_t)spans * vwarps;
-  fetch(slot0);
-  for (int64_t base = slot0; base < rows; base += visit) {
-    const unsigned have = have_next;
-#pragma unroll
-    for (int i = 0; i < kTileVpt; ++i) {
-      if (have & (1u << i)) {
-        float4 *d = reinterpret_cast<float4 *>(tile + ((threadIdx.x + i * QSB_THREADS) << 3));
-        d[0] = make_float4(r[i].v[0], r[i].v[1], r[i].v[2], r[i].v[3]);
-        d[1] = make_float4(r[i].v[4], r[i].v[5], r[i].v[6], r[i].v[7]);
-      }
-    }
-    __syncthreads();
-    have_next = 0;
-    if (base + visit < rows) fetch(base + visit);
-    for (int g = 0; g < spans; ++g) {
-      const int64_t base_g = base + (int64_t)g * vwarps;
-      if (base_g >= rows) break;
-      const int nr = (int)((rows - base_g < nslots) ? rows - base_g : nslots);
-      const int a = (int)((reinterpret_cast<uintptr_t>(x + base_g * inner) >> 2) & 7);
-#pragma unroll
-      for (int q = 0; q < kQ; ++q) {
-        const int rr = q * (8 * G) + w * G + gid;
-        if (rr < nr) {
-          const float *rowp = tile + g * span_stride + a + rr * inner;
-          float s = 0.f;  // <= 8 terms per lane in fp32, then fp64 (see the header note)
-          float vals[KI];
-#pragma unroll
-          for (int k = 0; k < KI; ++k)  // all the row's loads first, no loop overhead
-            if (gl + LPR * k < inner) vals[k] = rowp[gl + LPR * k];
-#pragma unroll
-          for (int k = 0; k < KI; ++k) {
-            if (gl + LPR * k < inner) {
-              const float v = vals[k];
-              if constexpr (WHAT & QSB_STAT_ABSMAX) {
-                const uint32_t b = __float_as_uint(v) & 0x7fffffffu;
-                acc[q].amax = b > acc[q].amax ? b : acc[q].amax;
-              }
-              if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ)) {
-                acc[q].mn = fminf(acc[q].mn, v);
-                acc[q].nan |= (v != v);
-              }
-              if constexpr (WHAT & QSB_STAT_MINMAX) acc[q].mx = fmaxf(acc[q].mx, v);
-              if constexpr (WHAT & QSB_STAT_ABSSUM) s = __fadd_rn(s, fabsf(v));
-              if constexpr (WHAT & QSB_STAT_NNZ) acc[q].nnz += (v != 0.0f) ? 1u : 0u;
-            }
-          }
-          if constexpr (WHAT & QSB_STAT_ABSSUM) acc[q].asum += (double)s;
-        }
-      }
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int q = 0; q < kQ; ++q) {
-    const int rr = q * (8 * G) + w * G + gid;
-    group_store<WHAT, LPR>(acc[q], lane, P, slot0 + rr, rr < nslots);
-  }
-  // the tile buffer (32 KB) is free now: the parameter step's shared memory (<= 20.5 KB) lives there
-  if constexpr (Tail::kFused) fused_tail<WHAT>(tail, P, reinterpret_cast<unsigned char *>(tile), pre);
-}
-
-// ---------------------------------------------------------------------------
 // stage 1, column mode.  partial index = chunk * ncols + col.
 // A CTA owns a band of rows (blockIdx.y) and `tpr` column-vectors of it (blockIdx.x); when
 // the tensor has fewer than 256 column-vectors ([N, 64] activations: 16 of them) the CTA's
@@ -983,7 +808,7 @@ __global__ void __launch_bounds__(QSB_THREADS)
   }
 }
 
-// stage 2 when fin_q == 1 (channel-last column mode, the tile kernel): entry j of channel c sits
+// stage 2 when fin_q == 1 (channel-last column mode): entry j of channel c sits
 // at j * channels + c, so a warp that walks j touches 32 sectors for 32 values (the finalize took
 // 12 us behind a 16 us stage 1 on [16384, 1000]).  Here a CTA owns 8 ADJACENT channels: thread t
 // reads channel (t & 7) of entries (t >> 3), (t >> 3) + 32, ... — each 8-lane group reads whole
@@ -1116,14 +941,11 @@ __global__ void tensor_min_kernel(const float *mn, int64_t channels, float *out)
 // Physical warps of the row kernel: SMs x resident CTAs x 8.  The CTA count per
 // SM is fixed (not queried per instantiation) so that the plan — and with it the
 // summation order — only depends on the device, never on which statistics run.
-static int g_reduce_seg_min = 1024;
-int64_t reduce_seg_min() { return g_reduce_seg_min; }
+constexpr int64_t kSegMin = 1024;
 // column mode on wide tensors (more column vectors than this): threads of a CTA along a row; the other
 // 256 / tpr threads are row lanes whose results are combined in shared memory before the partial
 // is written, so the partial array (and the finalize's read) shrinks by that factor
-static int g_col_tpr_wide = 64;  // measured: [16384,1000] 14.7 + 6.3 -> 14.2 + 3.7 us, [512,512,7,7] 15.4 + 7.5 -> 11.4 + 6.4 us vs 256
-void set_reduce_col_tpr_wide(int v) { g_col_tpr_wide = (v == 32 || v == 64 || v == 128) ? v : 256; }
-void set_reduce_seg_min(int v) { g_reduce_seg_min = v >= 256 ? v : 256; }
+constexpr int64_t kColTprWide = 64;  // measured: [16384,1000] 14.7 + 6.3 -> 14.2 + 3.7 us, [512,512,7,7] 15.4 + 7.5 -> 11.4 + 6.4 us vs 256
 
 ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner,
                             const void *x, int x_bytes) {
@@ -1131,39 +953,13 @@ ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner,
   p.row_variant = row_variant_for(inner);
   const int64_t warps_phys =
       (int64_t)device_props().sm_count * row_ctas_per_sm(p.row_variant) * (QSB_THREADS / 32);
-  if (inner > g_col_max_inner && inner >= kTileMinInner && inner <= kTileMaxInner) {
-    // short rows: the tile kernel.  One slot (virtual warp) per row of a tile, 3 CTAs of 32 slots
-    // per SM; slots = m * channels so that a slot only ever sees one channel.
-    p.row_mode = true;
-    p.rows = outer * channels;
-    p.seg = (inner + 7) / 8 * 8;
-    p.segs_per_row = 1;
-    p.tile_rows = (int)((kTileFloats - 7) / inner < kTileRowsMax ? (kTileFloats - 7) / inner : kTileRowsMax);
-    // one CTA visit covers `tile_spans` pieces of tile_rows rows (vwarps rows apart), each kept at its
-    // own offset inside a 32-byte sector: ~32 KB in flight per CTA whatever the row length
-    p.tile_span_stride = (int)((p.tile_rows * inner + 7 + 7) / 8 * 8);
-    p.tile_spans = kTileFloats / p.tile_span_stride;
-    const int64_t target = (int64_t)device_props().sm_count * kTileCtasPerSm * kTileRowsMax;
-    if (channels == 1) {
-      p.vwarps = p.rows < target ? p.rows : target;
-      p.fin_count = p.vwarps;
-    } else {
-      int64_t m = target / channels;
-      if (m > outer) m = outer;
-      if (m < 1) m = 1;
-      p.vwarps = m * channels;
-      p.fin_count = m;
-    }
-    p.fin_q = 1;
-    p.n_partials = p.vwarps;
-  } else if (inner > g_col_max_inner && inner >= kRowModeMinInner) {
+  if (inner > kColMaxInner) {
     p.row_mode = true;
     p.rows = outer * channels;
     // balanced segments: aim for >= 6 work items per physical warp, but keep every
-    // segment >= seg_min elements (two rounds of 4 x 256-bit loads per lane) unless the
+    // segment >= kSegMin elements (two rounds of 4 x 256-bit loads per lane) unless the
     // machine could not be filled otherwise
-    const int64_t seg_min = reduce_seg_min();
-    int64_t spr_max = inner / seg_min > 0 ? inner / seg_min : 1;
+    int64_t spr_max = inner / kSegMin > 0 ? inner / kSegMin : 1;
     int64_t spr = (6 * warps_phys + p.rows - 1) / p.rows;
     if (spr > spr_max) spr = spr_max;
     if (spr < 1) spr = 1;
@@ -1224,12 +1020,12 @@ ReducePlan make_plan(int64_t outer, int64_t channels, int64_t inner,
       if (c > 65535) c = 65535;
       return c;
     };
-    // wide tensors: from g_col_tpr_wide threads along the row upwards, the first width whose grid fills
+    // wide tensors: from kColTprWide threads along the row upwards, the first width whose grid fills
     // one wave best ([1024, 2048, 7, 7] at 64: 392 x 2 CTAs = 1.3 waves, 83 us instead of 71)
     int64_t tpr = tpr_max;
-    if (tpr_max > g_col_tpr_wide) {
+    if (tpr_max > kColTprWide) {
       double best = -1.0;
-      for (int64_t t = g_col_tpr_wide; t <= tpr_max; t <<= 1) {
+      for (int64_t t = kColTprWide; t <= tpr_max; t <<= 1) {
         const int64_t total = (threads + t - 1) / t * chunks_for(t);
         const int64_t waves = (total + want - 1) / want;
         const double eff = (double)total / (double)(waves * want);
@@ -1276,23 +1072,9 @@ template <int WHAT, class Tail = NoTail, class T = float>
 static int run_reduce(const T *x, const ReducePlan &pl, int64_t channels,
                       int64_t inner, const Partials &P, const FinalOut &out,
                       cudaStream_t stream, bool finalize = true, const Tail &tail = Tail{}) {
-  // dynamic shared memory of the fused parameter step (the tile kernel re-uses its tile buffer)
+  // dynamic shared memory of the fused parameter step
   const size_t dyn = std::is_same<Tail, StepTail>::value ? step_smem_bytes((int)channels, kLineStep<WHAT>) : 0;
-  if (pl.row_mode && pl.tile_rows > 0) {
-    // the tile kernel (only reachable through tuning key 20) stages fp32 sectors: fp32 input only
-    if constexpr (is_half16<T>) {
-      return QSB_E_UNSUPPORTED;
-    } else {
-      const int64_t grid = (pl.vwarps + pl.tile_rows - 1) / pl.tile_rows;
-      auto go = [&](auto kernel) {
-        return launch_k(kernel, dim3((unsigned)grid), dim3(QSB_THREADS), 0, stream, x, pl.rows, (int)inner,
-                        pl.tile_rows, pl.tile_spans, pl.tile_span_stride, pl.vwarps, P, tail);
-      };
-      if (inner <= 64) QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 4, 16, Tail>));
-      else if (inner <= 128) QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 8, 16, Tail>));
-      else QSB_CUDA_TRY(go(reduce_tile_kernel<WHAT, 8, 32, Tail>));
-    }
-  } else if (pl.row_mode) {
+  if (pl.row_mode) {
     constexpr int kWarps = QSB_THREADS / 32;
     int64_t grid = (int64_t)device_props().sm_count * row_ctas_per_sm(pl.row_variant);
     const int64_t need = (pl.vwarps + kWarps - 1) / kWarps;
@@ -1533,7 +1315,7 @@ static int reduce_prune_quant_step_impl(
   tail.a.timing = reinterpret_cast<unsigned long long *>(timing_out_dev);
   // the previous step's mask as an L2 residency hint: channels it keeps are about to be re-read by
   // the forward pass (only meaningful for a per-channel mask in row mode)
-  tail.keep_hint = (g_keep_hint && pl.row_mode && pl.tile_rows == 0 && channels > 1) ? mask : nullptr;
+  tail.keep_hint = (g_keep_hint && pl.row_mode && channels > 1) ? mask : nullptr;
   FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
   return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, StepTail, T>(x, pl, channels, inner, P, out, stream,
                                                                     /*finalize=*/false, tail);

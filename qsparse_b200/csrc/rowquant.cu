@@ -14,19 +14,17 @@
 // row ONCE into registers, reduces it, updates the row's parameter, and quantizes the row
 // from the registers: 8 B/elem, one launch, no dependency between CTAs.
 //
-// Two kernels:
-//   row_quant_kernel      the row lives in registers: a CTA per row (1 Ki .. 16 Ki elements, one
-//       barrier: every thread merges the warps' partials and derives the new parameter
-//       itself) or a warp per row (shorter rows).  Measured on [4096, 4096] (134 MB of
-//       traffic): 25.6 us scaler / 28.7 us line — the same as the plain fake-quant kernel
-//       alone on that tensor (28.6 us), against 50.2 us for reduce -> EMA -> quantize.
-//   row_quant_tma_kernel  alternative for the CTA-per-row range (tuning key 9): persistent CTAs,
-//       ONE thread streams the CTA's rows into a ring of shared-memory stages with
-//       cp.async.bulk (TMA engine, completion on an mbarrier) 2-4 rows ahead, so the bytes
-//       in flight are bounded by shared memory, not registers.  Measured 30.7 us for every
-//       (CTAs per SM, stages) in {2..8} x {2..4}: the row's dependent chain (wait -> LDS ->
-//       reduce -> barrier -> quantize -> store) bounds a persistent CTA, and one CTA per row
-//       with 5 CTAs per SM overlaps those chains better.  Kept selectable, not the default.
+// row_quant_kernel: the row lives in registers: a CTA per row (1 Ki .. 16 Ki elements, one
+// barrier: every thread merges the warps' partials and derives the new parameter itself) or a
+// warp per row (shorter rows).  Measured on [4096, 4096] (134 MB of traffic): 25.6 us scaler /
+// 28.7 us line — the same as the plain fake-quant kernel alone on that tensor (28.6 us), against
+// 50.2 us for reduce -> EMA -> quantize.
+//
+// A TMA-pipelined persistent variant (ONE thread streamed a CTA's rows into a ring of
+// shared-memory stages with cp.async.bulk, 2-4 rows ahead) was measured at 30.7 us for every
+// (CTAs per SM, stages) in {2..8} x {2..4} and removed: the row's dependent chain (wait -> LDS ->
+// reduce -> barrier -> quantize -> store) bounds a persistent CTA, and one CTA per row with
+// 5 CTAs per SM overlaps those chains better.
 //
 // Arithmetic is the same device code as the unfused kernels (fq_ops.cuh, param_math.cuh),
 // so the results are bit-identical to reduce_stats -> *_ema -> fq_*_fwd.
@@ -244,156 +242,6 @@ __global__ void __launch_bounds__(QSB_THREADS, (U <= 2 && !MASKED) ? QSB_K8_MIN_
     }
 }
 
-// ---------------------------------------------------------------------------
-// TMA-pipelined persistent variant (a CTA per row, rows staged in shared memory)
-// ---------------------------------------------------------------------------
-constexpr int kTmaMaxStages = 4;
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-  }
-}
-// one elected thread: expect `bytes` on the barrier, then bulk-copy global -> shared
-__device__ __forceinline__ void tma_load_row(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-               : "memory");
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-          smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
-
-template <int KIND, bool FZP, int U>
-__global__ void __launch_bounds__(QSB_THREADS)
-    row_quant_tma_kernel(const float *__restrict__ x, float *__restrict__ y, float *__restrict__ param,
-                         float *__restrict__ decimal_out, int64_t rows, int inner, RowConsts k,
-                         int stages) {
-  constexpr int V = 8;
-  constexpr int kWsz = (KIND == kRowLine) ? 2 : 1;
-  extern __shared__ __align__(128) unsigned char s_rows[];  // [stages][inner] floats
-  __shared__ uint64_t s_full[kTmaMaxStages];
-  __shared__ RowStat s_part[2][QSB_THREADS / 32];
-  __shared__ float s_dec[2];
-  const int tid = threadIdx.x, lane = tid & 31;
-  const int nvec = inner / V;
-  const uint32_t row_bytes = (uint32_t)inner * 4u;
-  const int64_t first = blockIdx.x, step = gridDim.x;
-  const int64_t n_mine = first < rows ? (rows - first + step - 1) / step : 0;
-
-  if (tid == 0) {
-    for (int st = 0; st < stages; ++st) mbar_init(&s_full[st], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  if (tid == 0) {
-    for (int st = 0; st < stages && st < n_mine; ++st)
-      tma_load_row(s_rows + (size_t)st * row_bytes, x + (first + st * step) * inner, row_bytes, &s_full[st]);
-  }
-
-  using RO = RowOp<KIND, FZP>;
-  const typename RO::Op op = RO::make(k);
-  int stage = 0;
-  uint32_t parity = 0;
-  for (int64_t i = 0; i < n_mine; ++i) {
-    const int64_t row = first + i * step;
-    const float2 w_old = load_param<KIND>(param + row * kWsz);  // in flight while we wait for the row
-    mbar_wait(&s_full[stage], parity);
-    const float4 *srow = reinterpret_cast<const float4 *>(s_rows + (size_t)stage * row_bytes);
-    VecF<V> a[U];
-    RowStat s{0u, INFINITY, -INFINITY, 0};
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-      if (u * QSB_THREADS + tid < nvec) {
-        const float4 q0 = srow[(u * QSB_THREADS + tid) * 2], q1 = srow[(u * QSB_THREADS + tid) * 2 + 1];
-        a[u].v[0] = q0.x, a[u].v[1] = q0.y, a[u].v[2] = q0.z, a[u].v[3] = q0.w;
-        a[u].v[4] = q1.x, a[u].v[5] = q1.y, a[u].v[6] = q1.z, a[u].v[7] = q1.w;
-#pragma unroll
-        for (int j = 0; j < V; ++j) stat_add<KIND>(s, a[u].v[j]);
-      }
-    s = stat_warp<KIND>(s);
-    RowStat *part = s_part[i & 1];  // alternate: a warp may run one iteration ahead of another
-    if (lane == 0) part[tid >> 5] = s;
-    __syncthreads();  // every thread has its part of the row in registers: the stage is free
-    if (tid == 0 && i + stages < n_mine)
-      tma_load_row(s_rows + (size_t)stage * row_bytes, x + (row + stages * step) * inner, row_bytes,
-                   &s_full[stage]);
-    s = part[0];
-#pragma unroll
-    for (int w = 1; w < QSB_THREADS / 32; ++w) stat_merge<KIND>(s, part[w]);
-    float2 pv = ema_param<KIND>(s, w_old, k);
-    if (tid == 0) store_param<KIND>(param + row * kWsz, pv);
-    if constexpr (KIND == kRowDecimal) {
-      if (tid == 0) s_dec[i & 1] = scale_to_decimal(pv.x);  // fp64 log2: once per row
-      __syncthreads();
-      pv.y = s_dec[i & 1];
-      if (tid == 0 && decimal_out) decimal_out[row] = pv.y;
-    }
-    const typename RO::Op::P p = RO::derive(op, pv);
-    float *yr = y + row * inner;
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-      if (u * QSB_THREADS + tid < nvec) {
-        VecF<V> o0, o1;
-        VecB<V> mb, ob;
-        apply_vec<typename RO::Op, V>(op, a[u], a[u], mb, false, p, o0, o1, ob);
-        st_vec<V, Hint::KEEP>(yr + (int64_t)(u * QSB_THREADS + tid) * V, o0);
-      }
-    if (++stage == stages) {
-      stage = 0;
-      parity ^= 1u;
-    }
-  }
-}
-
-static int g_row_tma = 0;       // tuning key 9: 1 = TMA-pipelined kernel for long rows, 0 = register kernel (default: measured faster)
-static int g_row_ctas_per_sm = 0;  // tuning key 10: persistent CTAs per SM (0 = as many as fit, at most 3)
-static int g_row_stages = 0;       // tuning key 11: ring stages (0 = auto)
-void set_row_tma(int v) { g_row_tma = v != 0; }
-void set_row_ctas_per_sm(int v) { g_row_ctas_per_sm = v; }
-void set_row_stages(int v) { g_row_stages = v; }
-
-template <int KIND, bool FZP, int U>
-static int launch_rows_tma(const float *x, float *y, float *param, float *decimal_out, int64_t rows,
-                           int64_t inner, const RowConsts &k, cudaStream_t stream) {
-  const int64_t row_bytes = inner * 4;
-  int stages = (int)(96 * 1024 / row_bytes);  // ~64-96 KB of rows in flight per CTA
-  if (g_row_stages > 0) stages = g_row_stages;
-  if (stages > kTmaMaxStages) stages = kTmaMaxStages;
-  if (stages < 2) stages = 2;
-  const size_t smem = (size_t)stages * row_bytes;
-  static size_t attr_bytes = 0;
-  if (smem > attr_bytes) {
-    QSB_CUDA_TRY(cudaFuncSetAttribute(row_quant_tma_kernel<KIND, FZP, U>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_bytes = smem;
-  }
-  int occ = 0;
-  QSB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, row_quant_tma_kernel<KIND, FZP, U>,
-                                                             QSB_THREADS, smem));
-  if (occ < 1) return QSB_E_UNSUPPORTED;
-  int per_sm = g_row_ctas_per_sm > 0 ? g_row_ctas_per_sm : 3;  // occupancy caps it below
-  if (per_sm > occ) per_sm = occ;
-  int64_t grid = (int64_t)device_props().sm_count * per_sm;
-  if (grid > rows) grid = rows;
-  row_quant_tma_kernel<KIND, FZP, U><<<(unsigned)grid, QSB_THREADS, smem, stream>>>(
-      x, y, param, decimal_out, rows, (int)inner, k, stages);
-  QSB_LAUNCH_CHECK();
-  return 0;
-}
-
 template <int KIND, bool FZP, int U, int G>
 static int launch_rows(const float *x, float *y, float *param, float *decimal_out, const uint8_t *mask,
                        int64_t rows, int64_t inner, const RowConsts &k, cudaStream_t stream) {
@@ -417,12 +265,6 @@ static int dispatch_rows(const float *x, float *y, float *param, float *decimal_
   if (inner <= 256) return launch_rows<KIND, FZP, 1, 32>(x, y, param, decimal_out, mask, rows, inner, k, stream);
   if (inner <= 512) return launch_rows<KIND, FZP, 2, 32>(x, y, param, decimal_out, mask, rows, inner, k, stream);
   if (inner <= 1024) return launch_rows<KIND, FZP, 4, 32>(x, y, param, decimal_out, mask, rows, inner, k, stream);
-  if (g_row_tma && !mask) {
-    if (inner <= 2048) return launch_rows_tma<KIND, FZP, 1>(x, y, param, decimal_out, rows, inner, k, stream);
-    if (inner <= 4096) return launch_rows_tma<KIND, FZP, 2>(x, y, param, decimal_out, rows, inner, k, stream);
-    if (inner <= 8192) return launch_rows_tma<KIND, FZP, 4>(x, y, param, decimal_out, rows, inner, k, stream);
-    if (inner <= 16384) return launch_rows_tma<KIND, FZP, 8>(x, y, param, decimal_out, rows, inner, k, stream);
-  }
   if (inner <= 2048) return launch_rows<KIND, FZP, 1, QSB_THREADS>(x, y, param, decimal_out, mask, rows, inner, k, stream);
   if (inner <= 4096) return launch_rows<KIND, FZP, 2, QSB_THREADS>(x, y, param, decimal_out, mask, rows, inner, k, stream);
   if (inner <= 8192) return launch_rows<KIND, FZP, 4, QSB_THREADS>(x, y, param, decimal_out, mask, rows, inner, k, stream);

@@ -51,7 +51,12 @@ static_assert(kBins0 == QSB_THREADS, "pass-0 merge maps one thread to one bin");
 
 // fast route
 constexpr int kSampleThreads = 1024;
-constexpr int kSampleCtas = 8;  // one thread-block cluster; PER samples per thread
+constexpr int kSampleCtas = 8;  // one thread-block cluster
+// samples per sampler thread: four neighbours per location (one 128-bit load), 32 Ki samples for the lines
+// 8 Ki single samples would touch — what matters for the layers of a weight set, where the sample is a
+// visible fraction of the tensor
+constexpr int kSamplePer = 4;
+constexpr int kPartitionU = 4;  // 256-bit loads in flight per thread of the select's partition pass
 constexpr int kFastBits = 11, kFastBins = 1 << kFastBits;
 constexpr int kCandShift = 3;      // candidate slots = n >> 3 (12.5 %)
 constexpr int kSegs = 32;          // independent candidate segments (one packed counter each)
@@ -640,6 +645,7 @@ __device__ __forceinline__ void select_sample_body(const float *__restrict__ v, 
                                                    const float *__restrict__ w, EmaC ec,
                                                    const uint32_t *hint) {
   static_assert(kFastBins == 2 * kSampleThreads, "two bins per thread");
+  static_assert(PER == 4, "four neighbours per sampler thread: one 128-bit load");
   constexpr int kSampleSize = kSampleThreads * kSampleCtas * PER;
   constexpr int kTieMinCount = kSampleSize / 50;  // >= 2 % of the sample in lo's bucket: ties at lo
   cg::cluster_group cluster = cg::this_cluster();
@@ -651,7 +657,6 @@ __device__ __forceinline__ void select_sample_body(const float *__restrict__ v, 
   const int tid = threadIdx.x;
   const unsigned rank = cluster.block_rank();
   const int i = (int)rank * kSampleThreads + tid;
-  const int64_t stride = n / kSampleSize;
 #ifdef QSB_SELECT_TIMING
   const long long t_start = clock64();
 #endif
@@ -685,27 +690,17 @@ __device__ __forceinline__ void select_sample_body(const float *__restrict__ v, 
     return;
   }
   float f[PER];
-  if constexpr (PER == 4) {
-    // four neighbours per location (one 128-bit load): 32 Ki samples for the lines 8 Ki would touch —
-    // what matters for the layers of a weight set, where the sample is a visible fraction of the tensor
-    const int64_t stride4 = n / (kSampleThreads * kSampleCtas);
-    const int64_t at = ((int64_t)i * stride4 + (stride4 >> 1)) & ~(int64_t)3;
-    const float4 q4 = *reinterpret_cast<const float4 *>(v + at);
-    f[0] = q4.x, f[1] = q4.y, f[2] = q4.z, f[3] = q4.w;
-    if constexpr (STEP) {  // fused prune step: sample the magnitudes the EMA is ABOUT to produce
-      const float4 w4 = *reinterpret_cast<const float4 *>(w + at);
-      f[0] = ema_full_step(f[0], w4.x, ec.t_f, ec.tp1, ec.rcp);
-      f[1] = ema_full_step(f[1], w4.y, ec.t_f, ec.tp1, ec.rcp);
-      f[2] = ema_full_step(f[2], w4.z, ec.t_f, ec.tp1, ec.rcp);
-      f[3] = ema_full_step(f[3], w4.w, ec.t_f, ec.tp1, ec.rcp);
-    }
-  } else {
-#pragma unroll
-    for (int q = 0; q < PER; ++q) {
-      const int64_t at = (int64_t)(q * kSampleThreads * kSampleCtas + i) * stride + (stride >> 1);
-      f[q] = v[at];
-      if constexpr (STEP) f[q] = ema_full_step(f[q], w[at], ec.t_f, ec.tp1, ec.rcp);
-    }
+  // four neighbours per location: one 128-bit load
+  const int64_t stride4 = n / (kSampleThreads * kSampleCtas);
+  const int64_t at = ((int64_t)i * stride4 + (stride4 >> 1)) & ~(int64_t)3;
+  const float4 q4 = *reinterpret_cast<const float4 *>(v + at);
+  f[0] = q4.x, f[1] = q4.y, f[2] = q4.z, f[3] = q4.w;
+  if constexpr (STEP) {  // fused prune step: sample the magnitudes the EMA is ABOUT to produce
+    const float4 w4 = *reinterpret_cast<const float4 *>(w + at);
+    f[0] = ema_full_step(f[0], w4.x, ec.t_f, ec.tp1, ec.rcp);
+    f[1] = ema_full_step(f[1], w4.y, ec.t_f, ec.tp1, ec.rcp);
+    f[2] = ema_full_step(f[2], w4.z, ec.t_f, ec.tp1, ec.rcp);
+    f[3] = ema_full_step(f[3], w4.w, ec.t_f, ec.tp1, ec.rcp);
   }
   for (int j = i; j < zero_vecs; j += kSampleThreads * kSampleCtas) zero_base[j] = make_uint4(0, 0, 0, 0);
   reinterpret_cast<uint2 *>(h0)[tid] = make_uint2(0, 0);
@@ -1155,7 +1150,7 @@ __global__ void __cluster_dims__(kSampleCtas, 1, 1) __launch_bounds__(kSampleThr
 }
 
 template <int U, bool ABS>
-__global__ void __launch_bounds__(QSB_THREADS, U == 2 ? 8 : 5)
+__global__ void __launch_bounds__(QSB_THREADS, 5)
     select_partition_kernel(const __grid_constant__ SegTable tab) {
   const SegDesc &d = tab.d[blockIdx.y];
   if (!d.fast || (int64_t)blockIdx.x * (QSB_THREADS * 8 * U) >= d.n) return;
@@ -1208,16 +1203,10 @@ __global__ void __launch_bounds__(QSB_THREADS)
   select_pass_body<PASS, V, ABS>(d.v, d.n, d.k, ws_of(d.hdr), fb, st_of(d.hdr), d.thr_out, d.fast ? d.hint : nullptr);
 }
 
-static int g_select_fast = 1;  // tuning key 4
-static int g_select_pdl = 1;   // tuning key 8: programmatic dependent launch inside a select
-static int g_partition_u = 4;  // tuning key 6: 256-bit loads in flight per thread (2 or 4)
-static int g_sample_per = 4;   // tuning key 7: samples per sampler thread (1, 2, 4 -> 8K, 16K, 32K samples)
+static int g_select_fast = 1;  // tuning key 4 (test hook): 0 forces the three generic passes
 constexpr int64_t kFastMinNBatched = 1 << 17;  // segments of a batch share the launches' fixed costs
 
 void set_select_fast(int v) { g_select_fast = v; }
-void set_select_pdl(int v) { g_select_pdl = v != 0; }
-void set_select_partition_u(int v) { g_partition_u = (v == 2) ? 2 : 4; }
-void set_select_sample_per(int v) { g_sample_per = (v == 1 || v == 2) ? v : 4; }
 
 // slots per candidate segment: n/8 in total, a multiple of 8 per segment, < 2^32
 static int64_t seg_slots(int64_t n) {
@@ -1233,7 +1222,7 @@ static int64_t seg_workspace_bytes(int64_t n) {
 template <class K, class... A>
 static int launch_seg(K kernel, dim3 grid, dim3 block, cudaStream_t stream, bool pdl, const SegTable &tab,
                       A... extra) {
-  if (pdl && g_select_pdl) {  // the previous kernel of this select is the dependency
+  if (pdl) {  // the previous kernel of this select is the dependency
     QSB_CUDA_TRY(launch_pdl(kernel, grid, block, 0, stream, tab, extra...));
     return 0;
   }
@@ -1264,19 +1253,8 @@ static int launch_pass(const SegTable &tab, int L, int64_t max_n, bool any_fast,
 }
 
 // descs[0..L): one launch sequence.  v8: every segment is 32-byte aligned (256-bit loads).
-// samples per sampler thread: the tuning value for one select; for a batch (small segments: 16 Ki
-// scattered samples of a 2.4 M-element layer would touch a fifth of its lines) 8 Ki locations x 4 neighbours
-static int g_step_sample_per = 4;   // tuning key 13: samples per sampler thread in the fused prune step
-static int g_step_sigma10 = 35;     // tuning key 14: pivot distance in 0.1 sigma in the fused prune step
-void set_step_sample_per(int v) { g_step_sample_per = (v == 1 || v == 2) ? v : 4; }
-void set_step_sigma10(int v) { g_step_sigma10 = v < 20 ? 20 : (v > 60 ? 60 : v); }
-static int sample_per(bool batched, bool step = false) {
-  return step ? g_step_sample_per : (batched ? 4 : g_sample_per);
-}
-
 template <bool ABS, bool STEP = false>
-static int run_group(SegDesc *descs, int L, bool v8, bool first_after_kernel, bool batched,
-                     cudaStream_t stream, EmaC ec = EmaC{}) {
+static int run_group(SegDesc *descs, int L, bool v8, bool first_after_kernel, cudaStream_t stream, EmaC ec = EmaC{}) {
   SegTable tab;
   int64_t max_n = 0, max_fast_n = 0;
   for (int i = 0; i < L; ++i) {
@@ -1289,16 +1267,10 @@ static int run_group(SegDesc *descs, int L, bool v8, bool first_after_kernel, bo
   if (first_after_kernel) {
     // pivots for the fast segments; zeroes every segment's header (no memset node)
     const dim3 sg(kSampleCtas, (unsigned)L);
-    const int per = sample_per(batched, STEP);
     // (PDL: the sampler starts with griddepcontrol.wait, so it is ordered after whatever precedes it
     // in the stream, but its launch latency overlaps that kernel's tail)
     const int abs_i = ABS ? 1 : 0;
-    if (per == 1)
-      rc = launch_seg(select_sample_kernel<1, STEP>, sg, dim3(kSampleThreads), stream, true, tab, abs_i, ec);
-    else if (per == 4)
-      rc = launch_seg(select_sample_kernel<4, STEP>, sg, dim3(kSampleThreads), stream, true, tab, abs_i, ec);
-    else
-      rc = launch_seg(select_sample_kernel<2, STEP>, sg, dim3(kSampleThreads), stream, true, tab, abs_i, ec);
+    rc = launch_seg(select_sample_kernel<kSamplePer, STEP>, sg, dim3(kSampleThreads), stream, true, tab, abs_i, ec);
     if (rc) return rc;
   }
   if constexpr (STEP) {
@@ -1307,12 +1279,10 @@ static int run_group(SegDesc *descs, int L, bool v8, bool first_after_kernel, bo
     const dim3 pg((unsigned)((max_n + tile - 1) / tile), (unsigned)L);
     if ((rc = launch_seg(step_partition_kernel, pg, dim3(QSB_THREADS), stream, true, tab, ec))) return rc;
   } else if (any_fast) {
-    const int u = g_partition_u;
-    const int64_t tile = (int64_t)QSB_THREADS * 8 * u;
+    const int64_t tile = (int64_t)QSB_THREADS * 8 * kPartitionU;
     const dim3 pg((unsigned)((max_fast_n + tile - 1) / tile), (unsigned)L);
-    rc = u == 4 ? launch_seg(select_partition_kernel<4, ABS>, pg, dim3(QSB_THREADS), stream, true, tab)
-                : launch_seg(select_partition_kernel<2, ABS>, pg, dim3(QSB_THREADS), stream, true, tab);
-    if (rc) return rc;
+    if ((rc = launch_seg(select_partition_kernel<kPartitionU, ABS>, pg, dim3(QSB_THREADS), stream, true, tab)))
+      return rc;
   }
   if (v8) {
     if ((rc = launch_pass<0, 8, ABS>(tab, L, max_n, any_fast, stream, first_after_kernel))) return rc;
@@ -1360,10 +1330,10 @@ static int64_t make_desc(SegDesc &d, const float *v, int64_t n, int64_t k, float
   d.hint = nullptr;
   d.fast = g_select_fast && aligned_to(v, 32) && n >= (batched ? kFastMinNBatched : kFastMinN);
   // sample ranks bracketing k: +-4.5 sigma of the binomial rank error, +3
-  const double m = (double)(kSampleThreads * kSampleCtas * sample_per(batched, step)), p = (double)k / (double)n;
+  const double m = (double)(kSampleThreads * kSampleCtas * kSamplePer), p = (double)k / (double)n;
   // a miss of the pivots costs one full redo of the step's masks (~the price of the step), so the fused
   // step brackets tighter than a select whose miss costs three full passes
-  const double sigmas = step ? g_step_sigma10 / 10.0 : 4.5;
+  const double sigmas = step ? 3.5 : 4.5;
   const double delta = sigmas * sqrt(m * p * (1.0 - p)) + 3.0;
   d.r_lo = (int)floor(p * m - delta);
   d.r_hi = (int)ceil(p * m + delta);
@@ -1400,8 +1370,8 @@ static int kth_value_batched_impl(const float *const *v, const int64_t *n, const
   int L = 0;
   auto flush = [&](bool v8) -> int {
     if (L == 0) return 0;
-    const int rc = take_abs ? run_group<true>(group, L, v8, true, batched, stream)
-                            : run_group<false>(group, L, v8, true, batched, stream);
+    const int rc = take_abs ? run_group<true>(group, L, v8, true, stream)
+                            : run_group<false>(group, L, v8, true, stream);
     L = 0;
     return rc;
   };
@@ -1481,7 +1451,7 @@ static int prune_step_batched_impl(float *const *magnitude, const float *const *
     hdr += step_seg_workspace_bytes(n[i]);
     group[L++] = d;
     if (L == kMaxSegs || i == count - 1) {
-      if ((rc = run_group<false, true>(group, L, true, true, true, stream, ec))) return rc;
+      if ((rc = run_group<false, true>(group, L, true, true, stream, ec))) return rc;
       L = 0;
     }
   }

@@ -56,6 +56,16 @@ def test_argument_errors_without_gpu():
     assert params(c, k=c) == -1 and params(c, k=-1) == -1                               # k outside [0, C) on a refresh
 
 
+def test_set_tuning_keys_without_gpu():
+    """qsb_set_tuning knows keys 2, 4, 12, 17, 18 and 21 only (21 is not called here: it changes a device limit)."""
+    from qsparse_b200 import _native
+    lib = _native.load_library()
+    for key in (0, 1, 3, 5, 6, 7, 8, 9, 10, 11, 13, 14, 15, 16, 19, 20, 22, -1):
+        assert lib.qsb_set_tuning(key, 0) == -1, key                                    # QSB_E_BADARG
+    for key, default in ((2, 1), (4, 1), (12, 1), (17, -1), (18, 1)):
+        assert lib.qsb_set_tuning(key, default) == 0, key
+
+
 def test_product_fails_loudly_on_cpu_tensors():
     import torch
     import qsparse_b200 as qs

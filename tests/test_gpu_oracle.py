@@ -543,8 +543,8 @@ def test_fused_step_kernel_equals_separate_kernels(shape, C):
                                      ((2, 1024, 300), 1024), ((5, 3, 1031), 3), ((2, 1, 9), 1), ((1, 1, 288), 1)])
 def test_one_launch_step_equals_two_launch_step(shape, C):
     """qsb_reduce_prune_quant_step (the reduction's last-arriving CTA runs the parameter step) must be
-    bit-identical to qsb_reduce_partials + qsb_prune_quant_step_params in every stage-1 mode (rows, tile,
-    columns, one channel), with the row-kernel variants and with / without the L2 keep hint; the arrival
+    bit-identical to qsb_reduce_partials + qsb_prune_quant_step_params in every stage-1 mode (rows, columns,
+    one channel), with the row-kernel variants and with / without the L2 keep hint; the arrival
     counter must be left at zero after every launch."""
     from qsparse_b200 import ops
     from qsparse_b200._native import channel_layout
@@ -699,13 +699,10 @@ ROW_SHAPES = [(33, 8), (64, 288), (7, 1000), (130, 1024), (5, 2048), (48, 4096),
               (9, 4, 6, 12)]
 
 
-@pytest.fixture(params=[0, 1], ids=["registers", "tma"])
+@pytest.fixture(params=[0], ids=["registers"])
 def row_variant(request):
-    """both kernels for rows of 1 Ki .. 16 Ki elements: register-resident (default) and TMA-pipelined"""
-    from qsparse_b200 import ops
-    ops.set_tuning(9, request.param)
+    """the register-resident kernel for rows of 1 Ki .. 16 Ki elements"""
     yield request.param
-    ops.set_tuning(9, 0)
 
 
 @pytest.mark.parametrize("shape", ROW_SHAPES)
