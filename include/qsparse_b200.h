@@ -169,6 +169,32 @@ int qsb_quant_export_int4(const float *x, uint8_t *q_out, int kind,
                           int64_t outer, int64_t channels, int64_t inner,
                           void *stream);
 
+/* Block-scaled FP8 / FP4 fake quantization (EXTENSION; DESIGN §2 "Block-scaled formats").
+ * x (element type x_dtype, QSB_DTYPE_*) is [rows, L] in memory order; each row splits into
+ * blocks of B consecutive elements (the last one may be shorter), a = the block's max |x|:
+ *   fmt 0 MXFP8: B 32, E4M3 elements, X = 2^clamp(e(a) - 8, -127, 127), y = cvt_e4m3(x / X) * X
+ *   fmt 1 MXFP4: B 32, E2M1 elements, X = 2^clamp(e(a) - 2, -127, 127), y = cvt_e2m1(x / X) * X
+ *   fmt 2 NVFP4: B 16, E2M1 elements, s_t = w / 2688, s_b = cvt_e4m3(a / 6 / s_t),
+ *                d = s_b * s_t, y = cvt_e2m1(x / d) * d  (+0 for the block when d == 0)
+ * e(a) = floor(log2 a) from the bits of a; cvt_* round to nearest even and saturate.  A block
+ * holding a NaN or +-inf gives NaN; for NVFP4 a NaN s_t gives NaN and a zero s_t +0 everywhere.
+ * w = *tensor_amax_dev (NVFP4 only; ignored otherwise).  y is fp32 [rows, L].  8 B/elem (fp32
+ * x), 6 B/elem (16-bit x).  NULL pointers, a bad fmt / dtype or negative sizes: QSB_E_BADARG. */
+#define QSB_BLOCK_MXFP8 0
+#define QSB_BLOCK_MXFP4 1
+#define QSB_BLOCK_NVFP4 2
+int qsb_fq_block_fwd_dt(const void *x, int x_dtype, float *y, int64_t rows, int64_t L, int fmt,
+                        const float *tensor_amax_dev, void *stream);
+
+/* The packed form of the same quantizer, in one pass:
+ *   codes  E4M3 (MXFP8): uint8 [rows, L];  E2M1: uint8 [rows, (L + 1) / 2], element 2i in the
+ *          low nibble, a zero pad nibble when L is odd (codes are 0 in a NaN or zero-scale block)
+ *   scales uint8 [rows, ceil(L / B)]: E8M0 (0xFF for a NaN block) or, for NVFP4, E4M3 s_b
+ *          (0x7F for a NaN block or a NaN s_t, 0 for a zero s_t).
+ * Decoding code * 2^(scale - 127), or code * RN(s_b * s_t), gives qsb_fq_block_fwd_dt's y. */
+int qsb_block_export_dt(const void *x, int x_dtype, uint8_t *codes, uint8_t *scales, int64_t rows,
+                        int64_t L, int fmt, const float *tensor_amax_dev, void *stream);
+
 /* ------------------------------------------------------------------------
  * K2  straight-through-estimator backward (and the fused prune backward).
  * ref: DecimalQuantization.backward qsparse/quantize.py:65-77,

@@ -6,6 +6,7 @@ from .convert import convert
 from .fuse import fuse_bn
 from .fused import fuse_prune_quantize
 from .quantize import quantize, DecimalQuantizer, ScalerQuantizer, AdaptiveQuantizer, PercentileQuantizer
+from .quantize import BlockScaledQuantizer, export_block_scaled, dequantize_block_scaled
 from .sparse import MagnitudePruningCallback, UniformPruningCallback, prune, devise_layerwise_pruning_schedule
 from .sparse import WeightSetPruner
 from .graphs import GraphedTrainStep

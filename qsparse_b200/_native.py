@@ -38,6 +38,8 @@ _SIGNATURES = {
                                       c_int64, _P]),
     "qsb_quant_export_int4": (c_int, [_P, _P, c_int, _P, c_int64, c_double, c_double, c_int, c_int64, c_int64,
                                       c_int64, _P]),
+    "qsb_fq_block_fwd_dt": (c_int, [_P, c_int, _P, c_int64, c_int64, c_int, _P, _P]),
+    "qsb_block_export_dt": (c_int, [_P, c_int, _P, _P, c_int64, c_int64, c_int, _P, _P]),
     "qsb_ste_bwd": (c_int, [_P, _P, _P, _P, c_int64, c_double, c_int, c_int, c_int, _P, c_int,
                             c_int64, c_int64, c_int64, _P]),
     "qsb_mask_apply": (c_int, [_P, _P, _P, c_int, c_int64, c_int64, c_int64, _P]),

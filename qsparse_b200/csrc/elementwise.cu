@@ -16,12 +16,6 @@ void set_select_fast(int v);
 
 namespace qsb {
 
-// Outputs that do not fit the L2 anyway (>= 96 MB) are stored with L2::evict_first: their dirty lines then leave the
-// cache while the kernel still runs instead of being written back under the NEXT kernel's traffic, and the lines a
-// predecessor tagged evict_last (the fused statistics kernel's keep hint) survive longer.  Bench step, A/B with two
-// library builds on one box: 142.0 -> 140.1 us (forward alone 140.8, backward alone 142.9), dense line 165.1 -> 164.0
-// (profiles/r02_store_hint_ab.json).  Smaller outputs keep the default policy: a consumer may find them in L2.
-constexpr int64_t kStreamStoreBytes = 96ll << 20;
 template <class Op, class IO>
 int launch_map_big_out(const Op &op, const IO &io, const Layout &L, cudaStream_t stream) {
   if (L.numel() * 4 >= kStreamStoreBytes) return launch_map<Op, Hint::STREAM, Hint::STREAM>(op, io, L, stream);

@@ -102,6 +102,13 @@ __device__ __forceinline__ void store_outb(uint8_t *outb, int64_t e, const VecB<
   }
 }
 
+// Outputs that do not fit the L2 anyway (>= 96 MB) are stored with L2::evict_first: their dirty lines then leave the
+// cache while the kernel still runs instead of being written back under the NEXT kernel's traffic, and the lines a
+// predecessor tagged evict_last (the fused statistics kernel's keep hint) survive longer.  Bench step, A/B with two
+// library builds on one box: 142.0 -> 140.1 us (forward alone 140.8, backward alone 142.9), dense line 165.1 -> 164.0
+// (profiles/r02_store_hint_ab.json).  Smaller outputs keep the default policy: a consumer may find them in L2.
+constexpr int64_t kStreamStoreBytes = 96ll << 20;
+
 // Tile order of the one-CTA-per-tile kernels (tuning key 2).  1 (default): last tile first.  The
 // tensor a streaming kernel reads was normally just produced / reduced front to
 // back, so its TAIL is what still sits in the 126 MB L2; walking backwards turns

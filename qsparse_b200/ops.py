@@ -215,6 +215,50 @@ def quant_export_int8(x, kind: int, param, bits: int, layout: Layout, pack4: boo
     return q
 
 
+# block-scaled FP8 / FP4 formats: name -> (C-ABI code, elements per block)
+BLOCK_FORMATS = {"mxfp8": (0, 32), "mxfp4": (1, 32), "nvfp4": (2, 16)}
+
+
+def _block_args(x, fmt: str, rows: int, L: int, tensor_amax):
+    N.require_cuda(x, "input")
+    if fmt not in BLOCK_FORMATS:
+        raise ValueError(f"fmt must be one of {sorted(BLOCK_FORMATS)}, got {fmt!r}")
+    if rows * L != x.numel():
+        raise ValueError(f"[rows, L] = [{rows}, {L}] does not cover the {x.numel()} elements of x")
+    if fmt == "nvfp4":
+        if tensor_amax is None:
+            raise ValueError("nvfp4 needs the tensor abs-max `tensor_amax` (a one-element CUDA tensor)")
+        N.require_cuda(tensor_amax, "tensor_amax")
+        tensor_amax = tensor_amax.detach().reshape(-1)[:1].float().contiguous()
+    else:
+        tensor_amax = None
+    return BLOCK_FORMATS[fmt][0], tensor_amax
+
+
+def fq_block_fwd(x, fmt: str, rows: int, L: int, tensor_amax=None):
+    """Block-scaled fake quantization of x walked as [rows, L] in its memory order (``qsb_fq_block_fwd_dt``).
+    x: fp32, bf16 or fp16, read natively; the result is fp32 in x's memory format.  ``tensor_amax``: nvfp4's w."""
+    lib = N.load_library()
+    code, w = _block_args(x, fmt, rows, L, tensor_amax)
+    y = _f32_like(x)
+    N.check(lib.qsb_fq_block_fwd_dt(N.ptr(x), c_int(N.dtype_code(x)), N.ptr(y), c_int64(rows), c_int64(L), c_int(code),
+                                    N.ptr(w), N.stream_ptr(x.device)), "qsb_fq_block_fwd_dt")
+    return y
+
+
+def block_export(x, fmt: str, rows: int, L: int, tensor_amax=None):
+    """(codes, scales) of the same quantizer in one pass (``qsb_block_export_dt``): uint8 codes [rows, L] (E4M3) or
+    [rows, ceil(L / 2)] (two E2M1 codes per byte, element 2i in the low nibble), uint8 scales [rows, ceil(L / B)]."""
+    lib = N.load_library()
+    code, w = _block_args(x, fmt, rows, L, tensor_amax)
+    B = BLOCK_FORMATS[fmt][1]
+    codes = torch.empty((rows, L if fmt == "mxfp8" else (L + 1) // 2), dtype=torch.uint8, device=x.device)
+    scales = torch.empty((rows, (L + B - 1) // B), dtype=torch.uint8, device=x.device)
+    N.check(lib.qsb_block_export_dt(N.ptr(x), c_int(N.dtype_code(x)), N.ptr(codes), N.ptr(scales), c_int64(rows),
+                                    c_int64(L), c_int(code), N.ptr(w), N.stream_ptr(x.device)), "qsb_block_export_dt")
+    return codes, scales
+
+
 # ----------------------------------------------------------------------------- K6
 def mask_apply(x, mask, layout: Layout, out=None, out_dtype=None):
     """``x * mask``; x and the result may differ in dtype when one of them is fp32 and the other bf16 / fp16

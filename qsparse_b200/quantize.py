@@ -200,6 +200,39 @@ class LineQuantization(torch.autograd.Function):
         return (grad_output,) + (None,) * 6
 
 
+def _block_rows(x: torch.Tensor, rows: str):
+    """(tensor whose memory the kernel walks, R, L) of the ``[R, L]`` view of a block-scaled quantizer.
+
+    ``rows="last"``: L is the innermost physical axis — the last axis of a contiguous tensor, C of a 4-D
+    ``channels_last`` one (walked in its NHWC order, so the output keeps x's memory format).  ``rows="leading"``:
+    the contiguous tensor as ``[x.shape[0], numel / x.shape[0]]``.  Anything else is made contiguous first."""
+    x = N.as_native(x)
+    if rows == "last" and not x.is_contiguous() and x.dim() == 4 and x.is_contiguous(memory_format=torch.channels_last):
+        L = int(x.shape[1])
+    else:
+        x = x.contiguous()
+        if rows == "last":
+            L = int(x.shape[-1]) if x.dim() else 1
+        else:
+            R = int(x.shape[0]) if x.dim() else 1
+            L = x.numel() // R if R else 0
+    return x, (x.numel() // L if L else 0), L
+
+
+class BlockScaledQuantization(torch.autograd.Function):
+    """Block-scaled FP8 / FP4 fake quantization (``BlockScaledQuantizer``) with an identity backward."""
+
+    @staticmethod
+    def forward(ctx, input: torch.Tensor, fmt: str = "nvfp4", rows: str = "last", tensor_amax=None):
+        N.require_cuda(input, "input")
+        xs, R, L = _block_rows(input.detach(), rows)
+        return ops.fq_block_fwd(xs, fmt, R, L, tensor_amax)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        return grad_output, None, None, None
+
+
 class _RowFusedSte(torch.autograd.Function):
     """K8 for the symmetric quantizers on a `channelwise=0` tensor: per-row abs-max -> scale EMA (into
     ``weight``, in place) -> [decimal] -> fake-quantize in ONE launch (``qsb_row_quant_fused``); the backward
@@ -509,6 +542,69 @@ class PercentileQuantizer(DecimalQuantizer):
         return None          # the fused abs-max routes do not apply
 
 
+class BlockScaledQuantizer(BaseQuantizer):
+    """EXTENSION (not in qsparse 2.0.1): quantization-aware training for the block-scaled FP8 / FP4 formats whose
+    operands B200 tensor cores take natively,
+
+        ``"mxfp8"``  blocks of 32, E4M3 elements, E8M0 power-of-two block scale   (OCP Microscaling v1.0)
+        ``"mxfp4"``  blocks of 32, E2M1 elements, E8M0 power-of-two block scale   (OCP Microscaling v1.0)
+        ``"nvfp4"``  blocks of 16, E2M1 elements, E4M3 block scale times the tensor scale ``w / 2688``
+
+    Blocks are runs of consecutive elements of the rows of x viewed as ``[R, L]``: ``rows="last"`` splits the
+    innermost physical axis (the reduction axis of a Linear weight and of ``[tokens, hidden]`` activations; C of a
+    ``channels_last`` tensor), ``rows="leading"`` the contiguous tensor as ``[x.shape[0], -1]`` (the reduction axis of
+    a conv weight).  The numerics are DESIGN §2 "Block-scaled formats"; the layer's ``bits`` is not used.
+
+    The block scales are derived from each input, so the layer's ``weight`` ``[1, 1]`` only holds nvfp4's ``w``: the
+    running mean of the tensor's abs-max, the ``DecimalQuantizer`` EMA at one bit.  The mx formats keep it at 0 and
+    ``optimize`` only counts calls.  Output is fp32; the backward is the identity (straight-through).  Per tensor
+    only (``channelwise=-1``).  ``export_block_scaled`` writes the packed codes and scales."""
+
+    weight_size = 1
+
+    def __init__(self, fmt: str = "nvfp4", rows: str = "last"):
+        super().__init__()
+        if fmt not in ops.BLOCK_FORMATS:
+            raise ValueError(f"fmt must be one of {sorted(ops.BLOCK_FORMATS)}, got {fmt!r}")
+        if rows not in ("last", "leading"):
+            raise ValueError(f'rows must be "last" or "leading", got {rows!r}')
+        self.fmt, self.rows = fmt, rows
+        self.t = 0  # Python int like DecimalQuantizer's: not part of state_dict
+
+    @staticmethod
+    def check_channelwise(channelwise: int):
+        if channelwise != -1:
+            raise ValueError("BlockScaledQuantizer scales blocks inside each row: it needs channelwise=-1, "
+                             f"got {channelwise}")
+
+    def optimize(self, x, bits, weight=None, batched=False, channel_index=-1, **kwargs):
+        self.check_channelwise(channel_index)
+        N.require_cuda(x, "x")
+        if self.fmt == "nvfp4":
+            with torch.no_grad():
+                xs, layout = _physical_layout(N.as_native(x.detach()), -1, False)
+                absmax = ops.reduce_stats(xs, layout, absmax=True)["absmax"]
+                if weight is None:
+                    weight = torch.zeros((1, 1), dtype=torch.float32, device=x.device)
+                target = weight.data if isinstance(weight, nn.Parameter) else weight
+                assert tuple(target.shape) == (1, 1) and target.is_contiguous()
+                if graphs.active():
+                    counter = graphs.quantizer_counter(self, x.device)
+                    ops.scale_ema_(target, absmax, 1, 0, t_dev=counter)
+                    counter.add_(1)
+                else:
+                    ops.scale_ema_(target, absmax, 1, self.t)
+        self.t += 1
+        return weight
+
+    def forward(self, x, bits, weight=None, channel_index=-1, **kwargs):
+        self.check_channelwise(channel_index)
+        return BlockScaledQuantization.apply(x, self.fmt, self.rows, weight if self.fmt == "nvfp4" else None)
+
+    def optimize_and_forward(self, *args, **kwargs):
+        return None          # no fused route: optimize() then forward()
+
+
 class ScalerQuantizer(DecimalQuantizer):
     """Same estimator without the power-of-two restriction (ref qsparse/quantize.py:370-378)."""
 
@@ -603,6 +699,8 @@ class QuantizeLayer(nn.Module):
     def __init__(self, bits: int = 8, channelwise: int = 1, timeout: int = 1000, callback: BaseQuantizer = None,
                  batch_dimension: int = 0, name: str = ""):
         super().__init__()
+        if isinstance(callback, BlockScaledQuantizer):
+            callback.check_channelwise(channelwise)
         if get_option("log_on_created"):
             logging.info(f"[Quantize{name if name == '' else f' @ {name}'}] bits={bits} "
                          f"channelwise={channelwise} timeout={timeout}")
@@ -707,6 +805,59 @@ def unpack_int4(exported: dict) -> torch.Tensor:
     if exported["kind"] == "line":
         return nib.reshape(shape)
     return ((nib.to(torch.int16) ^ 8) - 8).to(torch.int8).reshape(shape)   # sign-extend the 4-bit code
+
+
+def export_block_scaled(layer: "QuantizeLayer", x: torch.Tensor) -> dict:
+    """Packed deployment form of what a ``BlockScaledQuantizer`` layer computes for ``x``, in one pass
+    (``qsb_block_export_dt``):
+
+        codes         uint8 ``[R, L]`` E4M3 (mxfp8) or ``[R, ceil(L / 2)]`` E2M1 pairs, element 2i in the low nibble
+        scales        uint8 ``[R, ceil(L / B)]``: E8M0 (mx formats, 0xFF for a NaN block) or E4M3 (nvfp4)
+        tensor_scale  nvfp4's fp32 ``[1]`` ``w / 2688`` (None for the mx formats)
+
+    plus ``fmt``, ``shape`` (x's), ``rows``, ``L`` and ``channels_last`` (the ``[R, L]`` view walks x in NHWC
+    order).  ``dequantize_block_scaled`` turns it back into the layer's forward output bit for bit."""
+    assert isinstance(layer, QuantizeLayer) and layer.initted and isinstance(layer.callback, BlockScaledQuantizer)
+    cb = layer.callback
+    N.require_cuda(x, "x")
+    xs, R, L = _block_rows(x.detach(), cb.rows)
+    w = layer.weight.data if cb.fmt == "nvfp4" else None
+    codes, scales = ops.block_export(xs, cb.fmt, R, L, w)
+    tensor_scale = None
+    if w is not None:
+        # a tensor divisor: torch turns division by a Python scalar into a multiplication by its reciprocal
+        w1 = w.reshape(1).float()
+        tensor_scale = torch.div(w1, torch.full_like(w1, 2688.0))
+    return dict(codes=codes, scales=scales, tensor_scale=tensor_scale, fmt=cb.fmt, shape=tuple(x.shape),
+                rows=cb.rows, L=L, channels_last=not xs.is_contiguous())
+
+
+_E2M1_VALUES = (0.0, 0.5, 1.0, 1.5, 2.0, 3.0, 4.0, 6.0, -0.0, -0.5, -1.0, -1.5, -2.0, -3.0, -4.0, -6.0)
+
+
+def dequantize_block_scaled(exported: dict) -> torch.Tensor:
+    """The fp32 values of an ``export_block_scaled`` result, in x's shape (plain torch ops; a reader-side helper,
+    not a hot path): element code times its block's scale, ``2^(e - 127)`` or ``RN(s_b * tensor_scale)``."""
+    fmt, codes, scales, L = exported["fmt"], exported["codes"], exported["scales"], exported["L"]
+    B = ops.BLOCK_FORMATS[fmt][1]
+    R = codes.shape[0]
+    if fmt == "mxfp8":
+        v = codes.view(torch.float8_e4m3fn).float()
+    else:
+        lut = torch.tensor(_E2M1_VALUES, dtype=torch.float32, device=codes.device)
+        v = lut[torch.stack([codes & 0xF, codes >> 4], dim=-1).reshape(R, -1)[:, :L].long()]
+    if fmt == "nvfp4":
+        s = scales.view(torch.float8_e4m3fn).float() * exported["tensor_scale"]
+    else:
+        e = scales.to(torch.int32)
+        bits = torch.where(e == 0, torch.full_like(e, 0x00400000), e << 23)   # E8M0 0 is the subnormal 2^-127
+        s = torch.where(e == 255, torch.full_like(e, 0x7FC00000), bits).view(torch.float32)
+    y = v * s.repeat_interleave(B, dim=1)[:, :L]
+    shape = exported["shape"]
+    if exported["channels_last"]:
+        n, c, h, w = shape
+        return y.reshape(n, h, w, c).permute(0, 3, 1, 2)
+    return y.reshape(shape)
 
 
 def quantize(inp: nn.Module = None, bits: int = 8, channelwise: int = 1, timeout: int = 1000,
