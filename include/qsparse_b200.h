@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define QSB_ABI_VERSION 3
+#define QSB_ABI_VERSION 4
 
 /* argument errors */
 #define QSB_E_BADARG (-1)     /* null pointer / negative size / bad enum        */
@@ -254,18 +254,6 @@ int qsb_reduce_stats(const float *x, int what, int64_t outer, int64_t channels,
                      int64_t inner, float *absmax, float *mn, float *mx,
                      double *abssum, double *nnz, float *tensor_min,
                      void *workspace, int64_t workspace_bytes, void *stream);
-/* The same in ONE launch whenever the partial array is small enough for one CTA to combine in a
- * few L2 round trips (<= 256 channels with <= 12 x threads-per-channel partials each, e.g. the 64
- * channels of the bench tensor or per-tensor statistics; or one partial per channel, e.g. 4096
- * weight rows): the last-arriving CTA of the reduction combines the partials itself instead of a
- * second, latency-only launch.  Falls back to
- * the two-launch form otherwise.  arrival_counter_dev: one device uint32, zero before the first
- * use, left zero (one per stream that may run this concurrently). */
-int qsb_reduce_stats_fused(const float *x, int what, int64_t outer, int64_t channels,
-                           int64_t inner, float *absmax, float *mn, float *mx,
-                           double *abssum, double *nnz, float *tensor_min,
-                           void *workspace, int64_t workspace_bytes,
-                           unsigned int *arrival_counter_dev, void *stream);
 /* qsb_reduce_stats on an x of element type x_dtype (QSB_DTYPE_*).  The reduction plan —
  * segments, row bands, vectors of 8, fp32 pre-sums and with them the summation order — is
  * the same function of the shape for every dtype (vectors are counted from x[0], i.e. as

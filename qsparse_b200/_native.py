@@ -64,8 +64,6 @@ _SIGNATURES = {
                                            c_int64, c_int, c_int, c_int64, c_int64, _P, _P, _P, _P, _P]),
     "qsb_reduce_workspace_bytes": (c_int64, [c_int64, c_int64, c_int64]),
     "qsb_reduce_stats": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P]),
-    "qsb_reduce_stats_fused": (c_int, [_P, c_int, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P,
-                                       _P]),
     "qsb_scale_ema": (c_int, [_P, _P, c_int64, c_int, c_int64, _P]),
     "qsb_scale_to_decimal": (c_int, [_P, _P, c_int64, _P]),
     "qsb_lines_ema": (c_int, [_P, _P, _P, c_int64, c_int64, _P]),
@@ -164,7 +162,7 @@ def load_library() -> ctypes.CDLL:
         fn = getattr(lib, name)  # AttributeError if the symbol is missing
         fn.restype = res
         fn.argtypes = args
-    if lib.qsb_abi_version() != 3:
+    if lib.qsb_abi_version() != 4:
         raise NativeLibraryError("libqsparse_b200.so ABI version mismatch; rebuild it")
     _lib = lib
     return lib

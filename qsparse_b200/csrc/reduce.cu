@@ -145,11 +145,8 @@ __device__ __forceinline__ void warp_store(const Acc<WHAT> &a_in, int lane,
 // LAST at a device-wide counter — no separate finalize / parameter launch, and across GPUs
 // the peer exchange starts the moment this GPU's statistics are complete.  NoTail: plain stage 1.
 // ---------------------------------------------------------------------------
-struct NoTail {
-  static constexpr bool kFused = false;
-};
+struct NoTail {};
 struct StepTail {
-  static constexpr bool kFused = true;
   StepArgs a;
   unsigned int *arrival;     // zero before the first launch; the last CTA resets it
   const uint8_t *keep_hint;  // optional channel mask of the previous step (L2 residency hint)
@@ -194,215 +191,12 @@ __device__ __forceinline__ StepPrefetch fused_step_begin(const Tail &tail) {
   }
 }
 
-// ---------------------------------------------------------------------------
-// The same idea for the stand-alone reductions (qsb_reduce_stats): when the partial array is small
-// (final_tail_ok) the last-arriving CTA of stage 1 combines the partials itself, in a fixed order,
-// instead of a second launch that is pure latency
-// (3.5-5 us behind a 12-35 us stage 1).
-// ---------------------------------------------------------------------------
+// where stage 2 writes the finalized statistics (NULL: not wanted).  Stand-alone reductions always finalize in a
+// second launch: letting stage 1's last-arriving CTA do it was measured slower (DESIGN §8, row 8).
 struct FinalOut {
   float *absmax, *mn, *mx;
   double *abssum, *nnz;
 };
-struct FinalTail {
-  static constexpr bool kFused = true;
-  FinalOut out;
-  unsigned int *arrival;
-  int64_t channels, count, q;
-  int group;  // threads per channel in the tail
-};
-
-// One CTA finalizes every channel: `group` threads per channel (a power of two; the whole CTA for one channel),
-// all channels of a pass and all loads of a thread in flight at once — the tail is a handful of L2 round trips,
-// not one per channel.  The host only fuses shapes for which that holds (final_tail_ok).
-constexpr int kFinalBatch = 12;
-template <int WHAT>
-__device__ __forceinline__ void finalize_in_cta(const Partials &P, const FinalTail &t) {
-  const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5;
-  const float qnan = __uint_as_float(0x7fc00000u);
-  if (t.count == 1) {
-    // one partial per channel (e.g. 4096 weight rows): a strided copy, 8 independent loads per thread
-    for (int64_t c0 = tid; c0 < t.channels; c0 += 8 * (int64_t)nthr) {
-      uint32_t a_[8];
-      float n_[8], x_[8];
-      double s_[8], z_[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int64_t c = c0 + (int64_t)u * nthr;
-        if (c < t.channels) {
-          if constexpr (WHAT & QSB_STAT_ABSMAX) a_[u] = __ldcg(P.amax + c);
-          if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ)) n_[u] = __ldcg(P.mn + c);
-          if constexpr (WHAT & QSB_STAT_MINMAX) x_[u] = __ldcg(P.mx + c);
-          if constexpr (WHAT & QSB_STAT_ABSSUM) s_[u] = __ldcg(P.asum + c);
-          if constexpr (WHAT & QSB_STAT_NNZ) z_[u] = __ldcg(P.nnz + c);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int64_t c = c0 + (int64_t)u * nthr;
-        if (c < t.channels) {
-          if constexpr (WHAT & QSB_STAT_ABSMAX)
-            if (t.out.absmax) t.out.absmax[c] = __uint_as_float(a_[u]);
-          if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ)) {
-            bool nan = n_[u] != n_[u];
-            if constexpr (WHAT & QSB_STAT_MINMAX) nan = nan || (x_[u] != x_[u]);
-            if (t.out.mn) t.out.mn[c] = nan ? qnan : n_[u];
-            if constexpr (WHAT & QSB_STAT_MINMAX)
-              if (t.out.mx) t.out.mx[c] = nan ? qnan : x_[u];
-          }
-          if constexpr (WHAT & QSB_STAT_ABSSUM)
-            if (t.out.abssum) t.out.abssum[c] = s_[u];
-          if constexpr (WHAT & QSB_STAT_NNZ)
-            if (t.out.nnz) t.out.nnz[c] = z_[u];
-        }
-      }
-    }
-    return;
-  }
-  const int group = t.group;
-  const int gl = tid % group, gc = tid / group, cpp = nthr / group;
-  __shared__ uint32_t s_amax[32];
-  __shared__ float s_mn[32], s_mx[32];
-  __shared__ int s_nan[32];
-  __shared__ double s_asum[32], s_nnz[32];
-  for (int64_t base = 0; base < t.channels; base += cpp) {
-    const int64_t c = base + gc;
-    const bool act = c < t.channels;
-    uint32_t amax = 0;
-    float mn = INFINITY, mx = -INFINITY;
-    int nan = 0;
-    double asum = 0.0, nnz = 0.0;
-    if (act) {
-      for (int64_t j0 = gl; j0 < t.count; j0 += (int64_t)kFinalBatch * group) {
-        int64_t idx[kFinalBatch];
-        bool ok[kFinalBatch];
-#pragma unroll
-        for (int u = 0; u < kFinalBatch; ++u) {
-          const int64_t j = j0 + (int64_t)u * group;
-          ok[u] = j < t.count;
-          const int64_t hi = ok[u] ? (int64_t)((uint32_t)j / (uint32_t)t.q) : 0;
-          idx[u] = ok[u] ? hi * (t.channels * t.q) + c * t.q + (j - hi * t.q) : 0;
-        }
-        if constexpr (WHAT & QSB_STAT_ABSMAX) {
-          uint32_t b[kFinalBatch];
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) b[u] = ok[u] ? __ldcg(P.amax + idx[u]) : 0u;
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) amax = b[u] > amax ? b[u] : amax;
-        }
-        if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ)) {
-          float v[kFinalBatch];
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) v[u] = ok[u] ? __ldcg(P.mn + idx[u]) : INFINITY;
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) {
-            nan |= (v[u] != v[u]);
-            mn = fminf(mn, v[u]);
-          }
-        }
-        if constexpr (WHAT & QSB_STAT_MINMAX) {
-          float v[kFinalBatch];
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) v[u] = ok[u] ? __ldcg(P.mx + idx[u]) : -INFINITY;
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) {
-            nan |= (v[u] != v[u]);
-            mx = fmaxf(mx, v[u]);
-          }
-        }
-        if constexpr (WHAT & QSB_STAT_ABSSUM) {
-          double v[kFinalBatch];
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) v[u] = ok[u] ? __ldcg(P.asum + idx[u]) : 0.0;
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) asum += v[u];
-        }
-        if constexpr (WHAT & QSB_STAT_NNZ) {
-          double v[kFinalBatch];
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) v[u] = ok[u] ? __ldcg(P.nnz + idx[u]) : 0.0;
-#pragma unroll
-          for (int u = 0; u < kFinalBatch; ++u) nnz += v[u];
-        }
-      }
-    }
-    for (int o = (group < 32 ? group : 32) >> 1; o > 0; o >>= 1) {
-      const uint32_t a2 = __shfl_xor_sync(0xffffffffu, amax, o);
-      amax = a2 > amax ? a2 : amax;
-      mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-      mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-      nan |= __shfl_xor_sync(0xffffffffu, nan, o);
-      asum += __shfl_xor_sync(0xffffffffu, asum, o);
-      nnz += __shfl_xor_sync(0xffffffffu, nnz, o);
-    }
-    if (group > 32) {  // one channel, the whole CTA: combine the warps in warp order
-      if (lane == 0) {
-        s_amax[warp] = amax, s_mn[warp] = mn, s_mx[warp] = mx, s_nan[warp] = nan;
-        s_asum[warp] = asum, s_nnz[warp] = nnz;
-      }
-      __syncthreads();
-      if (gl == 0)
-        for (int w = 1; w < group / 32; ++w) {
-          amax = s_amax[warp + w] > amax ? s_amax[warp + w] : amax;
-          mn = fminf(mn, s_mn[warp + w]);
-          mx = fmaxf(mx, s_mx[warp + w]);
-          nan |= s_nan[warp + w];
-          asum += s_asum[warp + w];
-          nnz += s_nnz[warp + w];
-        }
-      __syncthreads();
-    }
-    if (act && gl == 0) {
-      if constexpr (WHAT & QSB_STAT_ABSMAX)
-        if (t.out.absmax) t.out.absmax[c] = __uint_as_float(amax);
-      if constexpr (WHAT & (QSB_STAT_MINMAX | QSB_STAT_NNZ))
-        if (t.out.mn) t.out.mn[c] = nan ? qnan : mn;
-      if constexpr (WHAT & QSB_STAT_MINMAX)
-        if (t.out.mx) t.out.mx[c] = nan ? qnan : mx;
-      if constexpr (WHAT & QSB_STAT_ABSSUM)
-        if (t.out.abssum) t.out.abssum[c] = asum;
-      if constexpr (WHAT & QSB_STAT_NNZ)
-        if (t.out.nnz) t.out.nnz[c] = nnz;
-    }
-  }
-}
-
-// which shapes the tail takes: a pure copy (one partial per channel), or ONE pass over the channels with
-// ONE batch of loads per thread
-inline bool final_tail_ok(int64_t channels, int64_t fin_count, int64_t fin_q) {
-  if (fin_count >= 0x7fffffffLL || fin_q >= 0x7fffffffLL) return false;
-  if (fin_count == 1) return channels <= 16384;
-  if (channels > QSB_THREADS) return false;
-  return fin_count <= (int64_t)kFinalBatch * step_group_for(channels, QSB_THREADS);
-}
-
-// last-arriver election shared by the two tails
-__device__ __forceinline__ bool cta_is_last(unsigned int *arrival) {
-  __shared__ int s_last;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned total = gridDim.x * gridDim.y;
-    __threadfence();
-    const int last = atomicAdd(arrival, 1u) == total - 1;
-    if (last) {
-      __threadfence();
-      *arrival = 0;
-    }
-    s_last = last;
-  }
-  __syncthreads();
-  return s_last != 0;
-}
-
-template <int WHAT>
-__device__ __forceinline__ void fused_tail(const FinalTail &t, const Partials &P, unsigned char *, const StepPrefetch &) {
-  if (cta_is_last(t.arrival)) finalize_in_cta<WHAT>(P, t);
-}
-template <int WHAT>
-__device__ __forceinline__ void fused_tail(const StepTail &t, const Partials &, unsigned char *smem,
-                                           const StepPrefetch &pre) {
-  fused_step_tail<kLineStep<WHAT>>(t, smem, pre);
-}
 
 // 256-bit load with a run-time L2 eviction policy (createpolicy): kept channels of the previous
 // mask are read evict_last — the forward pass re-reads exactly those a few microseconds later,
@@ -570,7 +364,7 @@ __global__ void __launch_bounds__(QSB_THREADS, MINB)
       warp_store<WHAT>(acc, lane, P, vw);
     }
   }
-  if constexpr (Tail::kFused) fused_tail<WHAT>(tail, P, qsb_dyn_smem, pre);
+  if constexpr (std::is_same<Tail, StepTail>::value) fused_step_tail<kLineStep<WHAT>>(tail, qsb_dyn_smem, pre);
 #ifdef QSB_KERNEL_TIMING
   if constexpr (std::is_same<Tail, StepTail>::value) ktime_end(0);
 #endif
@@ -682,7 +476,7 @@ __global__ void __launch_bounds__(QSB_THREADS)
   if constexpr (std::is_same<Tail, StepTail>::value) pdl_wait();  // the old state may have been written by the kernel just before
   const StepPrefetch pre = fused_step_begin<WHAT>(tail);
   reduce_cols_body<WHAT, V, T>(x, nrows, ncols, rows_per_chunk, tpr, P);
-  if constexpr (Tail::kFused) fused_tail<WHAT>(tail, P, qsb_dyn_smem, pre);
+  if constexpr (std::is_same<Tail, StepTail>::value) fused_step_tail<kLineStep<WHAT>>(tail, qsb_dyn_smem, pre);
 }
 
 // ---------------------------------------------------------------------------
@@ -1141,8 +935,7 @@ extern "C" int64_t qsb_reduce_workspace_bytes(int64_t outer, int64_t channels,
 template <class T>
 static int reduce_stats_impl(const T *x, int what, int64_t outer, int64_t channels, int64_t inner,
                              float *absmax, float *mn, float *mx, double *abssum, double *nnz,
-                             float *tensor_min, void *workspace, int64_t workspace_bytes,
-                             unsigned int *arrival, void *stream_) {
+                             float *tensor_min, void *workspace, int64_t workspace_bytes, void *stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
   if (!x || !workspace) return QSB_E_BADARG;
@@ -1156,17 +949,7 @@ static int reduce_stats_impl(const T *x, int what, int64_t outer, int64_t channe
   const Partials P = partials_from_workspace(workspace, pl.n_partials);
   FinalOut out{absmax, mn, mx, abssum, nnz};
   int rc;
-  // small partial arrays: the last-arriving CTA of stage 1 finalizes (one launch instead of two)
-  const bool fuse_final = arrival != nullptr && final_tail_ok(channels, pl.fin_count, pl.fin_q);
-  const FinalTail ft{out, arrival, channels, pl.fin_count, pl.fin_q, step_group_for(channels, QSB_THREADS)};
-  // the one-launch finalize is only offered for fp32 x (qsb_reduce_stats_fused); no 16-bit instantiation of it
-  auto go = [&](auto w) {
-    constexpr int W = decltype(w)::value;
-    if constexpr (!is_half16<T>) {
-      if (fuse_final) return run_reduce<W, FinalTail, T>(x, pl, channels, inner, P, out, stream, false, ft);
-    }
-    return run_reduce<W, NoTail, T>(x, pl, channels, inner, P, out, stream);
-  };
+  auto go = [&](auto w) { return run_reduce<decltype(w)::value, NoTail, T>(x, pl, channels, inner, P, out, stream); };
   switch (what) {
 #define QSB_CASE(W)                                  \
   case W:                                            \
@@ -1200,7 +983,7 @@ extern "C" int qsb_reduce_stats(const float *x, int what, int64_t outer, int64_t
                                 float *absmax, float *mn, float *mx, double *abssum, double *nnz,
                                 float *tensor_min, void *workspace, int64_t workspace_bytes, void *stream) {
   return reduce_stats_impl(x, what, outer, channels, inner, absmax, mn, mx, abssum, nnz, tensor_min, workspace,
-                           workspace_bytes, nullptr, stream);
+                           workspace_bytes, stream);
 }
 
 extern "C" int qsb_reduce_stats_dt(const void *x, int x_dtype, int what, int64_t outer, int64_t channels,
@@ -1209,21 +992,8 @@ extern "C" int qsb_reduce_stats_dt(const void *x, int x_dtype, int what, int64_t
   return dispatch_dtype(x_dtype, [&](auto *tx) {
     using T = std::remove_pointer_t<decltype(tx)>;
     return reduce_stats_impl(static_cast<const T *>(x), what, outer, channels, inner, absmax, mn, mx, abssum, nnz,
-                             tensor_min, workspace, workspace_bytes, nullptr, stream);
+                             tensor_min, workspace, workspace_bytes, stream);
   });
-}
-
-// The same in ONE launch whenever the partial array is small (channels x entries <= 16 Ki): the
-// last-arriving CTA of stage 1 combines the partials itself.  arrival_counter_dev as in
-// qsb_reduce_prune_quant_step (one zeroed uint32 per stream, left zero).
-extern "C" int qsb_reduce_stats_fused(const float *x, int what, int64_t outer, int64_t channels,
-                                      int64_t inner, float *absmax, float *mn, float *mx, double *abssum,
-                                      double *nnz, float *tensor_min, void *workspace,
-                                      int64_t workspace_bytes, unsigned int *arrival_counter_dev,
-                                      void *stream) {
-  if (!arrival_counter_dev) return QSB_E_BADARG;
-  return reduce_stats_impl(x, what, outer, channels, inner, absmax, mn, mx, abssum, nnz, tensor_min, workspace,
-                           workspace_bytes, arrival_counter_dev, stream);
 }
 
 // Stage 1 only: leaves the per-virtual-warp partials of sum|x| and max|x| (WHAT: sum|x| and min / max x) in the
@@ -1268,8 +1038,50 @@ extern "C" int qsb_reduce_partials(const float *x, int64_t outer, int64_t channe
 // finalize launch is cheaper than the serial tail (12 loads per thread and batch, 256 threads, <= 4 batches)
 constexpr int64_t kStepTailMaxEntries = 12288;
 
-// ONE launch for everything between "x is in HBM" and "apply" of the fused structured
-// prune -> pow2 quantize training step: the stage-1 reduction of sum|x| / max|x| whose
+// Stage 1 of the fused training step with its parameter step (step_epilogue.cuh): ONE launch whose
+// last-arriving CTA finalizes the partials and runs the step.  With too many partials per channel (column mode
+// on wide tensors) it is three launches instead: stage 1, a parallel finalize into a statistics row in the
+// workspace, then the step kernel on that row.  `a` is filled by fill_step_args / fill_line_step_args;
+// `keep_hint`: the previous step's mask (pow2 form) or NULL.
+template <int WHAT, class T>
+static int run_step(const T *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
+                    int64_t workspace_bytes, unsigned int *arrival_counter_dev, StepArgs a, const uint8_t *keep_hint,
+                    cudaStream_t stream) {
+  const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
+  if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
+  if (pl.fin_count > 0x7fffffffLL || pl.fin_q > 0x7fffffffLL) return QSB_E_UNSUPPORTED;
+  const Partials P = partials_from_workspace(workspace, pl.n_partials);
+  if (channels * pl.fin_count > kStepTailMaxEntries) {
+    if (workspace_bytes < partial_bytes(pl.n_partials) + 256 + stat_row_bytes(channels)) return QSB_E_WORKSPACE;
+    unsigned char *row = reinterpret_cast<unsigned char *>(
+        (reinterpret_cast<uintptr_t>(workspace) + 255) / 256 * 256 + (uintptr_t)partial_bytes(pl.n_partials));
+    double *row_sum = reinterpret_cast<double *>(row);
+    float *row_max = reinterpret_cast<float *>(row + (channels * 8 + 255) / 256 * 256);
+    float *row_min = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(row_max) +
+                                               (channels * 4 + 255) / 256 * 256);
+    // the pow2 form finalizes max|x| into row_max, the line form min / max x into row_min / row_max
+    const FinalOut out = kLineStep<WHAT> ? FinalOut{nullptr, row_min, row_max, row_sum, nullptr}
+                                         : FinalOut{row_max, nullptr, nullptr, row_sum, nullptr};
+    const int rc = run_reduce<WHAT, NoTail, T>(x, pl, channels, inner, P, out, stream);
+    if (rc) return rc;
+    if constexpr (kLineStep<WHAT>) a.row_min = row_min;
+    a.timing = nullptr;  // the phase stamps are those of the one-launch kernel
+    return launch_step_kernel_on_rows(a, row_sum, row_max, 1, 0, stream);
+  }
+  StepTail tail;
+  tail.a = a;
+  tail.a.P = P;
+  tail.a.fin_count = (int)pl.fin_count;
+  tail.a.fin_q = (int)pl.fin_q;
+  tail.arrival = arrival_counter_dev;
+  // channels the previous mask keeps are about to be re-read by the forward pass (only meaningful for a
+  // per-channel mask in row mode)
+  tail.keep_hint = (g_keep_hint && pl.row_mode && channels > 1) ? keep_hint : nullptr;
+  FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
+  return run_reduce<WHAT, StepTail, T>(x, pl, channels, inner, P, out, stream, /*finalize=*/false, tail);
+}
+
+// The fused structured prune -> pow2 quantize training step: the stage-1 reduction of sum|x| / max|x| whose
 // last-arriving CTA finalizes, exchanges the statistics row with the peer GPUs and derives
 // magnitude EMA / threshold / mask / scale / decimal (step_epilogue.cuh).
 template <class T>
@@ -1279,46 +1091,19 @@ static int reduce_prune_quant_step_impl(
     float *scale, float *decimal_out, qsb_p2p_group *group, int64_t step_stamp, double count,
     int64_t t_prune, int update_magnitude, int refresh_mask, int64_t k, int bits, int64_t t_quant,
     int update_scale, double *abssum_out, float *absmax_out, int stats_local,
-    int64_t *step_counter_dev, uint64_t *timing_out_dev, void *stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+    int64_t *step_counter_dev, uint64_t *timing_out_dev, void *stream) {
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
   if (channels > kStepFusedMaxChannels) return QSB_E_UNSUPPORTED;
   if (!x || !workspace || !arrival_counter_dev) return QSB_E_BADARG;
   if (!aligned_to(x, sizeof(T)) || !aligned_to(arrival_counter_dev, 4)) return QSB_E_ALIGN;
-  StepTail tail;
-  const int rc = fill_step_args(tail.a, magnitude, mask, scale, decimal_out, channels, group, step_stamp, count,
+  StepArgs a;
+  const int rc = fill_step_args(a, magnitude, mask, scale, decimal_out, channels, group, step_stamp, count,
                                 t_prune, update_magnitude, refresh_mask, k, bits, t_quant, update_scale,
                                 abssum_out, absmax_out, stats_local, step_counter_dev, QSB_THREADS);
   if (rc) return rc;
-  const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
-  if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
-  if (pl.fin_count > 0x7fffffffLL || pl.fin_q > 0x7fffffffLL) return QSB_E_UNSUPPORTED;
-  const Partials P = partials_from_workspace(workspace, pl.n_partials);
-  if (channels * pl.fin_count > kStepTailMaxEntries) {
-    // many partials per channel (column mode on wide tensors): stage 1, a parallel finalize into a statistics row
-    // in the workspace, then the parameter step as a one-CTA launch on that row — three launches
-    if (workspace_bytes < partial_bytes(pl.n_partials) + 256 + stat_row_bytes(channels)) return QSB_E_WORKSPACE;
-    unsigned char *row = reinterpret_cast<unsigned char *>(
-        (reinterpret_cast<uintptr_t>(workspace) + 255) / 256 * 256 + (uintptr_t)partial_bytes(pl.n_partials));
-    double *row_sum = reinterpret_cast<double *>(row);
-    float *row_max = reinterpret_cast<float *>(row + (channels * 8 + 255) / 256 * 256);
-    FinalOut out{row_max, nullptr, nullptr, row_sum, nullptr};
-    const int rc2 = run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, NoTail, T>(x, pl, channels, inner, P, out, stream);
-    if (rc2) return rc2;
-    tail.a.timing = nullptr;
-    return launch_step_kernel_on_rows(tail.a, row_sum, row_max, 1, 0, stream);
-  }
-  tail.a.P = P;
-  tail.a.fin_count = (int)pl.fin_count;
-  tail.a.fin_q = (int)pl.fin_q;
-  tail.arrival = arrival_counter_dev;
-  tail.a.timing = reinterpret_cast<unsigned long long *>(timing_out_dev);
-  // the previous step's mask as an L2 residency hint: channels it keeps are about to be re-read by
-  // the forward pass (only meaningful for a per-channel mask in row mode)
-  tail.keep_hint = (g_keep_hint && pl.row_mode && channels > 1) ? mask : nullptr;
-  FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
-  return run_reduce<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX, StepTail, T>(x, pl, channels, inner, P, out, stream,
-                                                                    /*finalize=*/false, tail);
+  a.timing = reinterpret_cast<unsigned long long *>(timing_out_dev);
+  return run_step<QSB_STAT_ABSSUM | QSB_STAT_ABSMAX>(x, outer, channels, inner, workspace, workspace_bytes,
+                                                     arrival_counter_dev, a, mask, (cudaStream_t)stream);
 }
 
 extern "C" int qsb_reduce_prune_quant_step_dt(
@@ -1354,43 +1139,7 @@ extern "C" int qsb_reduce_prune_quant_step(
 // The line form of the same step (AdaptiveQuantizer): the stage-1 reduction gathers sum|x| and min / max x, the
 // last-arriving CTA runs finalize -> magnitude EMA -> threshold -> mask -> (min, max) of x * mask -> lines EMA.
 // Same reduction plan, same summation order of sum|x| (the magnitudes equal those of the pow2 step bit for bit).
-template <class T>
-static int reduce_prune_line_step_impl(const T *x, int64_t outer, int64_t channels, int64_t inner, void *workspace,
-                                       int64_t workspace_bytes, unsigned int *arrival_counter_dev, const StepArgs &a,
-                                       cudaStream_t stream) {
-  constexpr int kWhat = QSB_STAT_ABSSUM | QSB_STAT_MINMAX;
-  if (!aligned_to(x, sizeof(T)) || !aligned_to(arrival_counter_dev, 4)) return QSB_E_ALIGN;
-  const ReducePlan pl = make_plan(outer, channels, inner, x, (int)sizeof(T));
-  if (workspace_bytes < partial_bytes(pl.n_partials) + 256) return QSB_E_WORKSPACE;
-  if (pl.fin_count > 0x7fffffffLL || pl.fin_q > 0x7fffffffLL) return QSB_E_UNSUPPORTED;
-  const Partials P = partials_from_workspace(workspace, pl.n_partials);
-  StepTail tail;
-  tail.a = a;
-  if (channels * pl.fin_count > kStepTailMaxEntries) {
-    // as the pow2 step: stage 1, a parallel finalize into a statistics row, the step kernel on that row
-    if (workspace_bytes < partial_bytes(pl.n_partials) + 256 + stat_row_bytes(channels)) return QSB_E_WORKSPACE;
-    unsigned char *row = reinterpret_cast<unsigned char *>(
-        (reinterpret_cast<uintptr_t>(workspace) + 255) / 256 * 256 + (uintptr_t)partial_bytes(pl.n_partials));
-    double *row_sum = reinterpret_cast<double *>(row);
-    float *row_max = reinterpret_cast<float *>(row + (channels * 8 + 255) / 256 * 256);
-    float *row_min = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(row_max) +
-                                               (channels * 4 + 255) / 256 * 256);
-    FinalOut out{nullptr, row_min, row_max, row_sum, nullptr};
-    const int rc = run_reduce<kWhat, NoTail, T>(x, pl, channels, inner, P, out, stream);
-    if (rc) return rc;
-    tail.a.row_min = row_min;
-    return launch_step_kernel_on_rows(tail.a, row_sum, row_max, 1, 0, stream);
-  }
-  tail.a.P = P;
-  tail.a.fin_count = (int)pl.fin_count;
-  tail.a.fin_q = (int)pl.fin_q;
-  tail.arrival = arrival_counter_dev;
-  // no L2 keep hint: the line forward reads the pruned channels too
-  tail.keep_hint = nullptr;
-  FinalOut out{nullptr, nullptr, nullptr, nullptr, nullptr};
-  return run_reduce<kWhat, StepTail, T>(x, pl, channels, inner, P, out, stream, /*finalize=*/false, tail);
-}
-
+// No L2 keep hint: the line forward reads the pruned channels too.
 extern "C" int qsb_reduce_prune_line_step_dt(
     const void *x, int x_dtype, int64_t outer, int64_t channels, int64_t inner, void *workspace,
     int64_t workspace_bytes, unsigned int *arrival_counter_dev, float *magnitude, uint8_t *mask, float *lines,
@@ -1408,7 +1157,9 @@ extern "C" int qsb_reduce_prune_line_step_dt(
   if (rc) return rc;
   return dispatch_dtype(x_dtype, [&](auto *tx) {
     using T = std::remove_pointer_t<decltype(tx)>;
-    return reduce_prune_line_step_impl(static_cast<const T *>(x), outer, channels, inner, workspace,
-                                       workspace_bytes, arrival_counter_dev, a, (cudaStream_t)stream);
+    const T *xt = static_cast<const T *>(x);
+    if (!aligned_to(xt, sizeof(T)) || !aligned_to(arrival_counter_dev, 4)) return QSB_E_ALIGN;
+    return run_step<QSB_STAT_ABSSUM | QSB_STAT_MINMAX>(xt, outer, channels, inner, workspace, workspace_bytes,
+                                                       arrival_counter_dev, a, nullptr, (cudaStream_t)stream);
   });
 }

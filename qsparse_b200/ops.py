@@ -274,14 +274,6 @@ def mask_apply(x, mask, layout: Layout, out=None, out_dtype=None):
 
 
 # ----------------------------------------------------------------------------- K3
-# True: small partial arrays are finalized by the reduction's last-arriving CTA (qsb_reduce_stats_fused, one launch).
-# Measured on B200 and NOT the default: the serial tail (fence, atomic, one L2 round trip, the writes; ~4-5 us) costs
-# more than a second launch whose latency programmatic dependent launch already hides — per-channel sum|x| + max|x|
-# of the bench tensor 37.9 us (two launches) vs 40.9 us (one), per-tensor abs-max 38.9 vs 38.9.  The training step's
-# fused kernel is a different trade: its tail replaces a whole dependent parameter kernel, not a 3.5 us finalize.
-FUSE_REDUCE_FINALIZE = False
-
-
 def reduce_stats(x, layout: Layout, absmax=False, minmax=False, abssum=False, nnz=False, out=None):
     """One read of x -> dict of per-channel statistics (device tensors).  ``out`` may
     supply pre-allocated result tensors (e.g. views into a statistics row that is
@@ -306,13 +298,6 @@ def reduce_stats(x, layout: Layout, absmax=False, minmax=False, abssum=False, nn
         res["tensor_min"] = torch.empty(1, dtype=torch.float32, device=dev)
     nbytes = lib.qsb_reduce_workspace_bytes(c_int64(outer), c_int64(ch), c_int64(inner))
     ws = N.workspace(dev, nbytes)
-    if FUSE_REDUCE_FINALIZE and x.dtype == torch.float32:
-        N.check(lib.qsb_reduce_stats_fused(N.ptr(x), c_int(what), c_int64(outer), c_int64(ch), c_int64(inner),
-                                           N.ptr(res.get("absmax")), N.ptr(res.get("min")), N.ptr(res.get("max")),
-                                           N.ptr(res.get("abssum")), N.ptr(res.get("nnz")),
-                                           N.ptr(res.get("tensor_min")), N.ptr(ws), c_int64(ws.numel()),
-                                           N.ptr(arrival_counter(dev)), N.stream_ptr(dev)), "qsb_reduce_stats_fused")
-        return res
     N.check(lib.qsb_reduce_stats_dt(N.ptr(x), c_int(N.dtype_code(x)), c_int(what), c_int64(outer), c_int64(ch),
                                     c_int64(inner), N.ptr(res.get("absmax")), N.ptr(res.get("min")),
                                     N.ptr(res.get("max")), N.ptr(res.get("abssum")), N.ptr(res.get("nnz")),

@@ -23,13 +23,15 @@ def test_header_symbols_are_exported():
     assert len(names) >= 25
     for name in names:
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
+    # removed in ABI 4: stand-alone reductions finalize in a second launch only
+    assert not hasattr(lib, "qsb_reduce_stats_fused")
 
 
 def test_python_binding_covers_header():
     from qsparse_b200 import _native
     assert sorted(_native.exported_symbols()) == declared_symbols()
     lib = _native.load_library()
-    assert lib.qsb_abi_version() == 3
+    assert lib.qsb_abi_version() == 4
     assert b"bad argument" in lib.qsb_error_string(-1)
 
 
