@@ -724,7 +724,12 @@ int qsb_host_prune_quant_step(qsb_host_ctx *ctx, const float *x_host,
  * transfers per direction per step instead of 3 serial ones.  Steps are applied to
  * the layer state in submission order.  Each slot needs its own four host buffers;
  * qsb_host_ctx_wait(ctx, slot) returns when that slot's y_host / gx_host are
- * complete (submitting to a busy slot waits for it first). */
+ * complete (submitting to a busy slot waits for it first).
+ * Returns its code before any CUDA call (no wait, no copy, no launch) for a NULL
+ * ctx / host buffer / magnitude / mask / scale / decimal, a slot other than 0 or 1,
+ * a zero or negative dimension, more channels or elements than the context was
+ * created for, k outside [0, channels) when t_prune > 0, or a group whose channel
+ * count differs (QSB_E_BADARG), and for channels > 4096 (QSB_E_UNSUPPORTED). */
 int qsb_host_prune_quant_step_submit(qsb_host_ctx *ctx, int slot,
                                      const float *x_host, const float *g_host,
                                      float *y_host, float *gx_host,

@@ -23,6 +23,7 @@
 
 #include "p2p_internal.cuh"
 #include "qsb_common.cuh"
+#include "step_epilogue.cuh"
 
 constexpr int kHostSlots = 2;  // steps in flight: step t+1 uploads while step t downloads
 
@@ -133,6 +134,19 @@ extern "C" int qsb_host_prune_quant_step_submit(
   if (outer <= 0 || channels <= 0 || inner <= 0) return QSB_E_BADARG;
   if (channels > c->max_channels || outer * channels * inner > c->max_elems)
     return QSB_E_BADARG;
+  // Everything the parameter step below would refuse is refused here, before the implicit wait,
+  // the workspace regrow and the first copy: an error return then leaves no copy running from or
+  // into the caller's host buffers.  The forward and backward read the decimal, so it is required.
+  if (channels > qsb::kStepMaxChannels) return QSB_E_UNSUPPORTED;
+  if (!decimal_dev) return QSB_E_BADARG;
+  const double count = (double)outer * (double)inner * (group ? (double)group->dev.world : 1.0);
+  {
+    qsb::StepArgs unused;
+    const int rc = qsb::fill_step_args(unused, magnitude_dev, mask_dev, scale_dev, decimal_dev, channels, group,
+                                       step_stamp, count, t_prune, 1, t_prune > 0, k, bits, t_quant, 1, nullptr,
+                                       nullptr, 0, nullptr, 1024);
+    if (rc) return rc;
+  }
   qsb_host_slot &sl = c->slot[slot];
   if (sl.busy) {  // the slot's previous step must have been waited for: its host buffers
     int rc = qsb_host_ctx_wait(c, slot);  // and device staging are about to be reused
@@ -207,10 +221,9 @@ extern "C" int qsb_host_prune_quant_step_submit(
     const double *abssum0 = reinterpret_cast<const double *>(c->d_stats);
     const float *absmax0 =
         reinterpret_cast<const float *>(c->d_stats + channels * sizeof(double));
-    const double world = group ? (double)group->dev.world : 1.0;
     rc = qsb_prune_quant_rows_step_params(
         magnitude_dev, mask_dev, scale_dev, decimal_dev, abssum0, absmax0, n_chunks,
-        c->stats_row_bytes, channels, group, step_stamp, (double)outer * (double)inner * world, t_prune, 1,
+        c->stats_row_bytes, channels, group, step_stamp, count, t_prune, 1,
         t_prune > 0, k, bits, t_quant, 1, c->s_comp);
     if (rc) return rc;
   }

@@ -585,6 +585,7 @@ def mask_build_apply(importance, thr, x, mask_out, take_abs=False, out=None):
 
 FUSED_STEP_MAX_CHANNELS = 1024      # the reduction's last CTA runs the step (kStepFusedMaxChannels)
 STEP_KERNEL_MAX_CHANNELS = 4096     # the one-CTA step kernel's shared memory (kStepMaxChannels, step_epilogue.cuh)
+STEP_MAX_ROWS = 4096                # statistics rows the parameter step combines (qsb_prune_quant_params)
 # A route choice, not a kernel limit: up to here the step kernel finalizes the reduction's partials itself (and
 # runs the peer exchange); above it the statistics are finalized first.  Moving it changes which launch sequence
 # runs for 2049-4096 channels, which has not been measured.
@@ -617,7 +618,8 @@ def _prune_quant_params_composed(magnitude, mask, scale, decimal_out, stats, cou
     arithmetic in the same order, as magnitude EMA -> exact k-th value -> mask -> abs-max of the kept channels
     -> scale EMA -> decimal launches."""
     ch = mask.numel()
-    bad = (update_magnitude not in (0, 1, 2) or n_rows < 1 or (update_magnitude and not count > 0)
+    # the kernel's row count limit too, so that both routes take the same arguments
+    bad = (update_magnitude not in (0, 1, 2) or not 1 <= n_rows <= STEP_MAX_ROWS or (update_magnitude and not count > 0)
            or (refresh_mask and not 0 <= k < ch))
     if bad:
         N.check(-1, "qsb_prune_quant_params")     # QSB_E_BADARG, as the kernel's entry point returns it
